@@ -9,6 +9,11 @@ convolutions, 5 maxpools, reorg, in-place routes, region layer) + get_region_box
 final pick.  `value` is measured with the batch resident in HBM, `e2e` through the public C API
 with host buffers (pinned H2D of the images and D2H of the detection lists inside the timed
 region).  One JSON line on stdout (rank 0).
+
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+also writes the detections of the last timed step of `value` as DIR/*.npy (see dump_outputs), so that two
+builds can be compared output for output: weights and images come from fixed seeds.
 """
 from __future__ import annotations
 
@@ -40,6 +45,7 @@ SEED_W, SEED_X = 1234, 42
 # NMS keeps ~8 of them.  The reference arm reads the same weights file.
 HEAD_GAIN = 13.0
 GATHER_CAP = 32  # detections per image carried by the fixed-size host gather of the multi-rank e2e loop
+DUMP_MAX_BYTES = 64 << 20  # --dump-outputs: larger detection tables are replaced by a fixed, seeded sample of rows
 
 
 def _peaks():
@@ -187,6 +193,29 @@ def cpu_baseline(tmp: Path, iters: int = 20, warmup: int = 1) -> dict:
                       f"({d1['seconds']:.1f} s)"}
 
 
+def dump_outputs(out: Path, dets, counts) -> None:
+    """What network_detect_wait handed to the caller after the last timed step, for rank 0's batch:
+    counts.npy      [batch]          detections the library reported per image;
+    detections.npy  [n][8]           image, box_index, obj_id, prob, x, y, w, h of every returned detection,
+                                     image by image in the library's order (at most MAX_DET per image).
+    float64 holds the int32 and float32 fields of y2_det exactly.  Should the two files exceed DUMP_MAX_BYTES (only
+    at very large --batch), detections.npy keeps a seeded sample of its rows, in their original order."""
+    import numpy as np
+    counts = np.asarray(counts, np.float64)
+    rows = [np.zeros((0, 8))]
+    for b, n in enumerate(counts):
+        d = dets[b * MAX_DET:b * MAX_DET + min(int(n), MAX_DET)]
+        rows.append(np.stack([np.full(len(d), b), d["box_index"], d["obj_id"], d["prob"], d["x"], d["y"], d["w"],
+                              d["h"]], axis=1).astype(np.float64))
+    det = np.concatenate(rows)
+    keep = (DUMP_MAX_BYTES - counts.nbytes - 1024) // (det.itemsize * 8)  # 1 KB for the two .npy headers
+    if len(det) > keep:
+        det = det[np.sort(np.random.default_rng(0).choice(len(det), keep, replace=False))]
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "counts.npy", counts)
+    np.save(out / "detections.npy", det)
+
+
 def run_reference(args) -> int:
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -261,9 +290,13 @@ def main() -> int:
     ap.add_argument("--batch", type=int, default=BATCH)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-out", default=None, help="write the per-layer timing table (json) here")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the detections of the last timed step as DIR/<name>.npy (rank 0's batch)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 20 if args.impl == "reference" else 300
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup is None:
         args.warmup = 3 if args.impl == "reference" else 30
     if args.impl == "reference":
@@ -407,6 +440,8 @@ def main() -> int:
     if rank == 0:
         sampler.start()
     ms_dev = timed(lambda: run_device(args.steps), 1)
+    # the steps below reuse dets / counts (the uint8 pipeline on other images): keep this step's result now
+    last_dets, last_counts = dets_np.copy(), counts_np.copy()
     sampling = "nvidia-smi -lms 100 over the timed region"
     if ms_dev < 400.0:
         # a short timed region (--steps given by the caller): nvidia-smi samples every 100 ms, so keep the same
@@ -596,6 +631,8 @@ def main() -> int:
     if rank == 0:
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(tmp)
+        if args.dump_outputs:  # before the bench line: a dump that cannot be written fails the run with no line out
+            dump_outputs(Path(args.dump_outputs), last_dets, last_counts)
         _emit(line)
         if args.profile_out:
             Path(args.profile_out).write_text(json.dumps({"batch": B, "layers": table, "line": line}, indent=1))

@@ -1,6 +1,7 @@
-"""Parity at the batch sizes BASELINE.json states, EVERY image, against the reference's own CPU forward
-(oracle/_ref/darknet_ref, compiled from the reference sources; call sequence of detector.c:454-512), plus the
-end-to-end detection agreement:
+"""Parity at the batch sizes BASELINE.json states, EVERY image, against the reference's CPU forward (call sequence
+of detector.c:454-512; ref_util.checker_bin: the compiled reference oracle/_ref/darknet_ref where present, else the
+oracle port oracle/y2_oracle.c, which tests/test_oracle_golden.py pins bit for bit to stored reference outputs of every
+layer type these cfgs use), plus the end-to-end detection agreement:
 
   * every dumped layer and the network output, all images of the batch:
       max|a-b| / max|b|  over the batch       <= 1e-2   (bf16 operands, fp32 accumulate: the north star's bf16 bound),
@@ -81,8 +82,7 @@ CASES = [
 @pytest.mark.timeout(1500)
 @pytest.mark.parametrize("name,side,batch,head_gain,thresh", CASES)
 def test_every_image_of_a_baseline_batch_matches_the_reference(tmp_path, name, side, batch, head_gain, thresh):
-    if not R.have_ref():
-        pytest.skip("oracle/_ref/darknet_ref not built")
+    checker = R.checker_bin()
     nms = 0.4
     kw = {}
     if name == "yolo9000":
@@ -100,7 +100,7 @@ def test_every_image_of_a_baseline_batch_matches_the_reference(tmp_path, name, s
     # layers above 400 MB per batch (the first two or three full-resolution tensors) are not dumped: they are
     # covered image by image at small batch in test_network_gpu.py and by the kernel tests at batch 64
     ref_dir.mkdir()
-    R.run_raw([R.REF_BIN, "forward", cfg, weights, inp, ref_dir, thresh or 0.24, nms, 1],
+    R.run_raw([checker, "forward", cfg, weights, inp, ref_dir, thresh or 0.24, nms, 1],
               env={"Y2_DUMP_MAX_MB": "400", "OMP_NUM_THREADS": str(os.cpu_count())})
 
     dn.set_gpu_index(0)
@@ -164,7 +164,7 @@ def test_every_image_of_a_baseline_batch_matches_the_reference(tmp_path, name, s
     rcfg = tmp_path / "region_only.cfg"  # the region layer alone: no need to allocate the whole detector again
     rcfg.write_text(synth.region_only_cfg(batch, lr_w, lr_h, anchors, classes_, num,
                                           f"tree={kw['tree']}\n" if "tree" in kw else ""))
-    R.region(R.REF_BIN, rcfg, rin, own_dir, thresh=thresh, nms=nms, cwd=tmp_path)
+    R.region(checker, rcfg, rin, own_dir, thresh=thresh, nms=nms, cwd=tmp_path)
     want = _dets_by_image(R.load(own_dir, "dets.f32"), batch)
     n_exact = 0
     for b in range(batch):
