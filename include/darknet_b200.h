@@ -353,7 +353,7 @@ void predict_classifier(char *datacfg, char *cfgfile, char *weightfile, char *fi
 void predict_classifier_image(network net, image im, char **names, int top, FILE *out); /* the lines for one image */
 
 /* =========================================================================================
- * B200 extensions (not in the reference): batched, device-resident detection.
+ * B200 extensions (not in the reference): batched, device-resident detection and classification.
  * ========================================================================================= */
 
 typedef struct y2_detection {
@@ -413,6 +413,38 @@ int network_detect_submit_frames(network net, const unsigned char *frames_hwc, i
                                  float thresh, float nms, int max_det);
 void network_detect_batch_frames(network net, const unsigned char *frames_hwc, int frame_w, int frame_h,
                                  float thresh, float nms, y2_detection *dets, int *counts, int max_det);
+/* ---- batched, device-resident classification: letterbox, forward pass, WordTree products and top-k run on the
+ * device and only `top` (index, probability) pairs per image come back, equal to what predict_classifier_image
+ * computes on the host (classifier.c:676-730: letterbox_image, network_predict, hierarchy_predictions for a WordTree
+ * classifier, top_k).  The network's output layer must be a class vector (softmax, avgpool, connected or dropout;
+ * a region network uses network_detect_*), 1 <= top <= min(outputs, Y2_CLASSIFY_MAX_TOP = 128), and a WordTree must list
+ * every parent before its children and be at most 64 levels deep.  hits: [batch][top], best first, in top_k's order (which also decides which of
+ * several equal probabilities are kept).  A NaN in the output ranks below every number. */
+#ifndef Y2_CLASS_HIT_DEFINED
+#define Y2_CLASS_HIT_DEFINED
+typedef struct y2_class_hit {
+    int index;
+    float prob;
+} y2_class_hit;
+#endif
+/* top-k (and the WordTree products) of the last forward pass (network_forward_device) */
+void network_classify_device(network net, int top, y2_class_hit *hits);
+/* upload + forward + classify of `batch` prepared images (fp32 planar CHW, already letterboxed), one synchronisation */
+void network_classify_batch(network net, const float *input, int top, y2_class_hit *hits);
+/* Decoded frames of any size, uint8 interleaved RGB [batch][frame_h][frame_w][3]: byte/255. and letterbox_image
+ * (image.c:1624-1644) run on the device, bit-identical to the host chain.  Frames at the network's size take the
+ * uint8 first-layer path when the network has one (letterbox is the identity there). */
+void network_classify_batch_frames(network net, const unsigned char *frames_hwc, int frame_w, int frame_h, int top,
+                                   y2_class_hit *hits);
+/* The submit/wait pipeline of network_detect_submit* for classification: the same two slots, staging buffers
+ * (network_pipeline_staging, _u8, _frames) and device inputs (network_pipeline_input_device).  Detection and
+ * classification batches may be interleaved; each wait must match the kind of the OLDEST batch in flight, and
+ * network_classify_wait's top must be the one that batch was submitted with. */
+int network_classify_submit(network net, const float *input, int top);
+int network_classify_submit_u8(network net, const unsigned char *input_hwc, int top);
+int network_classify_submit_frames(network net, const unsigned char *frames_hwc, int frame_w, int frame_h, int top);
+int network_classify_submit_resident(network net, int top);
+int network_classify_wait(network net, y2_class_hit *hits, int top);
 /* ---- the same over several GPUs of one box from ONE caller (one replica and one host thread per GPU; idiom of
  * train_networks, network_kernels.cu:346-376).  Replica i owns the next nets[i].batch images of the global batch;
  * detections land in the caller's arrays in image order - nothing else crosses GPUs. ------------------------- */
@@ -443,7 +475,7 @@ int network_launch_count(network net);
 int network_profile_layers(network net, float *ms_per_layer, int n);
 /* 1 -> run layers eagerly instead of replaying the captured CUDA graph */
 void network_set_eager(network net, int eager);
-/* sizeof(layer|network|network_state|y2_detection|box) for what = 0..4: lets a binding that
+/* sizeof(layer|network|network_state|y2_detection|box|y2_class_hit) for what = 0..5: lets a binding that
  * passes these structs by value check its mirror against the library it loaded. */
 size_t y2_abi_sizeof(int what);
 

@@ -188,6 +188,19 @@ int y2_gather_rows_f32(const float *src, void *dst, int batch, int c, int h, int
 int y2_resize_u8_to_f32(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w,
                         int h, y2_stream_t s);
 
+/* letterbox_image's geometry (image.c:1624-1644): the src_w x src_h image scaled to fit inside w x h keeping
+ * its aspect ratio - the side that limits (compared as (float)w / src_w < (float)h / src_h) gets the target
+ * extent, the other src_h*w/src_w resp. src_w*h/src_h in integer arithmetic - placed at
+ * ((w - new_w) / 2, (h - new_h) / 2).  new_w or new_h can be 0 (a very thin image): nothing is placed. */
+void y2_letterbox_geometry(int src_w, int src_h, int w, int h, int *new_w, int *new_h, int *dx, int *dy);
+/* Decoded frames -> letterboxed network input: uint8 interleaved RGB [B][src_h][src_w][3] -> fp32 planar
+ * [B][3][h][w], bit-identical to letterbox_image(im, w, h) (image.c:1624-1644) of the (float)(byte / 255.) image:
+ * resize_image into the window of y2_letterbox_geometry, .5f everywhere else.  A window 1 pixel wide takes
+ * resize_image's edge column.  A window 1 pixel high has no defined result: resize_image's vertical scale
+ * divides by zero there and the host code reads outside its image. */
+int y2_letterbox_u8_to_f32(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w, int h,
+                           y2_stream_t s);
+
 /* bf16 padded NHWC slice -> fp32 NCHW [B][C][H][W] (host-visible l.output layout). */
 int y2_unpack_to_nchw_f32(const void *src, float *dst, int batch, int c, int h, int w,
                           int cs, y2_stream_t s);
@@ -313,6 +326,25 @@ int y2_softmax_rows(const float *in, float *out, int rows, int n, float temp,
 /* softmax_tree of a [softmax] layer with tree= (softmax_layer.c:35-47): per row, one softmax per WordTree group */
 int y2_softmax_tree_rows(const float *in, float *out, int rows, int n, float temp, int n_groups,
                          const int *d_group_size, const int *d_group_offset, y2_stream_t s);
+/* hierarchy_predictions (tree.c:37-51, only_leaves = 0) + top_k (utils.c:179-193) per row of a classifier's
+ * output: row b is out[b * row_stride .. + n).  With d_tree_parent (parent[n], every parent before its child, at
+ * most Y2_CLASSIFY_MAX_TREE_DEPTH levels from a root to a leaf; -1 for a root) the WordTree products are formed first, in scratch: `out` is not modified.  hits[b][top] gets the
+ * `top` largest entries in descending order, exactly top_k's result on a NaN-free row, including which of several
+ * equal values it keeps and in which order (+0 and -0 are equal).  A NaN ranks below every number, so a row with
+ * NaNs still gives `top` distinct valid indices, the numbers first.
+ * 1 <= top <= min(n, Y2_CLASSIFY_MAX_TOP), n <= Y2_CLASSIFY_MAX_N. */
+#define Y2_CLASSIFY_MAX_TOP 128
+#define Y2_CLASSIFY_MAX_N 32768
+#define Y2_CLASSIFY_MAX_TREE_DEPTH 64
+#ifndef Y2_CLASS_HIT_DEFINED
+#define Y2_CLASS_HIT_DEFINED
+typedef struct y2_class_hit {
+    int index;
+    float prob;
+} y2_class_hit;
+#endif
+int y2_classify_topk(const float *out, int row_stride, int batch, int n, int top, const int *d_tree_parent,
+                     y2_class_hit *hits, y2_stream_t s);
 /* shortcut (replaces shortcut_layer.c:54-59 copy_ongpu + shortcut_gpu (blas_kernels.cu:618-651)
  * + activate_array_ongpu): out = act(in + add sampled per blas.c:57-81).  in/out: bf16 padded
  * NHWC of extent out_h x out_w, out_cpad stored channels (out_c real); add: the `from` layer. */

@@ -288,8 +288,11 @@ __device__ __forceinline__ float resize_part(const unsigned char *__restrict__ r
     return __fadd_rn(a, b);
 }
 
+// The resized image fills the window [dx, dx+nw) x [dy, dy+nh) of the w x h canvas and the rest is .5f: the whole
+// canvas for resize_image, the centred window of letterbox_image (image.c:1624-1644: fill_image(.5) + embed_image).
 __global__ void resize_u8_to_f32_kernel(const unsigned char *__restrict__ src, float *__restrict__ dst, int batch,
-                                        int sw, int sh, int w, int h, float w_scale, float h_scale)
+                                        int sw, int sh, int w, int h, int dx, int dy, int nw, int nh, float w_scale,
+                                        float h_scale)
 {
     __shared__ float lut[256];
     for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = (float)((double)(float)i / 255.);
@@ -297,20 +300,24 @@ __global__ void resize_u8_to_f32_kernel(const unsigned char *__restrict__ src, f
     const long long total = (long long)batch * 3 * h * w;
     for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total;
          t += (long long)gridDim.x * blockDim.x) {
-        const int c = (int)(t % w);
-        const int r = (int)((t / w) % h);
+        const int c = (int)(t % w) - dx;
+        const int r = (int)((t / w) % h) - dy;
+        if (c < 0 || c >= nw || r < 0 || r >= nh) {
+            dst[t] = .5f;
+            continue;
+        }
         const int k = (int)((t / ((long long)w * h)) % 3);
         const int b = (int)(t / ((long long)w * h * 3));
         const unsigned char *img = src + (size_t)b * sh * sw * 3;
         const float sy = __fmul_rn((float)r, h_scale);
         int iy = (int)sy;
         if (iy > sh - 1) iy = sh - 1;
-        const float dy = __fsub_rn(sy, (float)iy);
-        float val = __fmul_rn(__fsub_rn(1.f, dy), resize_part(img + (size_t)iy * sw * 3, lut, sw, w, c, k, w_scale));
-        if (!(r == h - 1 || sh == 1)) {
+        const float fy = __fsub_rn(sy, (float)iy);
+        float val = __fmul_rn(__fsub_rn(1.f, fy), resize_part(img + (size_t)iy * sw * 3, lut, sw, nw, c, k, w_scale));
+        if (!(r == nh - 1 || sh == 1)) {
             int iy1 = iy + 1;
             if (iy1 > sh - 1) iy1 = sh - 1;
-            val = __fadd_rn(val, __fmul_rn(dy, resize_part(img + (size_t)iy1 * sw * 3, lut, sw, w, c, k, w_scale)));
+            val = __fadd_rn(val, __fmul_rn(fy, resize_part(img + (size_t)iy1 * sw * 3, lut, sw, nw, c, k, w_scale)));
         }
         dst[t] = val;
     }
@@ -945,6 +952,20 @@ extern "C" int y2_gather_patches_bf16(const void *in, int in_cs, int cin_pad, in
     return Y2_OK;
 }
 
+// resize_image(byte/255. image, nw, nh) into the window at (dx, dy) of a .5f canvas of w x h
+static int resize_window(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w, int h, int dx,
+                         int dy, int nw, int nh, y2_stream_t s)
+{
+    // image.c:1954-1955: float w_scale = (float)(im.w - 1) / (w - 1)  (w == 1 divides by zero there too)
+    const float w_scale = (float)(src_w - 1) / (nw - 1);
+    const float h_scale = (float)(src_h - 1) / (nh - 1);
+    const long long total = (long long)batch * 3 * h * w;
+    resize_u8_to_f32_kernel<<<grid_for(total, 256), 256, 0, to_stream(s)>>>(src, dst, batch, src_w, src_h, w, h, dx,
+                                                                            dy, nw, nh, w_scale, h_scale);
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
+}
+
 extern "C" int y2_resize_u8_to_f32(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w,
                                    int h, y2_stream_t s)
 {
@@ -952,14 +973,32 @@ extern "C" int y2_resize_u8_to_f32(const unsigned char *src, float *dst, int bat
         set_error("y2_resize_u8_to_f32: invalid arguments (%dx%d -> %dx%d)", src_w, src_h, w, h);
         return Y2_EINVAL;
     }
-    // image.c:1954-1955: float w_scale = (float)(im.w - 1) / (w - 1)  (w == 1 divides by zero there too)
-    const float w_scale = (float)(src_w - 1) / (w - 1);
-    const float h_scale = (float)(src_h - 1) / (h - 1);
-    const long long total = (long long)batch * 3 * h * w;
-    resize_u8_to_f32_kernel<<<grid_for(total, 256), 256, 0, to_stream(s)>>>(src, dst, batch, src_w, src_h, w, h,
-                                                                            w_scale, h_scale);
-    Y2_LAUNCH_CHECK();
-    return Y2_OK;
+    return resize_window(src, dst, batch, src_w, src_h, w, h, 0, 0, w, h, s);
+}
+
+extern "C" void y2_letterbox_geometry(int src_w, int src_h, int w, int h, int *new_w, int *new_h, int *dx, int *dy)
+{
+    if (((float)w / src_w) < ((float)h / src_h)) {
+        *new_w = w;
+        *new_h = (src_h * w) / src_w;
+    } else {
+        *new_h = h;
+        *new_w = (src_w * h) / src_h;
+    }
+    *dx = (w - *new_w) / 2;
+    *dy = (h - *new_h) / 2;
+}
+
+extern "C" int y2_letterbox_u8_to_f32(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w,
+                                      int h, y2_stream_t s)
+{
+    if (!src || !dst || batch <= 0 || src_w <= 0 || src_h <= 0 || w <= 0 || h <= 0) {
+        set_error("y2_letterbox_u8_to_f32: invalid arguments (%dx%d -> %dx%d)", src_w, src_h, w, h);
+        return Y2_EINVAL;
+    }
+    int nw, nh, dx, dy;
+    y2_letterbox_geometry(src_w, src_h, w, h, &nw, &nh, &dx, &dy);
+    return resize_window(src, dst, batch, src_w, src_h, w, h, dx, dy, nw, nh, s);
 }
 
 extern "C" int y2_unpack_to_nchw_f32(const void *src, float *dst, int batch, int c, int h, int w, int cs,

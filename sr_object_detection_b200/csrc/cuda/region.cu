@@ -313,6 +313,34 @@ __global__ void region_boxes_flat_kernel(const float *__restrict__ pred, const f
 }
 
 // ---------------------------------------------------------------------------------
+// hierarchy_predictions (tree.c:37-51, only_leaves = 0) by one block: hv[j] = x[j] * hv[parent[j]], parents
+// precede children.  Walked in chunks of blockDim classes: a node climbs only to its first ancestor BELOW the
+// chunk, whose value is final, and multiplies back down in the reference's association (a WordTree is nearly
+// breadth-first, so that is one or two steps instead of the whole path to the root).  Every thread of the block
+// calls it; it ends with a __syncthreads, so hv is complete on return.  A node climbs at most 64 steps: trees
+// deeper than 64 levels are not supported (the classify entries refuse them at plan time).
+// ---------------------------------------------------------------------------------
+__device__ __forceinline__ void hierarchy_walk(const float *x, float *hv, const int *__restrict__ parent, int classes)
+{
+    for (int base = 0; base < classes; base += blockDim.x) {
+        const int j = base + threadIdx.x;
+        if (j < classes) {
+            int path[64];
+            int depth = 0;
+            int c = j;
+            while (c >= base && depth < 64) {
+                path[depth++] = c;
+                c = parent[c];
+            }
+            float v = (c >= 0) ? hv[c] : 1.f;  // x * 1.f is exact: a root keeps its own value
+            for (int d = depth - 1; d >= 0; --d) v = x[path[d]] * v;
+            hv[j] = v;
+        }
+        __syncthreads();
+    }
+}
+
+// ---------------------------------------------------------------------------------
 // get_region_boxes, softmax-tree variants (region_layer.c:349-366).  One block per box:
 // the class scores are staged in shared memory, hierarchy_predictions is evaluated per
 // node by walking to the root and multiplying back down (float multiply commutes, so
@@ -342,26 +370,7 @@ __global__ void __launch_bounds__(1024) region_boxes_tree_kernel(float *__restri
         __syncthreads();
         float scale = x[4];
         if (classfix == -1 && scale < .5) scale = 0;
-        // hierarchy_predictions (tree.c:37-51): v[j] = x[j] * v[parent[j]], parents precede children.  Walked
-        // in chunks of blockDim classes: a node climbs only to its first ancestor BELOW the chunk, whose value
-        // is final, and multiplies back down in the reference's association (a WordTree is nearly
-        // breadth-first, so that is one or two steps instead of the whole path to the root).
-        for (int base = 0; base < classes; base += blockDim.x) {
-            const int j = base + threadIdx.x;
-            if (j < classes) {
-                int path[64];
-                int depth = 0;
-                int c = j;
-                while (c >= base && depth < 64) {
-                    path[depth++] = c;
-                    c = parent[c];
-                }
-                float v = (c >= 0) ? hv[c] : 1.f;  // x * 1.f is exact: a root keeps its own value
-                for (int d = depth - 1; d >= 0; --d) v = sx[path[d]] * v;
-                hv[j] = v;
-            }
-            __syncthreads();
-        }
+        hierarchy_walk(sx, hv, parent, classes);
         float *pr = probs + bi * out_classes;
         if (map) {
             for (int j = threadIdx.x; j < classes; j += blockDim.x) x[5 + j] = hv[j];
@@ -950,6 +959,132 @@ __global__ void softmax_tree_rows_kernel(const float *__restrict__ in, float *__
     }
 }
 
+// ---------------------------------------------------------------------------------
+// classifier tail (classifier.c:676-730 after network_predict): hierarchy_predictions (tree.c:37-51) when a
+// tree is given, then top_k (utils.c:179-193).  One block per image.
+// top_k keeps a list sorted by value; an entry displaces the first list entry it is strictly greater than, and the
+// displaced one moves on down the list the same way.  Among equal values the order therefore depends on the order
+// of arrival (a displaced entry goes behind its equals), so the result is reproduced by running that same loop -
+// but only over the few entries that can matter: the values above the top-th largest value T, and the first `top`
+// entries equal to T.  An entry equal to T that comes later finds the list full of values >= T and changes
+// nothing; an entry below T never changes where the entries >= T end up.
+// Every entry gets the distinct 47-bit key (order(value) << 15) | (32767 - index); the m = 2*top-1 largest keys
+// hold all entries above T and at least `top` entries equal to T, lowest indices first (or, when there are fewer,
+// some below T, which is harmless).  A radix select over 8-bit digits finds the m-th largest key; those m entries,
+// in index order, go through top_k's loop on one thread, comparing order(value): +0 and -0 are equal and a NaN
+// is below every number.
+// ---------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned topk_order(float v)
+{
+    if (v != v) return 0u;                                   // NaN: below every number
+    const unsigned u = __float_as_uint(v == 0.f ? 0.f : v);  // -0 ties with +0
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+__device__ __forceinline__ unsigned long long topk_key(float v, int j)
+{
+    return ((unsigned long long)topk_order(v) << 15) | (unsigned)(32767 - j);
+}
+
+__global__ void __launch_bounds__(1024) classify_topk_kernel(const float *__restrict__ out, int row_stride, int batch,
+                                                             int n, int top, const int *__restrict__ parent,
+                                                             y2_class_hit *__restrict__ hits)
+{
+    extern __shared__ float val[]; // [n]: the row, after hierarchy_predictions
+    __shared__ unsigned hist[256];
+    __shared__ unsigned long long cand[2 * Y2_CLASSIFY_MAX_TOP - 1];
+    __shared__ unsigned ck[2 * Y2_CLASSIFY_MAX_TOP - 1];  // candidates in index order: order(value), index
+    __shared__ int ci[2 * Y2_CLASSIFY_MAX_TOP - 1];
+    __shared__ int lst[Y2_CLASSIFY_MAX_TOP];
+    __shared__ unsigned s_digit, s_remaining;
+    __shared__ int s_count;
+    const int lane = threadIdx.x & 31;
+    const int m = (2 * top - 1 < n) ? 2 * top - 1 : n;
+    for (int b = blockIdx.x; b < batch; b += gridDim.x) {
+        const float *row = out + (size_t)b * row_stride;
+        if (parent) {
+            hierarchy_walk(row, val, parent, n);
+        } else {
+            for (int j = threadIdx.x; j < n; j += blockDim.x) val[j] = row[j];
+            __syncthreads();
+        }
+        unsigned long long prefix = 0, mask = 0;
+        unsigned remaining = (unsigned)m;
+        for (int shift = 40; shift >= 0; shift -= 8) {
+            for (int i = threadIdx.x; i < 256; i += blockDim.x) hist[i] = 0;
+            __syncthreads();
+            for (int base = 0; base < n; base += blockDim.x) {
+                const int j = base + threadIdx.x;
+                unsigned bin = 256; // not counted
+                if (j < n) {
+                    const unsigned long long k = topk_key(val[j], j);
+                    if ((k & mask) == prefix) bin = (unsigned)(k >> shift) & 255u;
+                }
+                const unsigned peers = __match_any_sync(0xffffffffu, bin);
+                if (bin < 256 && lane == __ffs(peers) - 1) atomicAdd(&hist[bin], __popc(peers));
+            }
+            __syncthreads();
+            if (threadIdx.x < 32) {
+                // lane l owns digits 255-8l down to 248-8l; the lane in which the count from the top reaches
+                // `remaining` picks the digit
+                unsigned own = 0;
+                for (int q = 0; q < 8; ++q) own += hist[255 - 8 * lane - q];
+                unsigned incl = own;
+                for (int o = 1; o < 32; o <<= 1) {
+                    const unsigned t = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += t;
+                }
+                unsigned cum = incl - own;
+                if (cum < remaining && incl >= remaining) {
+                    int d = 255 - 8 * lane;
+                    while (cum + hist[d] < remaining) cum += hist[d--];
+                    s_digit = (unsigned)d;
+                    s_remaining = remaining - cum;
+                }
+            }
+            __syncthreads();
+            prefix |= (unsigned long long)s_digit << shift;
+            mask |= 255ull << shift;
+            remaining = s_remaining;
+        }
+        // prefix is now the m-th largest key: exactly m keys are >= prefix
+        if (threadIdx.x == 0) s_count = 0;
+        __syncthreads();
+        for (int j = threadIdx.x; j < n; j += blockDim.x) {
+            const unsigned long long k = topk_key(val[j], j);
+            if (k >= prefix) cand[atomicAdd(&s_count, 1)] = k;
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < m; i += blockDim.x) { // sort the candidates by index
+            const int j = 32767 - (int)(cand[i] & 32767u);
+            int rank = 0;
+            for (int q = 0; q < m; ++q) rank += (32767 - (int)(cand[q] & 32767u)) < j;
+            ck[rank] = (unsigned)(cand[i] >> 15);
+            ci[rank] = j;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) { // utils.c:179-193 over the candidates
+            for (int j = 0; j < top; ++j) lst[j] = -1;
+            for (int c = 0; c < m; ++c) {
+                int cur = c;
+                for (int j = 0; j < top && cur >= 0; ++j) {
+                    if (lst[j] < 0 || ck[cur] > ck[lst[j]]) {
+                        const int displaced = lst[j];
+                        lst[j] = cur;
+                        cur = displaced;
+                    }
+                }
+            }
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < top; i += blockDim.x) {
+            const int j = ci[lst[i]];
+            hits[(size_t)b * top + i] = y2_class_hit{j, val[j]};
+        }
+        __syncthreads();
+    }
+}
+
 static inline int grid_cap(long long blocks, int per_sm)
 {
     long long cap = (long long)sm_count() * per_sm;
@@ -1012,11 +1147,12 @@ extern "C" int y2_region_boxes_counted(float *pred, const float *d_biases, float
             return Y2_EINVAL;
         }
         const size_t smem = (size_t)classes * 2 * sizeof(float);
-        // the attribute is per device: a second network on another GPU needs it raised there too
+        // the attribute is per device: a second network on another GPU needs it raised there too.  Raised whatever
+        // the size: the kernel's static shared memory counts against the 48 KB default as well
         static bool attr_done[64] = {false};
         int dev = 0;
         Y2_CUDA_CHECK(cudaGetDevice(&dev));
-        if (smem > 48 * 1024 && (dev < 0 || dev >= 64 || !attr_done[dev])) {
+        if (dev < 0 || dev >= 64 || !attr_done[dev]) {
             Y2_CUDA_CHECK(cudaFuncSetAttribute(region_boxes_tree_kernel,
                                                cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
             if (dev >= 0 && dev < 64) attr_done[dev] = true;
@@ -1036,6 +1172,31 @@ extern "C" int y2_region_boxes_counted(float *pred, const float *d_biases, float
             pred, d_biases, boxes, probs, batch, lw, lh, n, classes, img_w, img_h, thresh, only_objectness,
             classfix, nz_count);
     }
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
+}
+
+extern "C" int y2_classify_topk(const float *out, int row_stride, int batch, int n, int top,
+                                const int *d_tree_parent, y2_class_hit *hits, y2_stream_t s)
+{
+    if (!out || !hits || batch <= 0 || n <= 0 || n > Y2_CLASSIFY_MAX_N || row_stride < n || top < 1 || top > n ||
+        top > Y2_CLASSIFY_MAX_TOP) {
+        set_error("y2_classify_topk: invalid arguments (n=%d row_stride=%d top=%d)", n, row_stride, top);
+        return Y2_EINVAL;
+    }
+    const size_t smem = (size_t)n * sizeof(float);
+    // raised on every device before its first launch, whatever n: the kernel's static shared memory (histogram and
+    // candidates, ~5.5 KB) counts against the 48 KB default too, so comparing n * 4 alone with 48 KB is not enough
+    static bool attr_done[64] = {false};
+    int dev = 0;
+    Y2_CUDA_CHECK(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64 || !attr_done[dev]) {
+        Y2_CUDA_CHECK(cudaFuncSetAttribute(classify_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           Y2_CLASSIFY_MAX_N * sizeof(float)));
+        if (dev >= 0 && dev < 64) attr_done[dev] = true;
+    }
+    classify_topk_kernel<<<grid_cap(batch, 2), 1024, smem, to_stream(s)>>>(out, row_stride, batch, n, top,
+                                                                          d_tree_parent, hits);
     Y2_LAUNCH_CHECK();
     return Y2_OK;
 }

@@ -1,11 +1,12 @@
 /*
- * Post-processing entry points of the drop-in API and the batched device-resident detection
- * extension.  The arithmetic runs in the region / NMS kernels; these functions only move the
+ * Post-processing entry points of the drop-in API and the batched device-resident detection and
+ * classification extensions.  The arithmetic runs in the region / NMS kernels; these functions only move the
  * caller-owned host arrays (boxes[total], probs[total][classes]) across, as the reference's
  * callers expect (detector.c:486-495, yolo_v2_class.cpp:71-73,215-216).
  *
  * Reference interfaces replaced: get_region_boxes (region_layer.c:328-379), do_nms_sort
- * (box.c:249-277), box_iou & friends (box.c:67-97).
+ * (box.c:249-277), box_iou & friends (box.c:67-97); for classification, the tail of predict_classifier
+ * (classifier.c:676-730: letterbox_image, hierarchy_predictions, top_k).
  */
 #include "y2_host.h"
 
@@ -328,25 +329,15 @@ static void pipe_reserve_frames(y2_net_rt *rt, int s, size_t bytes)
     ps->frames_cap = bytes;
 }
 
-/* input: fp32 planar [B][c][h][w] (u8 == 0), uint8 interleaved RGB [B][h][w][3] at the network's
- * resolution (u8 == 1), uint8 interleaved RGB frames [B][fh][fw][3] of any size (u8 == 2), or nothing: the slot's
- * device input already holds the batch (u8 == 3, network_detect_submit_resident) */
-static int submit_common(network net, const void *input, int u8, int fw, int fh, float thresh, float nms,
-                         int max_det)
+/* The input half of a submission, into slot s: the staging copy, the H2D copy on the copy stream, resize (or
+ * letterbox) and the forward pass on the network's stream.  input: fp32 planar [B][c][h][w] (u8 == 0), uint8
+ * interleaved RGB [B][h][w][3] at the network's resolution (u8 == 1), uint8 interleaved RGB frames [B][fh][fw][3]
+ * of any size (u8 == 2), or nothing: the slot's device input already holds the batch (u8 == 3, *_submit_resident) */
+static void submit_input(network net, int s, const void *input, int u8, int fw, int fh, int letterbox)
 {
     y2_net_rt *rt = y2_rt(net);
-    if (!rt) error("network_detect_submit: network has no device plan");
-    if (net.batch != rt->plan_batch) error("network batch changed without set_batch_network");
-    if (u8 == 1) pipe_init_u8(net);
-    else pipe_init(net);
-    if (u8 == 2 && (net.c != 3 || fw <= 0 || fh <= 0)) error("network_detect_submit_frames: needs 3-channel input and a frame size");
-    if (rt->pipe_inflight >= 2) error("network_detect_submit: two batches already in flight, call network_detect_wait");
-    Y2_CHECK(y2_set_device(rt->device));
-    const int s = (rt->pipe_head + rt->pipe_inflight) & 1;
     struct y2_pipe_slot *ps = &rt->pipe[s];
-    layer *l = region_of(net);
     const int B = net.batch;
-    pipe_reserve_dets(rt, s, B, max_det);
     /* pageable caller memory is staged through the slot's pinned buffer (a host copy; fill the slot's
      * staging buffer directly to avoid it) */
     if (u8 == 2) {
@@ -367,7 +358,9 @@ static int submit_common(network net, const void *input, int u8, int fw, int fh,
         Y2_CHECK(y2_event_record(ps->ev_h2d, rt->copy_stream));
         Y2_CHECK(y2_stream_wait_event(rt->stream, ps->ev_h2d));
     }
-    if (u8 == 2) /* byte/255. + resize_image on the device, into the slot's fp32 input */
+    if (u8 == 2 && letterbox) /* byte/255. + letterbox_image on the device, into the slot's fp32 input */
+        Y2_CHECK(y2_letterbox_u8_to_f32(ps->frames_dev, ps->in_dev, B, fw, fh, net.w, net.h, rt->stream));
+    else if (u8 == 2) /* byte/255. + resize_image on the device, into the slot's fp32 input */
         Y2_CHECK(y2_resize_u8_to_f32(ps->frames_dev, ps->in_dev, B, fw, fh, net.w, net.h, rt->stream));
     if (u8 == 1) {
         rt->input_u8 = 1; /* read while the layer list is captured */
@@ -378,16 +371,56 @@ static int submit_common(network net, const void *input, int u8, int fw, int fh,
     } else {
         y2_run_forward_from(net, ps->in_dev, &ps->graph, &ps->graph_valid);
     }
-    detect_tail(rt, l, net.layers[net.n - 2].b200, thresh, nms, ps->det_dev, ps->cnt_dev, ps->det_cap);
-    /* the detection lists travel on their own stream: the next batch's forward pass (same compute stream) does
-     * not wait behind the device -> host copies of this one */
+}
+
+/* checks shared by both kinds of submission; returns the slot the batch goes to */
+static int submit_slot(network net, int u8, int fw, int fh)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network submit: network has no device plan");
+    if (net.batch != rt->plan_batch) error("network batch changed without set_batch_network");
+    if (u8 == 1) pipe_init_u8(net);
+    else pipe_init(net);
+    if (u8 == 2 && (net.c != 3 || fw <= 0 || fh <= 0)) error("network submit of frames: needs 3-channel input and a frame size");
+    if (rt->pipe_inflight >= 2)
+        error("network submit: two batches already in flight, wait for one first");
+    Y2_CHECK(y2_set_device(rt->device));
+    return (rt->pipe_head + rt->pipe_inflight) & 1;
+}
+
+/* the tail half's results travel on their own stream: the next batch's forward pass (same compute stream) does not
+ * wait behind the device -> host copies of this one */
+static void submit_results(y2_net_rt *rt, int s)
+{
+    struct y2_pipe_slot *ps = &rt->pipe[s];
     Y2_CHECK(y2_event_record(ps->ev_tail, rt->stream));
     Y2_CHECK(y2_stream_wait_event(rt->d2h_stream, ps->ev_tail));
-    Y2_CHECK(y2_memcpy_d2h(ps->cnt_pinned, ps->cnt_dev, (size_t)B * sizeof(int), rt->d2h_stream));
-    Y2_CHECK(y2_memcpy_d2h(ps->det_pinned, ps->det_dev, (size_t)B * ps->det_cap * sizeof(y2_det), rt->d2h_stream));
+}
+
+static void submit_done(y2_net_rt *rt, int s, int kind)
+{
+    struct y2_pipe_slot *ps = &rt->pipe[s];
     Y2_CHECK(y2_event_record(ps->ev_done, rt->d2h_stream));
+    ps->kind = kind;
     ps->busy = 1;
     rt->pipe_inflight++;
+}
+
+static int submit_common(network net, const void *input, int u8, int fw, int fh, float thresh, float nms,
+                         int max_det)
+{
+    const int s = submit_slot(net, u8, fw, fh);
+    y2_net_rt *rt = y2_rt(net);
+    struct y2_pipe_slot *ps = &rt->pipe[s];
+    layer *l = region_of(net);
+    const int B = net.batch;
+    pipe_reserve_dets(rt, s, B, max_det);
+    submit_input(net, s, input, u8, fw, fh, 0);
+    detect_tail(rt, l, net.layers[net.n - 2].b200, thresh, nms, ps->det_dev, ps->cnt_dev, ps->det_cap);
+    submit_results(rt, s);
+    Y2_CHECK(y2_memcpy_d2h(ps->cnt_pinned, ps->cnt_dev, (size_t)B * sizeof(int), rt->d2h_stream));
+    Y2_CHECK(y2_memcpy_d2h(ps->det_pinned, ps->det_dev, (size_t)B * ps->det_cap * sizeof(y2_det), rt->d2h_stream));
+    submit_done(rt, s, Y2_PIPE_DETECT);
     return s;
 }
 
@@ -422,6 +455,8 @@ int network_detect_wait(network net, y2_detection *dets, int *counts, int max_de
     if (!rt || !rt->pipe_ready || rt->pipe_inflight <= 0) error("network_detect_wait: nothing in flight");
     const int s = rt->pipe_head;
     struct y2_pipe_slot *ps = &rt->pipe[s];
+    if (ps->kind != Y2_PIPE_DETECT)
+        error("network_detect_wait: the oldest batch in flight is a classify batch, call network_classify_wait");
     Y2_CHECK(y2_event_sync(ps->ev_done));
     const int B = net.batch;
     for (int b = 0; b < B; ++b) {
@@ -446,6 +481,14 @@ void network_detect_batch_u8(network net, const unsigned char *input_hwc, float 
     network_detect_wait(net, dets, counts, max_det);
 }
 
+/* frames at the network's resolution go to the uint8 first-layer kernel when the network has one */
+static int frames_take_u8(network net, int frame_w, int frame_h)
+{
+    y2_layer_rt *r0 = (y2_layer_rt *)net.layers[0].b200;
+    return frame_w == net.w && frame_h == net.h && r0 && r0->stem_fused && net.c == 3 &&
+           y2_stem_u8_supported(net.h, net.w);
+}
+
 /* Decoded frames of any size: upload the raw bytes, then byte/255. (load_image_stb) and resize_image
  * (image.c:1950-1993) run on the device, bit-identical to Detector::detect(filename)'s host path
  * (yolo_v2_class.cpp:173-206).  Frames already at the network's resolution take the uint8 first-layer
@@ -455,9 +498,7 @@ int network_detect_submit_frames(network net, const unsigned char *frames_hwc, i
 {
     y2_net_rt *rt = y2_rt(net);
     if (!rt) error("network_detect_submit_frames: network has no device plan");
-    y2_layer_rt *r0 = (y2_layer_rt *)net.layers[0].b200;
-    if (frame_w == net.w && frame_h == net.h && r0 && r0->stem_fused && net.c == 3 && y2_stem_u8_supported(net.h, net.w))
-        return submit_common(net, frames_hwc, 1, 0, 0, thresh, nms, max_det);
+    if (frames_take_u8(net, frame_w, frame_h)) return submit_common(net, frames_hwc, 1, 0, 0, thresh, nms, max_det);
     return submit_common(net, frames_hwc, 2, frame_w, frame_h, thresh, nms, max_det);
 }
 
@@ -466,9 +507,7 @@ unsigned char *network_pipeline_staging_frames(network net, int slot, int frame_
     y2_net_rt *rt = y2_rt(net);
     if (!rt || slot < 0 || slot > 1 || frame_w <= 0 || frame_h <= 0)
         error("network_pipeline_staging_frames: bad slot, frame size or unplanned network");
-    y2_layer_rt *r0 = (y2_layer_rt *)net.layers[0].b200;
-    if (frame_w == net.w && frame_h == net.h && r0 && r0->stem_fused && net.c == 3 && y2_stem_u8_supported(net.h, net.w))
-        return network_pipeline_staging_u8(net, slot);
+    if (frames_take_u8(net, frame_w, frame_h)) return network_pipeline_staging_u8(net, slot);
     pipe_init(net);
     Y2_CHECK(y2_set_device(rt->device));
     pipe_reserve_frames(rt, slot, (size_t)rt->cap_batch * frame_h * frame_w * 3);
@@ -482,4 +521,133 @@ void network_detect_batch_frames(network net, const unsigned char *frames_hwc, i
     if (rt && rt->pipe_inflight) error("network_detect_batch_frames: batches of the submit/wait pipeline are in flight");
     network_detect_submit_frames(net, frames_hwc, frame_w, frame_h, thresh, nms, max_det);
     network_detect_wait(net, dets, counts, max_det);
+}
+
+/* ---- batched, device-resident classification (extension) --------------------------------------- */
+/* the output layer the classify entries read, after the checks every entry makes */
+static layer *classify_layer(network net, int top)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network_classify: network has no device plan");
+    if (net.batch != rt->plan_batch) error("network batch changed without set_batch_network");
+    layer *l = &net.layers[y2_output_layer_index(net)];
+    y2_layer_rt *r = (y2_layer_rt *)l->b200;
+    if (l->type == REGION) error("network_classify: the network ends in a region layer, use network_detect_*");
+    if (!r || r->out_kind != Y2_KIND_F32_VEC)
+        error("network_classify: the output layer is not a class vector (softmax, avgpool, connected or dropout)");
+    if (l->outputs > Y2_CLASSIFY_MAX_N) error("network_classify: more outputs than Y2_CLASSIFY_MAX_N");
+    if (top < 1 || top > l->outputs || top > Y2_CLASSIFY_MAX_TOP)
+        error("network_classify: top must be in 1 .. min(outputs, Y2_CLASSIFY_MAX_TOP)");
+    if (net.hierarchy && (l->softmax_tree != net.hierarchy || net.hierarchy->n != l->outputs || !r->tree_parent_dev))
+        error("network_classify: the WordTree must belong to the output softmax layer, list every parent before "
+              "its children and be at most 64 levels deep");
+    return l;
+}
+
+/* hierarchy_predictions (net.hierarchy) + top_k for every image of the batch, on the network's stream. The output
+ * layer's rows are read in place (fp32 [B][out_cs]). */
+static void classify_tail(y2_net_rt *rt, network net, layer *l, int top, y2_class_hit *hits_dev)
+{
+    y2_layer_rt *r = (y2_layer_rt *)l->b200;
+    Y2_CHECK(y2_classify_topk((const float *)r->out, r->out_cs, net.batch, l->outputs, top,
+                              net.hierarchy ? r->tree_parent_dev : 0, hits_dev, rt->stream));
+}
+
+/* grows a [cap_batch][*cap] hit buffer pair to hold `top` hits per image */
+static void reserve_hits(y2_net_rt *rt, y2_class_hit **dev, y2_class_hit **pinned, int *cap, int top)
+{
+    if (*cap >= top && *dev) return;
+    y2_free(*dev);
+    y2_host_free(*pinned);
+    const size_t n = (size_t)rt->cap_batch * top;
+    Y2_CHECK(y2_malloc((void **)dev, n * sizeof(y2_class_hit)));
+    Y2_CHECK(y2_host_alloc((void **)pinned, n * sizeof(y2_class_hit)));
+    *cap = top;
+}
+
+void network_classify_device(network net, int top, y2_class_hit *hits)
+{
+    layer *l = classify_layer(net, top);
+    y2_net_rt *rt = y2_rt(net);
+    Y2_CHECK(y2_set_device(rt->device));
+    reserve_hits(rt, &rt->hits_dev, &rt->hits_pinned, &rt->hits_cap, top);
+    classify_tail(rt, net, l, top, rt->hits_dev);
+    const size_t bytes = (size_t)net.batch * top * sizeof(y2_class_hit);
+    Y2_CHECK(y2_memcpy_d2h(rt->hits_pinned, rt->hits_dev, bytes, rt->stream));
+    Y2_CHECK(y2_stream_sync(rt->stream));
+    memcpy(hits, rt->hits_pinned, bytes);
+}
+
+void network_classify_batch(network net, const float *input, int top, y2_class_hit *hits)
+{
+    classify_layer(net, top);
+    network_upload_input(net, input);
+    network_forward_device(net);
+    network_classify_device(net, top, hits);
+}
+
+static int classify_submit_common(network net, const void *input, int u8, int fw, int fh, int top)
+{
+    layer *l = classify_layer(net, top);
+    const int s = submit_slot(net, u8, fw, fh);
+    y2_net_rt *rt = y2_rt(net);
+    struct y2_pipe_slot *ps = &rt->pipe[s];
+    reserve_hits(rt, &ps->hits_dev, &ps->hits_pinned, &ps->hits_cap, top);
+    submit_input(net, s, input, u8, fw, fh, 1);
+    classify_tail(rt, net, l, top, ps->hits_dev);
+    submit_results(rt, s);
+    Y2_CHECK(y2_memcpy_d2h(ps->hits_pinned, ps->hits_dev, (size_t)net.batch * top * sizeof(y2_class_hit),
+                           rt->d2h_stream));
+    ps->hits_top = top;
+    submit_done(rt, s, Y2_PIPE_CLASSIFY);
+    return s;
+}
+
+int network_classify_submit(network net, const float *input, int top)
+{
+    return classify_submit_common(net, input, 0, 0, 0, top);
+}
+
+int network_classify_submit_u8(network net, const unsigned char *input_hwc, int top)
+{
+    return classify_submit_common(net, input_hwc, 1, 0, 0, top);
+}
+
+/* frames of any size: byte/255. and letterbox_image (image.c:1624-1644) on the device */
+int network_classify_submit_frames(network net, const unsigned char *frames_hwc, int frame_w, int frame_h, int top)
+{
+    if (!y2_rt(net)) error("network_classify_submit_frames: network has no device plan");
+    if (frames_take_u8(net, frame_w, frame_h)) return classify_submit_common(net, frames_hwc, 1, 0, 0, top);
+    return classify_submit_common(net, frames_hwc, 2, frame_w, frame_h, top);
+}
+
+int network_classify_submit_resident(network net, int top)
+{
+    return classify_submit_common(net, 0, 3, 0, 0, top);
+}
+
+int network_classify_wait(network net, y2_class_hit *hits, int top)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt || !rt->pipe_ready || rt->pipe_inflight <= 0) error("network_classify_wait: nothing in flight");
+    const int s = rt->pipe_head;
+    struct y2_pipe_slot *ps = &rt->pipe[s];
+    if (ps->kind != Y2_PIPE_CLASSIFY)
+        error("network_classify_wait: the oldest batch in flight is a detection batch, call network_detect_wait");
+    if (top != ps->hits_top) error("network_classify_wait: top differs from the one the batch was submitted with");
+    Y2_CHECK(y2_event_sync(ps->ev_done));
+    memcpy(hits, ps->hits_pinned, (size_t)net.batch * top * sizeof(y2_class_hit));
+    ps->busy = 0;
+    rt->pipe_head ^= 1;
+    rt->pipe_inflight--;
+    return s;
+}
+
+void network_classify_batch_frames(network net, const unsigned char *frames_hwc, int frame_w, int frame_h, int top,
+                                   y2_class_hit *hits)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (rt && rt->pipe_inflight) error("network_classify_batch_frames: batches of the submit/wait pipeline are in flight");
+    network_classify_submit_frames(net, frames_hwc, frame_w, frame_h, top);
+    network_classify_wait(net, hits, top);
 }

@@ -20,6 +20,7 @@ void y2_fatal(const char *where, int rc);
     } while (0)
 
 enum { Y2_KIND_BF16_PADDED = 0, Y2_KIND_F32_FLAT = 1, Y2_KIND_F32_VEC = 2, Y2_KIND_NONE = 3 };
+enum { Y2_PIPE_DETECT = 0, Y2_PIPE_CLASSIFY = 1 }; /* what a pipeline slot's batch computes */
 
 /* per-layer device plan, owned by net.layers[i].b200 */
 typedef struct y2_layer_rt {
@@ -58,7 +59,7 @@ typedef struct y2_layer_rt {
     int *reorg_table;   /* gather table of the layer (y2_reorg_table) */
     int write_order;    /* 1: this layer's kernel wrote its output last position first (y2_conv_plan_order) */
     float *stream_f32;  /* shortcut layers: fp32 copy of the output [B][H+1][W+1][cpad] (residual stream) */
-    /* region */
+    /* region; softmax with tree= (tree_parent_dev only: set when every parent precedes its child) */
     float *boxes_dev, *probs_dev;
     float *biases_dev;
     int *tree_parent_dev, *group_size_dev, *group_offset_dev, *map_dev;
@@ -94,6 +95,9 @@ typedef struct y2_net_rt {
     y2_det *det_dev, *det_pinned;
     int *cnt_dev, *cnt_pinned;
     int det_cap, det_batch;
+    /* class hits of network_classify_device, room for cap_batch x hits_cap */
+    y2_class_hit *hits_dev, *hits_pinned;
+    int hits_cap;
     float *export_dev;   /* fp32 scratch for layer export */
     size_t export_bytes;
     /* two-deep submit/wait pipeline (network_detect_submit): slot 0 shares in_dev / in_pinned / graph
@@ -114,6 +118,10 @@ typedef struct y2_net_rt {
         /* decoded frames of any size (network_detect_submit_frames): resized on the device into in_dev */
         unsigned char *frames_dev, *frames_pinned;
         size_t frames_cap;
+        int kind;           /* Y2_PIPE_* of the batch in the slot */
+        /* class hits of a classify batch ([B][hits_top]), room for cap_batch x hits_cap */
+        y2_class_hit *hits_dev, *hits_pinned;
+        int hits_cap, hits_top;
     } pipe[2];
     y2_stream_t copy_stream; /* host -> device uploads of the pipeline */
     y2_stream_t d2h_stream;  /* detection lists back to the host, under the next batch's forward pass */

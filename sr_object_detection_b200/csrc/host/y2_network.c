@@ -543,6 +543,8 @@ void y2_unplan_network(network *net)
     y2_host_free(rt->det_pinned);
     y2_free(rt->cnt_dev);
     y2_host_free(rt->cnt_pinned);
+    y2_free(rt->hits_dev);
+    y2_host_free(rt->hits_pinned);
     y2_free(rt->export_dev);
     pipe_free(rt);
     y2_stream_destroy(rt->stream);
@@ -1147,6 +1149,19 @@ void y2_plan_network(network *net)
             tree *t = l->softmax_tree;
             r->group_size_dev = (int *)dev_upload(t->group_size, (size_t)t->groups * sizeof(int));
             r->group_offset_dev = (int *)dev_upload(t->group_offset, (size_t)t->groups * sizeof(int));
+            /* hierarchy_predictions of the classify entries walks parents before children and at most
+             * Y2_CLASSIFY_MAX_TREE_DEPTH levels; the host path takes any tree, so another tree only leaves the
+             * classify entries unavailable */
+            int usable = 1;
+            int *depth = (int *)calloc((size_t)t->n, sizeof(int));
+            for (int j = 0; j < t->n && usable; ++j) {
+                const int p = t->parent[j];
+                if (p >= j) usable = 0;
+                else depth[j] = p < 0 ? 1 : depth[p] + 1;
+                if (depth[j] > Y2_CLASSIFY_MAX_TREE_DEPTH) usable = 0;
+            }
+            free(depth);
+            if (usable) r->tree_parent_dev = (int *)dev_upload(t->parent, (size_t)t->n * sizeof(int));
         } else if (l->type == REGION) {
             const size_t total = (size_t)l->w * l->h * l->n;
             r->probs_classes = l->map ? 200 : l->classes;
@@ -1483,6 +1498,8 @@ static void pipe_free(y2_net_rt *rt)
         y2_host_free(rt->pipe[s].det_pinned);
         y2_free(rt->pipe[s].cnt_dev);
         y2_host_free(rt->pipe[s].cnt_pinned);
+        y2_free(rt->pipe[s].hits_dev);
+        y2_host_free(rt->pipe[s].hits_pinned);
         if (rt->pipe[s].ev_h2d) y2_event_destroy(rt->pipe[s].ev_h2d);
         if (rt->pipe[s].ev_done) y2_event_destroy(rt->pipe[s].ev_done);
         if (rt->pipe[s].ev_tail) y2_event_destroy(rt->pipe[s].ev_tail);
@@ -1564,6 +1581,7 @@ size_t y2_abi_sizeof(int what)
     case 2: return sizeof(network_state);
     case 3: return sizeof(y2_detection);
     case 4: return sizeof(box);
+    case 5: return sizeof(y2_class_hit);
     default: return 0;
     }
 }
@@ -1827,6 +1845,8 @@ void free_network(network net)
         y2_host_free(rt->det_pinned);
         y2_free(rt->cnt_dev);
         y2_host_free(rt->cnt_pinned);
+        y2_free(rt->hits_dev);
+        y2_host_free(rt->hits_pinned);
         y2_free(rt->export_dev);
         pipe_free(rt);
         y2_stream_destroy(rt->stream);

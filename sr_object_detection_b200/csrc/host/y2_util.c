@@ -523,23 +523,16 @@ void embed_image(image source, image dest, int dx, int dy)
         }
 }
 
-/* image.c:1624-1644: scale to fit inside w x h keeping the aspect ratio (integer arithmetic of the
- * reference: the side that limits gets the target extent, the other im.h*w/im.w resp. im.w*h/im.h),
- * centre on a 0.5-grey canvas */
+/* image.c:1624-1644: scale to fit inside w x h keeping the aspect ratio (y2_letterbox_geometry), centre on a
+ * 0.5-grey canvas */
 image letterbox_image(image im, int w, int h)
 {
-    int new_w, new_h;
-    if (((float)w / im.w) < ((float)h / im.h)) {
-        new_w = w;
-        new_h = (im.h * w) / im.w;
-    } else {
-        new_h = h;
-        new_w = (im.w * h) / im.h;
-    }
+    int new_w, new_h, dx, dy;
+    y2_letterbox_geometry(im.w, im.h, w, h, &new_w, &new_h, &dx, &dy);
     image resized = resize_image(im, new_w, new_h);
     image boxed = make_image(w, h, im.c);
     fill_image(boxed, .5f);
-    embed_image(resized, boxed, (w - new_w) / 2, (h - new_h) / 2);
+    embed_image(resized, boxed, dx, dy);
     free_image(resized);
     return boxed;
 }

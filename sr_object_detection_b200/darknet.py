@@ -97,6 +97,11 @@ class Detection(C.Structure):
                 ("prob", C.c_float), ("obj_id", C.c_int), ("box_index", C.c_int)]
 
 
+class ClassHit(C.Structure):
+    """Mirror of `y2_class_hit`: one (index, probability) pair of a classify result."""
+    _fields_ = [("index", C.c_int), ("prob", C.c_float)]
+
+
 class Image(C.Structure):
     _fields_ = [("h", C.c_int), ("w", C.c_int), ("c", C.c_int), ("data", _fp)]
 
@@ -157,6 +162,14 @@ def lib() -> C.CDLL:
         "network_pipeline_staging_frames": (C.POINTER(C.c_ubyte), [Network, i, i, i]),
         "network_detect_submit_frames": (i, [Network, C.POINTER(C.c_ubyte), i, i, f, f, i]),
         "network_detect_batch_frames": (None, [Network, C.POINTER(C.c_ubyte), i, i, f, f, C.POINTER(Detection), _ip, i]),
+        "network_classify_device": (None, [Network, i, C.POINTER(ClassHit)]),
+        "network_classify_batch": (None, [Network, fp, i, C.POINTER(ClassHit)]),
+        "network_classify_batch_frames": (None, [Network, C.POINTER(C.c_ubyte), i, i, i, C.POINTER(ClassHit)]),
+        "network_classify_submit": (i, [Network, fp, i]),
+        "network_classify_submit_u8": (i, [Network, C.POINTER(C.c_ubyte), i]),
+        "network_classify_submit_frames": (i, [Network, C.POINTER(C.c_ubyte), i, i, i]),
+        "network_classify_submit_resident": (i, [Network, i]),
+        "network_classify_wait": (i, [Network, C.POINTER(ClassHit), i]),
         "parse_network_cfg_multi": (C.POINTER(Network), [C.c_char_p, C.c_char_p, _ip, i, i]),
         "free_network_multi": (None, [C.POINTER(Network), i]),
         "network_multi_batch": (i, [C.POINTER(Network), i]),
@@ -210,6 +223,7 @@ def lib() -> C.CDLL:
     assert l.y2_abi_sizeof(1) == C.sizeof(Network), (l.y2_abi_sizeof(1), C.sizeof(Network))
     assert l.y2_abi_sizeof(2) == C.sizeof(NetworkState)
     assert l.y2_abi_sizeof(3) == C.sizeof(Detection)
+    assert l.y2_abi_sizeof(5) == C.sizeof(ClassHit)
     _declared = True
     return l
 
@@ -327,6 +341,53 @@ def network_detect_batch(net: Network, images: np.ndarray | None, thresh: float,
         c = min(counts[b], max_det)
         out.append(arr[b * max_det:b * max_det + c].copy())
     return out, list(counts)
+
+
+def _hits_arrays(hits, batch: int, top: int):
+    arr = np.ctypeslib.as_array(hits).reshape(batch, top)
+    return arr["index"].astype(np.int32), arr["prob"].astype(np.float32)
+
+
+def _as_u8(a: np.ndarray):
+    assert a.dtype == np.uint8 and a.flags["C_CONTIGUOUS"]
+    return a.ctypes.data_as(C.POINTER(C.c_ubyte))
+
+
+def network_classify_batch(net: Network, images: np.ndarray | None = None, frames: np.ndarray | None = None,
+                           top: int = 5):
+    """Extension: batched forward + WordTree products + top-k on the device.  images: prepared fp32 [B][C][H][W]
+    (already letterboxed); frames: uint8 RGB [B][fh][fw][3] of any size, letterboxed on the device; neither: the
+    last forward pass.  Returns (indices int32 [B][top], probs float32 [B][top]), best first."""
+    hits = (ClassHit * (net.batch * top))()
+    if frames is not None:
+        assert frames.ndim == 4 and frames.shape[0] == net.batch and frames.shape[3] == 3, frames.shape
+        lib().network_classify_batch_frames(net, _as_u8(frames), frames.shape[2], frames.shape[1], top, hits)
+    elif images is not None:
+        assert images.size == net.batch * net.inputs, (images.shape, net.batch, net.inputs)
+        lib().network_classify_batch(net, _as_fp(images), top, hits)
+    else:
+        lib().network_classify_device(net, top, hits)
+    return _hits_arrays(hits, net.batch, top)
+
+
+def network_classify_submit(net: Network, images: np.ndarray | None = None, frames: np.ndarray | None = None,
+                            u8: np.ndarray | None = None, top: int = 5) -> int:
+    """Queue one batch on the submit/wait pipeline: prepared fp32 images, frames of any size, uint8 images at the
+    network size (u8), or none of them (the slot's device input already holds the batch).  Returns the slot."""
+    if frames is not None:
+        return lib().network_classify_submit_frames(net, _as_u8(frames), frames.shape[2], frames.shape[1], top)
+    if u8 is not None:
+        return lib().network_classify_submit_u8(net, _as_u8(u8), top)
+    if images is not None:
+        return lib().network_classify_submit(net, _as_fp(images), top)
+    return lib().network_classify_submit_resident(net, top)
+
+
+def network_classify_wait(net: Network, top: int = 5):
+    """The oldest classify batch in flight: (indices int32 [B][top], probs float32 [B][top])."""
+    hits = (ClassHit * (net.batch * top))()
+    lib().network_classify_wait(net, hits, top)
+    return _hits_arrays(hits, net.batch, top)
 
 
 class _DevBuf:

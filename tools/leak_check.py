@@ -1,5 +1,6 @@
 #!/usr/bin/env python
-"""Developer tool (GPU box): device-memory leak check - parse / predict / detect / resize / free in a loop."""
+"""Developer tool (GPU box): device-memory leak check - parse / predict / detect / resize / free in a loop, and
+parse / classify / change the batch / free for a classifier."""
 import sys
 import tempfile
 from pathlib import Path
@@ -41,12 +42,34 @@ def cycle(name, side, batch):
     dn.free_network(net)
 
 
-for name, side, batch in (("tiny-yolo-voc", 416, 8), ("yolo-voc", 416, 64)):
-    cycle(name, side, batch)  # warm: allocator pools, per-device scratch
+def classify_cycle(name, side, batch):
+    text = synth.CFGS[name](batch=batch, w=side, h=side)
+    (tmp / "c.cfg").write_text(text)
+    w = tmp / f"{name}.weights"
+    if not w.exists():
+        synth.write_weights(w, text, seed=1234)
+    net = dn.parse_network_cfg(tmp / "c.cfg")
+    dn.load_weights(net, w)
+    frames = np.random.default_rng(1).integers(0, 256, size=(batch, 375, 500, 3), dtype=np.uint8)
+    dn.network_classify_batch(net, frames=frames, top=5)
+    lib = dn.lib()
+    for _ in range(2):  # two batches in flight, then drain
+        slot = lib.network_pipeline_next_slot(net)
+        lib.network_classify_submit_frames(net, lib.network_pipeline_staging_frames(net, slot, 500, 375), 500, 375, 5)
+    dn.network_classify_wait(net, top=5)
+    dn.network_classify_wait(net, top=5)
+    dn.set_batch_network(net, max(1, batch // 2))
+    dn.network_classify_batch(net, frames=np.ascontiguousarray(frames[:max(1, batch // 2)]), top=5)
+    dn.free_network(net)
+
+
+for fn, name, side, batch in ((cycle, "tiny-yolo-voc", 416, 8), (cycle, "yolo-voc", 416, 64),
+                              (classify_cycle, "darknet19_448", 448, 16)):
+    fn(name, side, batch)  # warm: allocator pools, per-device scratch
     torch.cuda.synchronize()
     free0, _ = torch.cuda.mem_get_info()
     for _ in range(15):
-        cycle(name, side, batch)
+        fn(name, side, batch)
     torch.cuda.synchronize()
     free1, _ = torch.cuda.mem_get_info()
     print(f"{name} b{batch}: free before {free0 >> 20} MiB, after 15 cycles {free1 >> 20} MiB, delta {(free0 - free1) >> 20} MiB")
