@@ -413,6 +413,19 @@ int network_detect_submit_frames(network net, const unsigned char *frames_hwc, i
                                  float thresh, float nms, int max_det);
 void network_detect_batch_frames(network net, const unsigned char *frames_hwc, int frame_w, int frame_h,
                                  float thresh, float nms, y2_detection *dets, int *counts, int max_det);
+/* A list of n decoded frames (1 <= n <= batch), each uint8 interleaved RGB [frame_h[i]][frame_w[i]][3] with its own
+ * size: byte/255. and resize_image run on the device for every frame in one launch, bit-identical per frame to the
+ * host chain of network_detect_batch_frames.  dets: [n][max_det], counts: [n]; the wait of such a batch fills only
+ * the first n images.  network_pipeline_staging_frame_list grows the slot's pinned buffer for this list, returns its
+ * base and fills offsets[n]: a frame already written at base + offsets[i] is not copied again on the host (every
+ * other frame is); the buffer moves when a later call needs it larger. */
+unsigned char *network_pipeline_staging_frame_list(network net, int slot, int n, const int *frame_w,
+                                                   const int *frame_h, size_t *offsets);
+int network_detect_submit_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                     const int *frame_h, float thresh, float nms, int max_det);
+void network_detect_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                     const int *frame_h, float thresh, float nms, y2_detection *dets, int *counts,
+                                     int max_det);
 /* ---- batched, device-resident classification: letterbox, forward pass, WordTree products and top-k run on the
  * device and only `top` (index, probability) pairs per image come back, equal to what predict_classifier_image
  * computes on the host (classifier.c:676-730: letterbox_image, network_predict, hierarchy_predictions for a WordTree
@@ -445,6 +458,12 @@ int network_classify_submit_u8(network net, const unsigned char *input_hwc, int 
 int network_classify_submit_frames(network net, const unsigned char *frames_hwc, int frame_w, int frame_h, int top);
 int network_classify_submit_resident(network net, int top);
 int network_classify_wait(network net, y2_class_hit *hits, int top);
+/* A list of n frames of any sizes (as network_detect_submit_frame_list, same staging call), each letterboxed on the
+ * device: hits [n][top].  A letterbox window 1 pixel high has no defined result, as for the uniform entry. */
+int network_classify_submit_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                       const int *frame_h, int top);
+void network_classify_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                       const int *frame_h, int top, y2_class_hit *hits);
 /* ---- the same over several GPUs of one box from ONE caller (one replica and one host thread per GPU; idiom of
  * train_networks, network_kernels.cu:346-376).  Replica i owns the next nets[i].batch images of the global batch;
  * detections land in the caller's arrays in image order - nothing else crosses GPUs. ------------------------- */

@@ -201,6 +201,27 @@ void y2_letterbox_geometry(int src_w, int src_h, int w, int h, int *new_w, int *
 int y2_letterbox_u8_to_f32(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w, int h,
                            y2_stream_t s);
 
+/* A list of decoded frames, each with its own size, packed into one buffer: frame i (uint8 interleaved RGB
+ * [src_h][src_w][3]) starts at byte `offset`, and its resized image fills the window [dx, dx+new_w) x
+ * [dy, dy+new_h) of the network canvas, with resize_image's scales (image.c:1954-1955) computed on the host. */
+typedef struct y2_frame_window {
+    unsigned long long offset;
+    int src_w, src_h;
+    int dx, dy, new_w, new_h;
+    float w_scale, h_scale;
+} y2_frame_window;
+/* The layout of such a list for a w x h network: frames in list order, each at a 16-byte-aligned offset, then the
+ * table of n records (at *table_offset, also 16-byte aligned).  letterbox = 0: every window is the whole canvas
+ * (resize_image); 1: the window of y2_letterbox_geometry (letterbox_image).  win (may be NULL) receives the n
+ * records.  Returns the packed size in bytes, frames and table, or 0 when n < 1 or a size is <= 0. */
+size_t y2_frame_list_layout(int n, const int *frame_w, const int *frame_h, int w, int h, int letterbox,
+                            y2_frame_window *win, size_t *table_offset);
+/* Packed frames -> fp32 planar [batch][3][h][w] in one launch: image i < n is byte/255. + resize_image into the
+ * window of table[i] (a device pointer, normally inside the packed buffer) on a .5f canvas, bit-identical to the
+ * host chain; images n..batch-1 are all .5f.  A window 1 pixel high has no defined result (see above). */
+int y2_frames_u8_to_f32(const unsigned char *packed, const y2_frame_window *table, int n, float *dst, int batch,
+                        int w, int h, y2_stream_t s);
+
 /* bf16 padded NHWC slice -> fp32 NCHW [B][C][H][W] (host-visible l.output layout). */
 int y2_unpack_to_nchw_f32(const void *src, float *dst, int batch, int c, int h, int w,
                           int cs, y2_stream_t s);

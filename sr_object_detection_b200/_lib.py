@@ -35,6 +35,25 @@ class Det(C.Structure):
                 ("prob", C.c_float), ("obj_id", C.c_int), ("box_index", C.c_int)]
 
 
+class FrameWindow(C.Structure):
+    """Mirror of `y2_frame_window`: where one frame of a packed frame list sits and the window it fills."""
+    _fields_ = [("offset", C.c_ulonglong), ("src_w", C.c_int), ("src_h", C.c_int), ("dx", C.c_int), ("dy", C.c_int),
+                ("new_w", C.c_int), ("new_h", C.c_int), ("w_scale", C.c_float), ("h_scale", C.c_float)]
+
+
+def frame_list_layout(sizes, w: int, h: int, letterbox: bool):
+    """y2_frame_list_layout for frames of sizes [(frame_w, frame_h), ...] on a w x h network: (records, table offset,
+    packed size in bytes)."""
+    lib = load()
+    n = len(sizes)
+    fw = (C.c_int * max(n, 1))(*[s[0] for s in sizes])
+    fh = (C.c_int * max(n, 1))(*[s[1] for s in sizes])
+    win = (FrameWindow * max(n, 1))()
+    toff = C.c_size_t()
+    total = lib.y2_frame_list_layout(n, fw, fh, w, h, int(letterbox), win, C.byref(toff))
+    return list(win)[:n], toff.value, total
+
+
 def lib_path() -> Path:
     return _build.LIB
 
@@ -103,6 +122,9 @@ def _declare(lib: C.CDLL) -> None:
         "y2_gather_patches_bf16": (i, [vp, i, i, i, i, vp, i, i, i, i, i, i, vp]),
         "y2_gather_rows_f32": (i, [vp, vp, i, i, i, i, i, i, i, i, i, i, vp]),
         "y2_resize_u8_to_f32": (i, [vp, vp, i, i, i, i, i, vp]),
+        "y2_frame_list_layout": (C.c_size_t, [i, C.POINTER(i), C.POINTER(i), i, i, i, C.POINTER(FrameWindow),
+                                              C.POINTER(C.c_size_t)]),
+        "y2_frames_u8_to_f32": (i, [vp, vp, i, vp, i, i, i, vp]),
         "y2_unpack_to_nchw_f32": (i, [vp, vp, i, i, i, i, i, vp]),
         "y2_flat_to_nchw_f32": (i, [vp, vp, i, i, i, i, vp]),
         "y2_nchw_to_flat_f32": (i, [vp, vp, i, i, i, vp]),

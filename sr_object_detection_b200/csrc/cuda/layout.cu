@@ -274,52 +274,70 @@ __global__ void gather_patches_bf16_kernel(const __nv_bfloat16 *__restrict__ in,
 // recomputed for the two source rows a target pixel needs instead of materialising `part`.
 // Quirk kept: the last target row takes only the (1-dy) term (image.c:1985 `continue`).
 // ---------------------------------------------------------------------------------
-__device__ __forceinline__ float resize_part(const unsigned char *__restrict__ row, const float *lut, int sw, int w,
-                                             int c, int k, float w_scale)
-{
-    if (c == w - 1 || sw == 1) return lut[row[(size_t)(sw - 1) * 3 + k]];
-    const float sx = __fmul_rn((float)c, w_scale);
-    int ix = (int)sx;
-    const float dx = __fsub_rn(sx, (float)ix);
-    int ix1 = ix + 1;
-    if (ix1 > sw - 1) ix1 = sw - 1; // the reference would assert here; unreachable for exact scales
-    const float a = __fmul_rn(__fsub_rn(1.f, dx), lut[row[(size_t)ix * 3 + k]]);
-    const float b = __fmul_rn(dx, lut[row[(size_t)ix1 * 3 + k]]);
-    return __fadd_rn(a, b);
-}
 
 // The resized image fills the window [dx, dx+nw) x [dy, dy+nh) of the w x h canvas and the rest is .5f: the whole
 // canvas for resize_image, the centred window of letterbox_image (image.c:1624-1644: fill_image(.5) + embed_image).
-__global__ void resize_u8_to_f32_kernel(const unsigned char *__restrict__ src, float *__restrict__ dst, int batch,
-                                        int sw, int sh, int w, int h, int dx, int dy, int nw, int nh, float w_scale,
-                                        float h_scale)
+// Image b = blockIdx.y reads its record once: table[b], or for a uniform batch (table == NULL) the by-value record
+// with the frame at uni.offset + b * stride.  One thread per output pixel writes all three planes from the same
+// 3-byte taps.  Images b >= n are the .5f canvas.
+__global__ void frames_u8_to_f32_kernel(const unsigned char *__restrict__ packed,
+                                        const y2_frame_window *__restrict__ table, y2_frame_window uni,
+                                        unsigned long long stride, int n, float *__restrict__ dst, int w, int h)
 {
     __shared__ float lut[256];
     for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = (float)((double)(float)i / 255.);
     __syncthreads();
-    const long long total = (long long)batch * 3 * h * w;
-    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total;
-         t += (long long)gridDim.x * blockDim.x) {
-        const int c = (int)(t % w) - dx;
-        const int r = (int)((t / w) % h) - dy;
-        if (c < 0 || c >= nw || r < 0 || r >= nh) {
-            dst[t] = .5f;
-            continue;
+    const int b = blockIdx.y;
+    const int hw = w * h;
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= hw) return;
+    float *out = dst + (size_t)b * 3 * hw + p;
+    const int y = p / w;
+    y2_frame_window f = uni;
+    if (b < n) {
+        if (table) f = table[b];
+        else f.offset += (unsigned long long)b * stride;
+    }
+    const int c = p - y * w - f.dx, r = y - f.dy;
+    if (b >= n || c < 0 || c >= f.new_w || r < 0 || r >= f.new_h) {
+        out[0] = .5f;
+        out[hw] = .5f;
+        out[2 * hw] = .5f;
+        return;
+    }
+    const int sw = f.src_w, sh = f.src_h;
+    const unsigned char *img = packed + f.offset;
+    // horizontal taps of resize_part: the edge column, or ix / ix1 with weight dx
+    const bool edge = c == f.new_w - 1 || sw == 1;
+    int ix = sw - 1, ix1 = sw - 1;
+    float dx = 0.f;
+    if (!edge) {
+        const float sx = __fmul_rn((float)c, f.w_scale);
+        ix = (int)sx;
+        dx = __fsub_rn(sx, (float)ix);
+        ix1 = ix + 1;
+        if (ix1 > sw - 1) ix1 = sw - 1; // the reference would assert here; unreachable for exact scales
+    }
+    const float sy = __fmul_rn((float)r, f.h_scale);
+    int iy = (int)sy;
+    if (iy > sh - 1) iy = sh - 1;
+    const float fy = __fsub_rn(sy, (float)iy);
+    const bool two_rows = !(r == f.new_h - 1 || sh == 1); // image.c:1985: the last row takes the (1-dy) term only
+    int iy1 = iy + 1;
+    if (iy1 > sh - 1) iy1 = sh - 1;
+    const unsigned char *r0 = img + (size_t)iy * sw * 3, *r1 = img + (size_t)iy1 * sw * 3;
+    const unsigned char *a0 = r0 + ix * 3, *b0 = r0 + ix1 * 3, *a1 = r1 + ix * 3, *b1 = r1 + ix1 * 3;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        float part0 = lut[a0[k]];
+        if (!edge) part0 = __fadd_rn(__fmul_rn(__fsub_rn(1.f, dx), part0), __fmul_rn(dx, lut[b0[k]]));
+        float val = __fmul_rn(__fsub_rn(1.f, fy), part0);
+        if (two_rows) {
+            float part1 = lut[a1[k]];
+            if (!edge) part1 = __fadd_rn(__fmul_rn(__fsub_rn(1.f, dx), part1), __fmul_rn(dx, lut[b1[k]]));
+            val = __fadd_rn(val, __fmul_rn(fy, part1));
         }
-        const int k = (int)((t / ((long long)w * h)) % 3);
-        const int b = (int)(t / ((long long)w * h * 3));
-        const unsigned char *img = src + (size_t)b * sh * sw * 3;
-        const float sy = __fmul_rn((float)r, h_scale);
-        int iy = (int)sy;
-        if (iy > sh - 1) iy = sh - 1;
-        const float fy = __fsub_rn(sy, (float)iy);
-        float val = __fmul_rn(__fsub_rn(1.f, fy), resize_part(img + (size_t)iy * sw * 3, lut, sw, nw, c, k, w_scale));
-        if (!(r == nh - 1 || sh == 1)) {
-            int iy1 = iy + 1;
-            if (iy1 > sh - 1) iy1 = sh - 1;
-            val = __fadd_rn(val, __fmul_rn(fy, resize_part(img + (size_t)iy1 * sw * 3, lut, sw, nw, c, k, w_scale)));
-        }
-        dst[t] = val;
+        out[(size_t)k * hw] = val;
     }
 }
 
@@ -952,18 +970,71 @@ extern "C" int y2_gather_patches_bf16(const void *in, int in_cs, int cin_pad, in
     return Y2_OK;
 }
 
-// resize_image(byte/255. image, nw, nh) into the window at (dx, dy) of a .5f canvas of w x h
-static int resize_window(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w, int h, int dx,
-                         int dy, int nw, int nh, y2_stream_t s)
+static const int FRAMES_THREADS = 256;
+
+static int launch_frames(const unsigned char *packed, const y2_frame_window *table, const y2_frame_window &uni,
+                         unsigned long long stride, int n, float *dst, int batch, int w, int h, y2_stream_t s)
 {
-    // image.c:1954-1955: float w_scale = (float)(im.w - 1) / (w - 1)  (w == 1 divides by zero there too)
-    const float w_scale = (float)(src_w - 1) / (nw - 1);
-    const float h_scale = (float)(src_h - 1) / (nh - 1);
-    const long long total = (long long)batch * 3 * h * w;
-    resize_u8_to_f32_kernel<<<grid_for(total, 256), 256, 0, to_stream(s)>>>(src, dst, batch, src_w, src_h, w, h, dx,
-                                                                            dy, nw, nh, w_scale, h_scale);
+    const long long hw = (long long)w * h;
+    if (batch > 65535 || hw > 0x7fffffffLL - FRAMES_THREADS) {
+        set_error("y2_frames_u8_to_f32: batch %d or canvas %dx%d beyond the launch limits", batch, w, h);
+        return Y2_EINVAL;
+    }
+    const dim3 grid((unsigned)((hw + FRAMES_THREADS - 1) / FRAMES_THREADS), (unsigned)batch);
+    frames_u8_to_f32_kernel<<<grid, FRAMES_THREADS, 0, to_stream(s)>>>(packed, table, uni, stride, n, dst, w, h);
     Y2_LAUNCH_CHECK();
     return Y2_OK;
+}
+
+// The window of one frame: the whole canvas (resize_image) or letterbox_image's, with resize_image's scales.
+static y2_frame_window frame_window(int src_w, int src_h, int w, int h, int letterbox)
+{
+    y2_frame_window f = {};
+    f.src_w = src_w;
+    f.src_h = src_h;
+    f.new_w = w;
+    f.new_h = h;
+    if (letterbox) y2_letterbox_geometry(src_w, src_h, w, h, &f.new_w, &f.new_h, &f.dx, &f.dy);
+    // image.c:1954-1955: float w_scale = (float)(im.w - 1) / (w - 1)  (w == 1 divides by zero there too)
+    f.w_scale = (float)(src_w - 1) / (f.new_w - 1);
+    f.h_scale = (float)(src_h - 1) / (f.new_h - 1);
+    return f;
+}
+
+extern "C" size_t y2_frame_list_layout(int n, const int *frame_w, const int *frame_h, int w, int h, int letterbox,
+                                       y2_frame_window *win, size_t *table_offset)
+{
+    if (n < 1 || !frame_w || !frame_h || w <= 0 || h <= 0) return 0;
+    size_t off = 0;
+    for (int i = 0; i < n; ++i) {
+        if (frame_w[i] <= 0 || frame_h[i] <= 0) return 0;
+        if (win) {
+            win[i] = frame_window(frame_w[i], frame_h[i], w, h, letterbox);
+            win[i].offset = off;
+        }
+        off += ((size_t)frame_w[i] * frame_h[i] * 3 + 15) & ~(size_t)15;
+    }
+    if (table_offset) *table_offset = off;
+    return off + (size_t)n * sizeof(y2_frame_window);
+}
+
+extern "C" int y2_frames_u8_to_f32(const unsigned char *packed, const y2_frame_window *table, int n, float *dst,
+                                   int batch, int w, int h, y2_stream_t s)
+{
+    if (!packed || !table || !dst || n < 1 || n > batch || w <= 0 || h <= 0) {
+        set_error("y2_frames_u8_to_f32: invalid arguments (n=%d batch=%d %dx%d)", n, batch, w, h);
+        return Y2_EINVAL;
+    }
+    const y2_frame_window none = {};
+    return launch_frames(packed, table, none, 0, n, dst, batch, w, h, s);
+}
+
+// a uniform batch: one record passed by value, frame b at b * src_h * src_w * 3
+static int uniform_frames(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w, int h,
+                          int letterbox, y2_stream_t s)
+{
+    const y2_frame_window f = frame_window(src_w, src_h, w, h, letterbox);
+    return launch_frames(src, nullptr, f, (unsigned long long)src_w * src_h * 3, batch, dst, batch, w, h, s);
 }
 
 extern "C" int y2_resize_u8_to_f32(const unsigned char *src, float *dst, int batch, int src_w, int src_h, int w,
@@ -973,7 +1044,7 @@ extern "C" int y2_resize_u8_to_f32(const unsigned char *src, float *dst, int bat
         set_error("y2_resize_u8_to_f32: invalid arguments (%dx%d -> %dx%d)", src_w, src_h, w, h);
         return Y2_EINVAL;
     }
-    return resize_window(src, dst, batch, src_w, src_h, w, h, 0, 0, w, h, s);
+    return uniform_frames(src, dst, batch, src_w, src_h, w, h, 0, s);
 }
 
 extern "C" void y2_letterbox_geometry(int src_w, int src_h, int w, int h, int *new_w, int *new_h, int *dx, int *dy)
@@ -996,9 +1067,7 @@ extern "C" int y2_letterbox_u8_to_f32(const unsigned char *src, float *dst, int 
         set_error("y2_letterbox_u8_to_f32: invalid arguments (%dx%d -> %dx%d)", src_w, src_h, w, h);
         return Y2_EINVAL;
     }
-    int nw, nh, dx, dy;
-    y2_letterbox_geometry(src_w, src_h, w, h, &nw, &nh, &dx, &dy);
-    return resize_window(src, dst, batch, src_w, src_h, w, h, dx, dy, nw, nh, s);
+    return uniform_frames(src, dst, batch, src_w, src_h, w, h, 1, s);
 }
 
 extern "C" int y2_unpack_to_nchw_f32(const void *src, float *dst, int batch, int c, int h, int w, int cs,

@@ -318,31 +318,101 @@ unsigned char *network_pipeline_staging_u8(network net, int slot)
     return rt->pipe[slot].in_u8_pinned;
 }
 
-static void pipe_reserve_frames(y2_net_rt *rt, int s, size_t bytes)
+/* grows slot s's frame buffers to `bytes`; with old_pinned, the old pinned buffer is handed to the caller (to copy
+ * frames out of it before freeing it) instead of being freed here */
+static void pipe_reserve_frames(y2_net_rt *rt, int s, size_t bytes, unsigned char **old_pinned)
 {
     struct y2_pipe_slot *ps = &rt->pipe[s];
     if (ps->frames_cap >= bytes) return;
     y2_free(ps->frames_dev);
-    y2_host_free(ps->frames_pinned);
+    if (old_pinned) *old_pinned = ps->frames_pinned;
+    else y2_host_free(ps->frames_pinned);
     Y2_CHECK(y2_malloc((void **)&ps->frames_dev, bytes));
     Y2_CHECK(y2_host_alloc((void **)&ps->frames_pinned, bytes));
     ps->frames_cap = bytes;
 }
 
+/* n frames of their own sizes (the *_frame_list entries) */
+typedef struct {
+    int n;
+    const unsigned char *const *frames;
+    const int *w, *h;
+} frame_list;
+
+/* the refusals of every frame-list entry, before anything is staged */
+static void check_frame_list(network net, const frame_list *fl)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network frame list: network has no device plan");
+    if (net.c != 3) error("network frame list: needs a network with 3 input channels");
+    if (fl->n < 1 || fl->n > net.batch) error("network frame list: the list must hold 1 .. batch frames");
+    if (!fl->frames || !fl->w || !fl->h) error("network frame list: NULL frame, width or height array");
+    for (int i = 0; i < fl->n; ++i) {
+        if (!fl->frames[i]) error("network frame list: NULL frame pointer");
+        if (fl->w[i] <= 0 || fl->h[i] <= 0) error("network frame list: a frame size of 0 or less");
+    }
+}
+
+unsigned char *network_pipeline_staging_frame_list(network net, int slot, int n, const int *frame_w,
+                                                   const int *frame_h, size_t *offsets)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network_pipeline_staging_frame_list: network has no device plan");
+    if (slot < 0 || slot > 1 || n < 1 || n > net.batch || !offsets)
+        error("network_pipeline_staging_frame_list: bad slot or offsets, or a list not of 1 .. batch frames");
+    const size_t bytes = y2_frame_list_layout(n, frame_w, frame_h, net.w, net.h, 0, NULL, NULL);
+    if (!bytes) error("network_pipeline_staging_frame_list: a frame size of 0 or less");
+    pipe_init(net);
+    Y2_CHECK(y2_set_device(rt->device));
+    pipe_reserve_frames(rt, slot, bytes, NULL);
+    y2_frame_window *win = (y2_frame_window *)calloc((size_t)n, sizeof(y2_frame_window));
+    if (!win) error("network_pipeline_staging_frame_list: out of host memory");
+    y2_frame_list_layout(n, frame_w, frame_h, net.w, net.h, 0, win, NULL);
+    for (int i = 0; i < n; ++i) offsets[i] = (size_t)win[i].offset;
+    free(win);
+    return rt->pipe[slot].frames_pinned;
+}
+
+/* A frame list into slot s: the frames and the record table behind them in the slot's pinned buffer (frames already
+ * at their place there are not copied), then one H2D copy of the whole region on the copy stream.  Returns the
+ * table's offset in the region. */
+static size_t stage_frame_list(network net, int s, const frame_list *fl, int letterbox)
+{
+    y2_net_rt *rt = y2_rt(net);
+    struct y2_pipe_slot *ps = &rt->pipe[s];
+    size_t table_off = 0;
+    const size_t bytes = y2_frame_list_layout(fl->n, fl->w, fl->h, net.w, net.h, letterbox, NULL, &table_off);
+    unsigned char *old = NULL;
+    pipe_reserve_frames(rt, s, bytes, &old);
+    y2_frame_window *win = (y2_frame_window *)(ps->frames_pinned + table_off);
+    y2_frame_list_layout(fl->n, fl->w, fl->h, net.w, net.h, letterbox, win, NULL);
+    for (int i = 0; i < fl->n; ++i) {
+        unsigned char *dst = ps->frames_pinned + win[i].offset;
+        if (fl->frames[i] != dst) memcpy(dst, fl->frames[i], (size_t)fl->w[i] * fl->h[i] * 3);
+    }
+    Y2_CHECK(y2_host_free(old));
+    Y2_CHECK(y2_memcpy_h2d(ps->frames_dev, ps->frames_pinned, bytes, rt->copy_stream));
+    return table_off;
+}
+
 /* The input half of a submission, into slot s: the staging copy, the H2D copy on the copy stream, resize (or
  * letterbox) and the forward pass on the network's stream.  input: fp32 planar [B][c][h][w] (u8 == 0), uint8
  * interleaved RGB [B][h][w][3] at the network's resolution (u8 == 1), uint8 interleaved RGB frames [B][fh][fw][3]
- * of any size (u8 == 2), or nothing: the slot's device input already holds the batch (u8 == 3, *_submit_resident) */
+ * of any size (u8 == 2), nothing: the slot's device input already holds the batch (u8 == 3, *_submit_resident), or
+ * a frame_list (u8 == 4) */
 static void submit_input(network net, int s, const void *input, int u8, int fw, int fh, int letterbox)
 {
     y2_net_rt *rt = y2_rt(net);
     struct y2_pipe_slot *ps = &rt->pipe[s];
     const int B = net.batch;
+    size_t table_off = 0;
     /* pageable caller memory is staged through the slot's pinned buffer (a host copy; fill the slot's
      * staging buffer directly to avoid it) */
-    if (u8 == 2) {
+    if (u8 == 4) {
+        table_off = stage_frame_list(net, s, (const frame_list *)input, letterbox);
+    } else if (u8 == 2) {
         const size_t bytes = (size_t)B * fh * fw * 3;
-        pipe_reserve_frames(rt, s, bytes);
+        pipe_reserve_frames(rt, s, bytes, NULL);
         if (input && input != ps->frames_pinned) memcpy(ps->frames_pinned, input, bytes);
         Y2_CHECK(y2_memcpy_h2d(ps->frames_dev, ps->frames_pinned, bytes, rt->copy_stream));
     } else if (u8 == 1) {
@@ -358,7 +428,10 @@ static void submit_input(network net, int s, const void *input, int u8, int fw, 
         Y2_CHECK(y2_event_record(ps->ev_h2d, rt->copy_stream));
         Y2_CHECK(y2_stream_wait_event(rt->stream, ps->ev_h2d));
     }
-    if (u8 == 2 && letterbox) /* byte/255. + letterbox_image on the device, into the slot's fp32 input */
+    if (u8 == 4) /* byte/255. + resize_image or letterbox_image per frame, one launch, .5f behind the list */
+        Y2_CHECK(y2_frames_u8_to_f32(ps->frames_dev, (const y2_frame_window *)(ps->frames_dev + table_off),
+                                     ((const frame_list *)input)->n, ps->in_dev, B, net.w, net.h, rt->stream));
+    else if (u8 == 2 && letterbox) /* byte/255. + letterbox_image on the device, into the slot's fp32 input */
         Y2_CHECK(y2_letterbox_u8_to_f32(ps->frames_dev, ps->in_dev, B, fw, fh, net.w, net.h, rt->stream));
     else if (u8 == 2) /* byte/255. + resize_image on the device, into the slot's fp32 input */
         Y2_CHECK(y2_resize_u8_to_f32(ps->frames_dev, ps->in_dev, B, fw, fh, net.w, net.h, rt->stream));
@@ -397,11 +470,12 @@ static void submit_results(y2_net_rt *rt, int s)
     Y2_CHECK(y2_stream_wait_event(rt->d2h_stream, ps->ev_tail));
 }
 
-static void submit_done(y2_net_rt *rt, int s, int kind)
+static void submit_done(y2_net_rt *rt, int s, int kind, int n_images)
 {
     struct y2_pipe_slot *ps = &rt->pipe[s];
     Y2_CHECK(y2_event_record(ps->ev_done, rt->d2h_stream));
     ps->kind = kind;
+    ps->n_images = n_images;
     ps->busy = 1;
     rt->pipe_inflight++;
 }
@@ -414,13 +488,14 @@ static int submit_common(network net, const void *input, int u8, int fw, int fh,
     struct y2_pipe_slot *ps = &rt->pipe[s];
     layer *l = region_of(net);
     const int B = net.batch;
+    const int n = u8 == 4 ? ((const frame_list *)input)->n : B; /* the tail runs on all B, n come back */
     pipe_reserve_dets(rt, s, B, max_det);
     submit_input(net, s, input, u8, fw, fh, 0);
     detect_tail(rt, l, net.layers[net.n - 2].b200, thresh, nms, ps->det_dev, ps->cnt_dev, ps->det_cap);
     submit_results(rt, s);
-    Y2_CHECK(y2_memcpy_d2h(ps->cnt_pinned, ps->cnt_dev, (size_t)B * sizeof(int), rt->d2h_stream));
-    Y2_CHECK(y2_memcpy_d2h(ps->det_pinned, ps->det_dev, (size_t)B * ps->det_cap * sizeof(y2_det), rt->d2h_stream));
-    submit_done(rt, s, Y2_PIPE_DETECT);
+    Y2_CHECK(y2_memcpy_d2h(ps->cnt_pinned, ps->cnt_dev, (size_t)n * sizeof(int), rt->d2h_stream));
+    Y2_CHECK(y2_memcpy_d2h(ps->det_pinned, ps->det_dev, (size_t)n * ps->det_cap * sizeof(y2_det), rt->d2h_stream));
+    submit_done(rt, s, Y2_PIPE_DETECT, n);
     return s;
 }
 
@@ -458,8 +533,7 @@ int network_detect_wait(network net, y2_detection *dets, int *counts, int max_de
     if (ps->kind != Y2_PIPE_DETECT)
         error("network_detect_wait: the oldest batch in flight is a classify batch, call network_classify_wait");
     Y2_CHECK(y2_event_sync(ps->ev_done));
-    const int B = net.batch;
-    for (int b = 0; b < B; ++b) {
+    for (int b = 0; b < ps->n_images; ++b) {
         int c = ps->cnt_pinned[b];
         counts[b] = c;
         if (c > max_det) c = max_det;
@@ -502,6 +576,25 @@ int network_detect_submit_frames(network net, const unsigned char *frames_hwc, i
     return submit_common(net, frames_hwc, 2, frame_w, frame_h, thresh, nms, max_det);
 }
 
+int network_detect_submit_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                     const int *frame_h, float thresh, float nms, int max_det)
+{
+    const frame_list fl = {n, frames, frame_w, frame_h};
+    check_frame_list(net, &fl);
+    return submit_common(net, &fl, 4, 0, 0, thresh, nms, max_det);
+}
+
+void network_detect_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                     const int *frame_h, float thresh, float nms, y2_detection *dets, int *counts,
+                                     int max_det)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (rt && rt->pipe_inflight)
+        error("network_detect_batch_frame_list: batches of the submit/wait pipeline are in flight");
+    network_detect_submit_frame_list(net, n, frames, frame_w, frame_h, thresh, nms, max_det);
+    network_detect_wait(net, dets, counts, max_det);
+}
+
 unsigned char *network_pipeline_staging_frames(network net, int slot, int frame_w, int frame_h)
 {
     y2_net_rt *rt = y2_rt(net);
@@ -510,7 +603,7 @@ unsigned char *network_pipeline_staging_frames(network net, int slot, int frame_
     if (frames_take_u8(net, frame_w, frame_h)) return network_pipeline_staging_u8(net, slot);
     pipe_init(net);
     Y2_CHECK(y2_set_device(rt->device));
-    pipe_reserve_frames(rt, slot, (size_t)rt->cap_batch * frame_h * frame_w * 3);
+    pipe_reserve_frames(rt, slot, (size_t)rt->cap_batch * frame_h * frame_w * 3, NULL);
     return rt->pipe[slot].frames_pinned;
 }
 
@@ -592,14 +685,14 @@ static int classify_submit_common(network net, const void *input, int u8, int fw
     const int s = submit_slot(net, u8, fw, fh);
     y2_net_rt *rt = y2_rt(net);
     struct y2_pipe_slot *ps = &rt->pipe[s];
+    const int n = u8 == 4 ? ((const frame_list *)input)->n : net.batch;
     reserve_hits(rt, &ps->hits_dev, &ps->hits_pinned, &ps->hits_cap, top);
     submit_input(net, s, input, u8, fw, fh, 1);
     classify_tail(rt, net, l, top, ps->hits_dev);
     submit_results(rt, s);
-    Y2_CHECK(y2_memcpy_d2h(ps->hits_pinned, ps->hits_dev, (size_t)net.batch * top * sizeof(y2_class_hit),
-                           rt->d2h_stream));
+    Y2_CHECK(y2_memcpy_d2h(ps->hits_pinned, ps->hits_dev, (size_t)n * top * sizeof(y2_class_hit), rt->d2h_stream));
     ps->hits_top = top;
-    submit_done(rt, s, Y2_PIPE_CLASSIFY);
+    submit_done(rt, s, Y2_PIPE_CLASSIFY, n);
     return s;
 }
 
@@ -636,7 +729,7 @@ int network_classify_wait(network net, y2_class_hit *hits, int top)
         error("network_classify_wait: the oldest batch in flight is a detection batch, call network_detect_wait");
     if (top != ps->hits_top) error("network_classify_wait: top differs from the one the batch was submitted with");
     Y2_CHECK(y2_event_sync(ps->ev_done));
-    memcpy(hits, ps->hits_pinned, (size_t)net.batch * top * sizeof(y2_class_hit));
+    memcpy(hits, ps->hits_pinned, (size_t)ps->n_images * top * sizeof(y2_class_hit));
     ps->busy = 0;
     rt->pipe_head ^= 1;
     rt->pipe_inflight--;
@@ -649,5 +742,23 @@ void network_classify_batch_frames(network net, const unsigned char *frames_hwc,
     y2_net_rt *rt = y2_rt(net);
     if (rt && rt->pipe_inflight) error("network_classify_batch_frames: batches of the submit/wait pipeline are in flight");
     network_classify_submit_frames(net, frames_hwc, frame_w, frame_h, top);
+    network_classify_wait(net, hits, top);
+}
+
+int network_classify_submit_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                       const int *frame_h, int top)
+{
+    const frame_list fl = {n, frames, frame_w, frame_h};
+    check_frame_list(net, &fl);
+    return classify_submit_common(net, &fl, 4, 0, 0, top);
+}
+
+void network_classify_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
+                                       const int *frame_h, int top, y2_class_hit *hits)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (rt && rt->pipe_inflight)
+        error("network_classify_batch_frame_list: batches of the submit/wait pipeline are in flight");
+    network_classify_submit_frame_list(net, n, frames, frame_w, frame_h, top);
     network_classify_wait(net, hits, top);
 }

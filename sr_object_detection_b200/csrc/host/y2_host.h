@@ -119,6 +119,7 @@ typedef struct y2_net_rt {
         unsigned char *frames_dev, *frames_pinned;
         size_t frames_cap;
         int kind;           /* Y2_PIPE_* of the batch in the slot */
+        int n_images;       /* images the wait hands back: the list length of a frame list, else the batch */
         /* class hits of a classify batch ([B][hits_top]), room for cap_batch x hits_cap */
         y2_class_hit *hits_dev, *hits_pinned;
         int hits_cap, hits_top;

@@ -162,6 +162,14 @@ def lib() -> C.CDLL:
         "network_pipeline_staging_frames": (C.POINTER(C.c_ubyte), [Network, i, i, i]),
         "network_detect_submit_frames": (i, [Network, C.POINTER(C.c_ubyte), i, i, f, f, i]),
         "network_detect_batch_frames": (None, [Network, C.POINTER(C.c_ubyte), i, i, f, f, C.POINTER(Detection), _ip, i]),
+        "network_pipeline_staging_frame_list": (C.POINTER(C.c_ubyte), [Network, i, i, _ip, _ip,
+                                                                        C.POINTER(C.c_size_t)]),
+        "network_detect_submit_frame_list": (i, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f, i]),
+        "network_detect_batch_frame_list": (None, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f,
+                                                   C.POINTER(Detection), _ip, i]),
+        "network_classify_submit_frame_list": (i, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i]),
+        "network_classify_batch_frame_list": (None, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i,
+                                                     C.POINTER(ClassHit)]),
         "network_classify_device": (None, [Network, i, C.POINTER(ClassHit)]),
         "network_classify_batch": (None, [Network, fp, i, C.POINTER(ClassHit)]),
         "network_classify_batch_frames": (None, [Network, C.POINTER(C.c_ubyte), i, i, i, C.POINTER(ClassHit)]),
@@ -344,7 +352,7 @@ def network_detect_batch(net: Network, images: np.ndarray | None, thresh: float,
 
 
 def _hits_arrays(hits, batch: int, top: int):
-    arr = np.ctypeslib.as_array(hits).reshape(batch, top)
+    arr = np.ctypeslib.as_array(hits)[:batch * top].reshape(batch, top)
     return arr["index"].astype(np.int32), arr["prob"].astype(np.float32)
 
 
@@ -353,11 +361,70 @@ def _as_u8(a: np.ndarray):
     return a.ctypes.data_as(C.POINTER(C.c_ubyte))
 
 
+def _frame_list_args(frames):
+    """(n, frame pointers, widths, heights) of a sequence of uint8 [h][w][3] arrays, for the *_frame_list entries"""
+    n = len(frames)
+    for a in frames:
+        assert a.dtype == np.uint8 and a.ndim == 3 and a.shape[2] == 3 and a.flags["C_CONTIGUOUS"], (a.dtype, a.shape)
+    ptrs = (C.POINTER(C.c_ubyte) * max(n, 1))(*[_as_u8(a) for a in frames])
+    fw = (C.c_int * max(n, 1))(*[a.shape[1] for a in frames])
+    fh = (C.c_int * max(n, 1))(*[a.shape[0] for a in frames])
+    return n, ptrs, fw, fh
+
+
+def network_pipeline_staging_frame_list(net: Network, slot: int, sizes):
+    """The slot's pinned staging buffer laid out for frames of sizes [(frame_w, frame_h), ...]: one writable uint8
+    [h][w][3] view per frame at its place.  Fill the views and pass them as the frame list to skip the host copy;
+    they stay valid until a larger list makes the slot's buffer grow."""
+    n = len(sizes)
+    fw = (C.c_int * max(n, 1))(*[s[0] for s in sizes])
+    fh = (C.c_int * max(n, 1))(*[s[1] for s in sizes])
+    offsets = (C.c_size_t * max(n, 1))()
+    base = C.cast(lib().network_pipeline_staging_frame_list(net, slot, n, fw, fh, offsets), C.c_void_p).value
+    return [np.ctypeslib.as_array(C.cast(base + offsets[i], C.POINTER(C.c_ubyte)), shape=(h, w, 3))
+            for i, (w, h) in enumerate(sizes)]
+
+
+def _det_lists(dets, counts, n: int, max_det: int):
+    arr = np.ctypeslib.as_array(dets)
+    return [arr[b * max_det:b * max_det + min(counts[b], max_det)].copy() for b in range(n)], list(counts)[:n]
+
+
+def network_detect_frame_list(net: Network, frames, thresh: float, nms: float, max_det: int = 256):
+    """Extension: detection on a list of 1 .. batch decoded frames (uint8 [h][w][3] arrays, each of its own size),
+    resized on the device.  Returns (per-image detection arrays, counts) for len(frames) images."""
+    n, ptrs, fw, fh = _frame_list_args(frames)
+    dets = (Detection * (max(n, 1) * max_det))()
+    counts = (C.c_int * max(n, 1))()
+    lib().network_detect_batch_frame_list(net, n, ptrs, fw, fh, thresh, nms, dets, counts, max_det)
+    return _det_lists(dets, counts, n, max_det)
+
+
+def network_detect_submit_frame_list(net: Network, frames, thresh: float, nms: float, max_det: int = 256) -> int:
+    """Queue a frame list on the submit/wait pipeline; network_detect_wait_n(net, len(frames), ...) collects it."""
+    n, ptrs, fw, fh = _frame_list_args(frames)
+    return lib().network_detect_submit_frame_list(net, n, ptrs, fw, fh, thresh, nms, max_det)
+
+
+def network_detect_wait_n(net: Network, n: int, max_det: int = 256):
+    """network_detect_wait for the oldest detection batch in flight, which holds n images"""
+    dets = (Detection * (net.batch * max_det))()
+    counts = (C.c_int * net.batch)()
+    lib().network_detect_wait(net, dets, counts, max_det)
+    return _det_lists(dets, counts, n, max_det)
+
+
 def network_classify_batch(net: Network, images: np.ndarray | None = None, frames: np.ndarray | None = None,
-                           top: int = 5):
+                           top: int = 5, frame_list=None):
     """Extension: batched forward + WordTree products + top-k on the device.  images: prepared fp32 [B][C][H][W]
-    (already letterboxed); frames: uint8 RGB [B][fh][fw][3] of any size, letterboxed on the device; neither: the
-    last forward pass.  Returns (indices int32 [B][top], probs float32 [B][top]), best first."""
+    (already letterboxed); frames: uint8 RGB [B][fh][fw][3] of any size, letterboxed on the device; frame_list: a
+    sequence of 1 .. B uint8 [h][w][3] arrays of their own sizes, letterboxed on the device; none: the last forward
+    pass.  Returns (indices int32 [n][top], probs float32 [n][top]), best first, n = B or len(frame_list)."""
+    if frame_list is not None:
+        n, ptrs, fw, fh = _frame_list_args(frame_list)
+        hits = (ClassHit * (max(n, 1) * top))()
+        lib().network_classify_batch_frame_list(net, n, ptrs, fw, fh, top, hits)
+        return _hits_arrays(hits, n, top)
     hits = (ClassHit * (net.batch * top))()
     if frames is not None:
         assert frames.ndim == 4 and frames.shape[0] == net.batch and frames.shape[3] == 3, frames.shape
@@ -371,9 +438,14 @@ def network_classify_batch(net: Network, images: np.ndarray | None = None, frame
 
 
 def network_classify_submit(net: Network, images: np.ndarray | None = None, frames: np.ndarray | None = None,
-                            u8: np.ndarray | None = None, top: int = 5) -> int:
+                            u8: np.ndarray | None = None, top: int = 5, frame_list=None) -> int:
     """Queue one batch on the submit/wait pipeline: prepared fp32 images, frames of any size, uint8 images at the
-    network size (u8), or none of them (the slot's device input already holds the batch).  Returns the slot."""
+    network size (u8), a list of frames of their own sizes (frame_list; collect it with
+    network_classify_wait(net, top, n=len(frame_list))), or none of them (the slot's device input already holds the
+    batch).  Returns the slot."""
+    if frame_list is not None:
+        n, ptrs, fw, fh = _frame_list_args(frame_list)
+        return lib().network_classify_submit_frame_list(net, n, ptrs, fw, fh, top)
     if frames is not None:
         return lib().network_classify_submit_frames(net, _as_u8(frames), frames.shape[2], frames.shape[1], top)
     if u8 is not None:
@@ -383,11 +455,12 @@ def network_classify_submit(net: Network, images: np.ndarray | None = None, fram
     return lib().network_classify_submit_resident(net, top)
 
 
-def network_classify_wait(net: Network, top: int = 5):
-    """The oldest classify batch in flight: (indices int32 [B][top], probs float32 [B][top])."""
+def network_classify_wait(net: Network, top: int = 5, n: int | None = None):
+    """The oldest classify batch in flight, which holds n images (default: the batch): (indices int32 [n][top], probs
+    float32 [n][top])."""
     hits = (ClassHit * (net.batch * top))()
     lib().network_classify_wait(net, hits, top)
-    return _hits_arrays(hits, net.batch, top)
+    return _hits_arrays(hits, net.batch if n is None else n, top)
 
 
 class _DevBuf:

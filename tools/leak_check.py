@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Developer tool (GPU box): device-memory leak check - parse / predict / detect / resize / free in a loop, and
-parse / classify / change the batch / free for a classifier."""
+"""Developer tool (GPU box): device-memory leak check - parse / predict / detect / resize / free in a loop,
+parse / classify / change the batch / free for a classifier, and frame lists whose packed size grows and shrinks."""
 import sys
 import tempfile
 from pathlib import Path
@@ -63,8 +63,31 @@ def classify_cycle(name, side, batch):
     dn.free_network(net)
 
 
+def frame_list_cycle(name, side, batch):
+    text = synth.CFGS[name](batch=batch, w=side, h=side)
+    (tmp / "f.cfg").write_text(text)
+    w = tmp / f"{name}.weights"
+    if not w.exists():
+        synth.write_weights(w, text, seed=1234)
+    net = dn.parse_network_cfg(tmp / "f.cfg")
+    dn.load_weights(net, w)
+    rng = np.random.default_rng(2)
+    # packed sizes small, large, small, larger: the slots' staging buffers grow between batches
+    for n, (fw, fh) in ((1, (500, 375)), (batch, (1280, 720)), (2, (640, 480)), (batch, (1920, 1080))):
+        frames = [rng.integers(0, 256, size=(fh - i, fw + i, 3), dtype=np.uint8) for i in range(n)]
+        dn.network_detect_submit_frame_list(net, frames, 0.02, 0.4, 64)
+        views = dn.network_pipeline_staging_frame_list(net, dn.lib().network_pipeline_next_slot(net),
+                                                       [(f.shape[1], f.shape[0]) for f in frames])
+        for v, f in zip(views, frames):
+            v[...] = f
+        dn.network_detect_submit_frame_list(net, views, 0.02, 0.4, 64)
+        dn.network_detect_wait_n(net, n, 64)
+        dn.network_detect_wait_n(net, n, 64)
+    dn.free_network(net)
+
+
 for fn, name, side, batch in ((cycle, "tiny-yolo-voc", 416, 8), (cycle, "yolo-voc", 416, 64),
-                              (classify_cycle, "darknet19_448", 448, 16)):
+                              (classify_cycle, "darknet19_448", 448, 16), (frame_list_cycle, "tiny-yolo-voc", 416, 16)):
     fn(name, side, batch)  # warm: allocator pools, per-device scratch
     torch.cuda.synchronize()
     free0, _ = torch.cuda.mem_get_info()
