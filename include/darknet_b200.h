@@ -426,6 +426,29 @@ int network_detect_submit_frame_list(network net, int n, const unsigned char *co
 void network_detect_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
                                      const int *frame_h, float thresh, float nms, y2_detection *dets, int *counts,
                                      int max_det);
+/* ---- many video streams in one batch, each frame detected on the 3-frame mean of its stream: per stream the
+ * result is bit-identical to Detector::detect(img, thresh, use_mean = true) (yolo_v2_class.cpp:206-216) on that
+ * stream's frames in order.  A stream is a ring of the last 3 region outputs, all zero at the start, and a
+ * frame_index: a frame writes slot frame_index, is decoded on (((0 + slot0) + slot1) + slot2) / 3 in float, then
+ * frame_index = (frame_index + 1) % 3.  The mean and the ring update run on the device; only the detections come
+ * back.  Needs a flat-softmax region head (no softmax tree).
+ * Streams live in the network's runtime and are freed by free_network.  open (re)allocates and starts every stream
+ * over; ids are 0 .. max_streams-1.  set_batch_network keeps the streams; after resize_network open them again. */
+void network_streams_open(network net, int max_streams);
+/* The stream starts over (zero ring, frame_index 0).  Ordered after batches already submitted. */
+void network_stream_reset(network net, int stream);
+/* A frame list (as network_detect_submit_frame_list, same staging call) whose image i belongs to stream
+ * stream_ids[i].  A stream may appear several times in one list; its frames are taken in list order.  Collected by
+ * network_detect_wait (n images).  Streams batches share the two pipeline slots with every other kind. */
+int network_detect_submit_streams(network net, int n, const int *stream_ids, const unsigned char *const *frames,
+                                  const int *frame_w, const int *frame_h, float thresh, float nms, int max_det);
+/* The same with the batch already in the slot's device input (fp32 planar at the network's size); images n..batch-1
+ * of it are run through the network but neither decoded nor entered into any stream. */
+int network_detect_submit_streams_resident(network net, int n, const int *stream_ids, float thresh, float nms,
+                                           int max_det);
+void network_detect_batch_streams(network net, int n, const int *stream_ids, const unsigned char *const *frames,
+                                  const int *frame_w, const int *frame_h, float thresh, float nms,
+                                  y2_detection *dets, int *counts, int max_det);
 /* ---- batched, device-resident classification: letterbox, forward pass, WordTree products and top-k run on the
  * device and only `top` (index, probability) pairs per image come back, equal to what predict_classifier_image
  * computes on the host (classifier.c:676-730: letterbox_image, network_predict, hierarchy_predictions for a WordTree

@@ -294,6 +294,31 @@ int y2_region_boxes_counted(float *pred, const float *d_biases, float *boxes, fl
                             int tree_n, const int *d_tree_parent, const int *d_map, int map_n,
                             int *nz_count, y2_stream_t s);
 
+/* ---- 3-frame mean of video streams (replaces, for many streams in one batch, the ring + mean_arrays of
+ *      yolo_v2_class.cpp:206-213 and utils.c:420-433) ---------------------------------------------------------- */
+/* Stream s owns ring rows 3s .. 3s+2 (slots 0..2) of a ring [max_streams][3][outputs].  For image i of a batch:
+ *   src[j]  >= 0: slot j is row src[j] of this batch's region output (an image at or before i wrote it);
+ *          == -1: slot j has not been written since open / reset and reads as +0.0f;
+ *          <= -2: slot j is ring row -2 - src[j] as it stood before the batch;
+ *   commit >= 0: the ring row image i's region output is copied to after the means; -1 when a later image of the
+ *          same stream in this batch writes that row. */
+typedef struct y2_stream_src {
+    int src[3];
+    int commit;
+} y2_stream_src;
+/* The Detector's ring rule (write slot frame_index, mean over the three slots, frame_index = (frame_index + 1) % 3)
+ * for a list of n images, image i from stream stream_ids[i], a stream's images in list order.  frame_index and
+ * frames_seen ([max_streams]; frames since open / reset, saturating at 3; both 0 for a fresh stream) are read and
+ * advanced; plan[n] receives the records.  Host only; Y2_EINVAL (nothing changed) for an id outside 0..max_streams-1. */
+int y2_stream_plan(int n, const int *stream_ids, int max_streams, int *frame_index, int *frames_seen,
+                   y2_stream_src *plan);
+/* mean[i][e] = ((0 + slot0) + slot1) + slot2) / 3 in float with round-to-nearest for the n images of table (a device
+ * copy of y2_stream_plan's records); out: the batch's region output [>= n][outputs], ring as above, mean [n][outputs]. */
+int y2_stream_mean(const float *out, const float *ring, const y2_stream_src *table, int n, int outputs, float *mean,
+                   y2_stream_t s);
+/* ring[table[i].commit] = out[i] for every committing image; launch after y2_stream_mean of the same table. */
+int y2_stream_commit(const float *out, float *ring, const y2_stream_src *table, int n, int outputs, y2_stream_t s);
+
 /* ---- do_nms_sort (replaces box.c:249-277) ------------------------------------------- */
 /* boxes [B][total][4], probs [B][total][classes] updated in place. */
 int y2_nms_sort(const float *boxes, float *probs, int batch, int total, int classes,

@@ -54,6 +54,24 @@ def frame_list_layout(sizes, w: int, h: int, letterbox: bool):
     return list(win)[:n], toff.value, total
 
 
+class StreamSrc(C.Structure):
+    """Mirror of `y2_stream_src`: where the 3 ring slots of an image's stream come from, and the ring row it commits."""
+    _fields_ = [("src", C.c_int * 3), ("commit", C.c_int)]
+
+
+def stream_plan(stream_ids, max_streams: int, frame_index, frames_seen):
+    """y2_stream_plan for one list of stream ids: (records, advanced frame_index, advanced frames_seen).  The counter
+    lists are not modified; a bad id raises Y2Error."""
+    lib = load()
+    n = len(stream_ids)
+    ids = (C.c_int * max(n, 1))(*stream_ids)
+    fi = (C.c_int * max_streams)(*frame_index)
+    seen = (C.c_int * max_streams)(*frames_seen)
+    plan = (StreamSrc * max(n, 1))()
+    check(lib.y2_stream_plan(n, ids, max_streams, fi, seen, plan), "y2_stream_plan")
+    return list(plan)[:n], list(fi), list(seen)
+
+
 def lib_path() -> Path:
     return _build.LIB
 
@@ -125,6 +143,9 @@ def _declare(lib: C.CDLL) -> None:
         "y2_frame_list_layout": (C.c_size_t, [i, C.POINTER(i), C.POINTER(i), i, i, i, C.POINTER(FrameWindow),
                                               C.POINTER(C.c_size_t)]),
         "y2_frames_u8_to_f32": (i, [vp, vp, i, vp, i, i, i, vp]),
+        "y2_stream_plan": (i, [i, C.POINTER(i), i, C.POINTER(i), C.POINTER(i), C.POINTER(StreamSrc)]),
+        "y2_stream_mean": (i, [vp, vp, vp, i, i, vp, vp]),
+        "y2_stream_commit": (i, [vp, vp, vp, i, i, vp]),
         "y2_unpack_to_nchw_f32": (i, [vp, vp, i, i, i, i, i, vp]),
         "y2_flat_to_nchw_f32": (i, [vp, vp, i, i, i, i, vp]),
         "y2_nchw_to_flat_f32": (i, [vp, vp, i, i, i, vp]),

@@ -800,6 +800,83 @@ __global__ void tree_nms_collect_kernel(const TreeRec *__restrict__ rec, int tot
     if (threadIdx.x == 0) count[b] = s_base;
 }
 
+// 3-frame mean of video streams ----------------------------------------------------
+// yolo_v2_class.cpp:206-213: every frame is decoded on mean_arrays (utils.c:420-433) over its stream's ring of the
+// last three region outputs: avg = 0; avg += ring[0]; avg += ring[1]; avg += ring[2]; avg /= 3, in float, by ring
+// slot.  The sources of the three slots come from y2_stream_plan (one y2_stream_src per image, on blockIdx.y).
+// A block covers STREAM_CHUNK elements of one image row, 4 per thread (one float4 when every row is 16-byte aligned).
+constexpr int STREAM_THREADS = 256;
+constexpr int STREAM_CHUNK = STREAM_THREADS * 4;
+
+// the row a source code names (y2_stream_src), NULL for a slot not written since open / reset
+__device__ __forceinline__ const float *stream_row(int code, const float *out, const float *ring, int outputs)
+{
+    if (code >= 0) return out + (size_t)code * outputs;
+    if (code == -1) return nullptr;
+    return ring + (size_t)(-2 - code) * outputs;
+}
+
+__device__ __forceinline__ float stream_mean3(float a, float b, float c)
+{
+    return __fdiv_rn(__fadd_rn(__fadd_rn(__fadd_rn(0.f, a), b), c), 3.f);
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(STREAM_THREADS) stream_mean_kernel(const float *__restrict__ out,
+                                                                     const float *__restrict__ ring,
+                                                                     const y2_stream_src *__restrict__ table,
+                                                                     int outputs, float *__restrict__ mean)
+{
+    const y2_stream_src rec = table[blockIdx.y];
+    const float *s0 = stream_row(rec.src[0], out, ring, outputs);
+    const float *s1 = stream_row(rec.src[1], out, ring, outputs);
+    const float *s2 = stream_row(rec.src[2], out, ring, outputs);
+    float *dst = mean + (size_t)blockIdx.y * outputs;
+    const int base = blockIdx.x * STREAM_CHUNK;
+    if (VEC) {
+        const int e = base + threadIdx.x * 4;
+        if (e >= outputs) return;
+        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+        const float4 a = s0 ? __ldg((const float4 *)(s0 + e)) : z;
+        const float4 b = s1 ? __ldg((const float4 *)(s1 + e)) : z;
+        const float4 c = s2 ? __ldg((const float4 *)(s2 + e)) : z;
+        *(float4 *)(dst + e) = make_float4(stream_mean3(a.x, b.x, c.x), stream_mean3(a.y, b.y, c.y),
+                                           stream_mean3(a.z, b.z, c.z), stream_mean3(a.w, b.w, c.w));
+    } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int e = base + q * STREAM_THREADS + threadIdx.x;
+            if (e < outputs)
+                dst[e] = stream_mean3(s0 ? __ldg(s0 + e) : 0.f, s1 ? __ldg(s1 + e) : 0.f, s2 ? __ldg(s2 + e) : 0.f);
+        }
+    }
+}
+
+// image i's region output row -> its ring row (rec.commit >= 0).  A separate launch from the mean: an earlier image
+// of the same list may still read the old value of a ring row that a later one commits to.
+template <bool VEC>
+__global__ void __launch_bounds__(STREAM_THREADS) stream_commit_kernel(const float *__restrict__ out,
+                                                                       float *__restrict__ ring,
+                                                                       const y2_stream_src *__restrict__ table,
+                                                                       int outputs)
+{
+    const int row = table[blockIdx.y].commit;
+    if (row < 0) return;
+    const float *src = out + (size_t)blockIdx.y * outputs;
+    float *dst = ring + (size_t)row * outputs;
+    const int base = blockIdx.x * STREAM_CHUNK;
+    if (VEC) {
+        const int e = base + threadIdx.x * 4;
+        if (e < outputs) *(float4 *)(dst + e) = __ldg((const float4 *)(src + e));
+    } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int e = base + q * STREAM_THREADS + threadIdx.x;
+            if (e < outputs) dst[e] = __ldg(src + e);
+        }
+    }
+}
+
 // classifier tail ------------------------------------------------------------------
 // avgpool_layer.c:40-55: sequential float sum over h*w, then / (h*w).  One thread per
 // (b, c) keeps the reference's summation order; reads are coalesced along c.
@@ -1208,6 +1285,83 @@ extern "C" int y2_region_boxes(float *pred, const float *d_biases, float *boxes,
 {
     return y2_region_boxes_counted(pred, d_biases, boxes, probs, batch, lw, lh, n, classes, img_w, img_h, thresh,
                                    only_objectness, classfix, tree_n, d_tree_parent, d_map, map_n, nullptr, s);
+}
+
+extern "C" int y2_stream_plan(int n, const int *stream_ids, int max_streams, int *frame_index, int *frames_seen,
+                              y2_stream_src *plan)
+{
+    if (n < 1 || !stream_ids || max_streams < 1 || !frame_index || !frames_seen || !plan) return Y2_EINVAL;
+    for (int i = 0; i < n; ++i)
+        if (stream_ids[i] < 0 || stream_ids[i] >= max_streams) return Y2_EINVAL;
+    // slot[i]: the ring slot image i writes, its stream's frame_index advanced by the stream's earlier images here
+    int *slot = (int *)malloc((size_t)n * sizeof(int));
+    if (!slot) return Y2_ENOMEM;
+    for (int i = 0; i < n; ++i) {
+        const int s = stream_ids[i];
+        int before = 0;
+        for (int k = 0; k < i; ++k) before += stream_ids[k] == s;
+        slot[i] = (frame_index[s] + before) % 3;
+    }
+    for (int i = 0; i < n; ++i) {
+        const int s = stream_ids[i];
+        for (int j = 0; j < 3; ++j) {
+            // the latest writer of slot j up to and including image i: this batch, else the ring as it stood
+            int code = frames_seen[s] > j ? -2 - (s * 3 + j) : -1;
+            for (int k = i; k >= 0; --k)
+                if (stream_ids[k] == s && slot[k] == j) {
+                    code = k;
+                    break;
+                }
+            plan[i].src[j] = code;
+        }
+        plan[i].commit = s * 3 + slot[i];
+        for (int k = i + 1; k < n; ++k)
+            if (stream_ids[k] == s && slot[k] == slot[i]) plan[i].commit = -1;
+    }
+    for (int i = 0; i < n; ++i) {
+        const int s = stream_ids[i];
+        frame_index[s] = (frame_index[s] + 1) % 3;
+        if (frames_seen[s] < 3) frames_seen[s]++;
+    }
+    free(slot);
+    return Y2_OK;
+}
+
+static bool stream_vec_ok(int outputs, const void *a, const void *b, const void *c)
+{
+    return outputs % 4 == 0 && (((uintptr_t)a | (uintptr_t)b | (uintptr_t)c) & 15) == 0;
+}
+
+extern "C" int y2_stream_mean(const float *out, const float *ring, const y2_stream_src *table, int n, int outputs,
+                              float *mean, y2_stream_t s)
+{
+    if (!out || !ring || !table || !mean || n < 1 || n > 65535 || outputs < 1) {
+        set_error("y2_stream_mean: invalid arguments (n=%d outputs=%d)", n, outputs);
+        return Y2_EINVAL;
+    }
+    const dim3 grid((outputs + STREAM_CHUNK - 1) / STREAM_CHUNK, n);
+    if (stream_vec_ok(outputs, out, ring, mean))
+        stream_mean_kernel<true><<<grid, STREAM_THREADS, 0, to_stream(s)>>>(out, ring, table, outputs, mean);
+    else
+        stream_mean_kernel<false><<<grid, STREAM_THREADS, 0, to_stream(s)>>>(out, ring, table, outputs, mean);
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
+}
+
+extern "C" int y2_stream_commit(const float *out, float *ring, const y2_stream_src *table, int n, int outputs,
+                                y2_stream_t s)
+{
+    if (!out || !ring || !table || n < 1 || n > 65535 || outputs < 1) {
+        set_error("y2_stream_commit: invalid arguments (n=%d outputs=%d)", n, outputs);
+        return Y2_EINVAL;
+    }
+    const dim3 grid((outputs + STREAM_CHUNK - 1) / STREAM_CHUNK, n);
+    if (stream_vec_ok(outputs, out, ring, ring))
+        stream_commit_kernel<true><<<grid, STREAM_THREADS, 0, to_stream(s)>>>(out, ring, table, outputs);
+    else
+        stream_commit_kernel<false><<<grid, STREAM_THREADS, 0, to_stream(s)>>>(out, ring, table, outputs);
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
 }
 
 // ws: caller-owned scratch of y2_collect_ws_bytes(batch, total, classes) bytes (per-box maxima of wide class

@@ -168,14 +168,14 @@ static layer *region_of(network net)
     return l;
 }
 
-/* get_region_boxes + do_nms_sort + the final pick for the whole batch on the network's stream: the decode
- * counts the NMS candidates while it writes the probabilities, the suppression pass marks losers negative
- * and the pick reads negative as zero (3 launches; the counters and scratch are the network's own) */
-static void detect_tail(y2_net_rt *rt, layer *l, void *head_rt, float thresh, float nms, y2_det *det_dev, int *cnt_dev,
-                        int det_cap)
+/* get_region_boxes + do_nms_sort + the final pick for the first B images of pred ([B][outputs], the region output or
+ * the 3-frame means of a streams batch) on the network's stream: the decode counts the NMS candidates while it writes
+ * the probabilities, the suppression pass marks losers negative and the pick reads negative as zero (3 launches; the
+ * counters and scratch are the network's own) */
+static void detect_tail(y2_net_rt *rt, layer *l, void *head_rt, float *pred, int B, float thresh, float nms,
+                        y2_det *det_dev, int *cnt_dev, int det_cap)
 {
     y2_layer_rt *r = (y2_layer_rt *)l->b200;
-    const int B = l->batch;
     const int total = l->w * l->h * l->n;
     if (l->softmax_tree && rt->defer_region) {
         /* softmax tree: only the groups on the path of classes above .5 are evaluated, straight from the head's
@@ -187,7 +187,7 @@ static void detect_tail(y2_net_rt *rt, layer *l, void *head_rt, float thresh, fl
         Y2_CHECK(y2_tree_nms_collect(r->tree_rec_dev, B, total, thresh, nms, det_dev, cnt_dev, det_cap, rt->stream));
         return;
     }
-    Y2_CHECK(y2_region_boxes_counted((float *)r->out, r->biases_dev, r->boxes_dev, r->probs_dev, B, l->w, l->h, l->n,
+    Y2_CHECK(y2_region_boxes_counted(pred, r->biases_dev, r->boxes_dev, r->probs_dev, B, l->w, l->h, l->n,
                                      l->classes, 1.f, 1.f, thresh, 0, l->classfix,
                                      l->softmax_tree ? l->softmax_tree->n : 0, r->tree_parent_dev, 0, 0,
                                      r->nms_cnt_dev, rt->stream));
@@ -217,7 +217,8 @@ void network_detect_device(network net, float thresh, float nms, y2_detection *d
         Y2_CHECK(y2_malloc((void **)&rt->cnt_dev, (size_t)rt->det_batch * sizeof(int)));
         Y2_CHECK(y2_host_alloc((void **)&rt->cnt_pinned, (size_t)rt->det_batch * sizeof(int)));
     }
-    detect_tail(rt, l, net.layers[net.n - 2].b200, thresh, nms, rt->det_dev, rt->cnt_dev, rt->det_cap);
+    detect_tail(rt, l, net.layers[net.n - 2].b200, (float *)((y2_layer_rt *)l->b200)->out, B, thresh, nms, rt->det_dev,
+                rt->cnt_dev, rt->det_cap);
     Y2_CHECK(y2_memcpy_d2h(rt->cnt_pinned, rt->cnt_dev, (size_t)B * sizeof(int), rt->stream));
     Y2_CHECK(y2_memcpy_d2h(rt->det_pinned, rt->det_dev, (size_t)B * rt->det_cap * sizeof(y2_det), rt->stream));
     Y2_CHECK(y2_stream_sync(rt->stream));
@@ -480,18 +481,134 @@ static void submit_done(y2_net_rt *rt, int s, int kind, int n_images)
     rt->pipe_inflight++;
 }
 
-static int submit_common(network net, const void *input, int u8, int fw, int fh, float thresh, float nms,
-                         int max_det)
+/* ---- video streams: each image is decoded on the 3-frame mean of its stream (yolo_v2_class.cpp:206-216) ------- */
+static layer *streams_region(network net)
+{
+    layer *l = region_of(net);
+    if (l->softmax_tree || y2_rt(net)->defer_region)
+        error("network streams: needs a flat-softmax region head (a softmax tree defers the region forward, so there "
+              "is no dense region output to average)");
+    return l;
+}
+
+/* the refusals of every streams submission, before anything is staged */
+static void check_streams(network net, int n, const int *stream_ids)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network streams: network has no device plan");
+    const layer *l = streams_region(net);
+    const y2_streams *st = rt->streams;
+    if (!st) error("network streams: streams not opened, call network_streams_open");
+    if (l->outputs != st->outputs)
+        error("network streams: the region output size differs from the one the streams were opened with (after "
+              "resize_network, open them again)");
+    if (n < 1 || n > net.batch) error("network streams: the list must hold 1 .. batch images");
+    if (!stream_ids) error("network streams: NULL stream id array");
+    for (int i = 0; i < n; ++i)
+        if (stream_ids[i] < 0 || stream_ids[i] >= st->max_streams)
+            error("network streams: a stream id outside 0 .. max_streams-1");
+}
+
+void y2_streams_free(y2_net_rt *rt)
+{
+    y2_streams *st = rt->streams;
+    if (!st) return;
+    y2_free(st->ring_dev);
+    y2_free(st->mean_dev);
+    for (int s = 0; s < 2; ++s) {
+        y2_free(st->table_dev[s]);
+        y2_host_free(st->table_pinned[s]);
+    }
+    free(st->frame_index);
+    free(st->frames_seen);
+    free(st);
+    rt->streams = NULL;
+}
+
+void network_streams_open(network net, int max_streams)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network_streams_open: network has no device plan");
+    if (max_streams < 1) error("network_streams_open: max_streams must be 1 or more");
+    const layer *l = streams_region(net);
+    Y2_CHECK(y2_set_device(rt->device));
+    Y2_CHECK(y2_stream_sync(rt->stream)); /* batches in flight read and write the old ring */
+    y2_streams_free(rt);
+    y2_streams *st = (y2_streams *)calloc(1, sizeof(y2_streams));
+    if (!st) error("network_streams_open: out of host memory");
+    st->max_streams = max_streams;
+    st->outputs = l->outputs;
+    st->frame_index = (int *)calloc((size_t)max_streams, sizeof(int));
+    st->frames_seen = (int *)calloc((size_t)max_streams, sizeof(int));
+    if (!st->frame_index || !st->frames_seen) error("network_streams_open: out of host memory");
+    /* not cleared: a ring row is read only after it was written (y2_stream_plan reads unwritten slots as zero) */
+    Y2_CHECK(y2_malloc((void **)&st->ring_dev, (size_t)max_streams * 3 * l->outputs * sizeof(float)));
+    rt->streams = st;
+}
+
+void network_stream_reset(network net, int stream)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network_stream_reset: network has no device plan");
+    y2_streams *st = rt->streams;
+    if (!st) error("network_stream_reset: streams not opened, call network_streams_open");
+    if (stream < 0 || stream >= st->max_streams) error("network_stream_reset: a stream id outside 0 .. max_streams-1");
+    /* host only: batches already submitted keep the table they were given */
+    st->frame_index[stream] = 0;
+    st->frames_seen[stream] = 0;
+}
+
+/* A streams batch into slot s: its ring plan in the slot's table, copied on the copy stream (ahead of the slot's
+ * input copies, so the slot's ev_h2d covers it) */
+static void streams_stage(y2_net_rt *rt, int s, int n, const int *stream_ids, int batch)
+{
+    y2_streams *st = rt->streams;
+    const int cap_b = batch > rt->cap_batch ? batch : rt->cap_batch;
+    if (st->mean_cap < batch) {
+        Y2_CHECK(y2_stream_sync(rt->stream)); /* the other slot's decode may still read the means */
+        y2_free(st->mean_dev);
+        Y2_CHECK(y2_malloc((void **)&st->mean_dev, (size_t)cap_b * st->outputs * sizeof(float)));
+        st->mean_cap = cap_b;
+    }
+    if (st->table_cap[s] < batch) {
+        y2_free(st->table_dev[s]);
+        y2_host_free(st->table_pinned[s]);
+        Y2_CHECK(y2_malloc((void **)&st->table_dev[s], (size_t)cap_b * sizeof(y2_stream_src)));
+        Y2_CHECK(y2_host_alloc((void **)&st->table_pinned[s], (size_t)cap_b * sizeof(y2_stream_src)));
+        st->table_cap[s] = cap_b;
+    }
+    Y2_CHECK(y2_stream_plan(n, stream_ids, st->max_streams, st->frame_index, st->frames_seen, st->table_pinned[s]));
+    Y2_CHECK(y2_memcpy_h2d(st->table_dev[s], st->table_pinned[s], (size_t)n * sizeof(y2_stream_src), rt->copy_stream));
+}
+
+/* n images come back.  stream_ids (n of them): a streams batch, decoded on the 3-frame means; else the tail runs on
+ * the region output of all B images. */
+static int submit_common(network net, const void *input, int u8, int fw, int fh, int n, const int *stream_ids,
+                         float thresh, float nms, int max_det)
 {
     const int s = submit_slot(net, u8, fw, fh);
     y2_net_rt *rt = y2_rt(net);
     struct y2_pipe_slot *ps = &rt->pipe[s];
     layer *l = region_of(net);
+    y2_layer_rt *r = (y2_layer_rt *)l->b200;
+    void *head_rt = net.layers[net.n - 2].b200;
     const int B = net.batch;
-    const int n = u8 == 4 ? ((const frame_list *)input)->n : B; /* the tail runs on all B, n come back */
     pipe_reserve_dets(rt, s, B, max_det);
+    if (stream_ids) streams_stage(rt, s, n, stream_ids, B);
     submit_input(net, s, input, u8, fw, fh, 0);
-    detect_tail(rt, l, net.layers[net.n - 2].b200, thresh, nms, ps->det_dev, ps->cnt_dev, ps->det_cap);
+    if (stream_ids) {
+        y2_streams *st = rt->streams;
+        if (u8 == 3) { /* no input copy: the compute stream waits for the table alone */
+            Y2_CHECK(y2_event_record(ps->ev_h2d, rt->copy_stream));
+            Y2_CHECK(y2_stream_wait_event(rt->stream, ps->ev_h2d));
+        }
+        Y2_CHECK(y2_stream_mean((const float *)r->out, st->ring_dev, st->table_dev[s], n, st->outputs, st->mean_dev,
+                                rt->stream));
+        Y2_CHECK(y2_stream_commit((const float *)r->out, st->ring_dev, st->table_dev[s], n, st->outputs, rt->stream));
+        detect_tail(rt, l, head_rt, st->mean_dev, n, thresh, nms, ps->det_dev, ps->cnt_dev, ps->det_cap);
+    } else {
+        detect_tail(rt, l, head_rt, (float *)r->out, B, thresh, nms, ps->det_dev, ps->cnt_dev, ps->det_cap);
+    }
     submit_results(rt, s);
     Y2_CHECK(y2_memcpy_d2h(ps->cnt_pinned, ps->cnt_dev, (size_t)n * sizeof(int), rt->d2h_stream));
     Y2_CHECK(y2_memcpy_d2h(ps->det_pinned, ps->det_dev, (size_t)n * ps->det_cap * sizeof(y2_det), rt->d2h_stream));
@@ -501,19 +618,19 @@ static int submit_common(network net, const void *input, int u8, int fw, int fh,
 
 int network_detect_submit(network net, const float *input, float thresh, float nms, int max_det)
 {
-    return submit_common(net, input, 0, 0, 0, thresh, nms, max_det);
+    return submit_common(net, input, 0, 0, 0, net.batch, NULL, thresh, nms, max_det);
 }
 
 int network_detect_submit_u8(network net, const unsigned char *input_hwc, float thresh, float nms, int max_det)
 {
-    return submit_common(net, input_hwc, 1, 0, 0, thresh, nms, max_det);
+    return submit_common(net, input_hwc, 1, 0, 0, net.batch, NULL, thresh, nms, max_det);
 }
 
 /* The batch is already in the slot's device input (network_pipeline_input_device(net, slot), e.g. written by another
  * kernel or uploaded once): forward + decode + NMS + pick without any host -> device copy, pipelined like the others. */
 int network_detect_submit_resident(network net, float thresh, float nms, int max_det)
 {
-    return submit_common(net, 0, 3, 0, 0, thresh, nms, max_det);
+    return submit_common(net, 0, 3, 0, 0, net.batch, NULL, thresh, nms, max_det);
 }
 
 float *network_pipeline_input_device(network net, int slot)
@@ -551,7 +668,7 @@ void network_detect_batch_u8(network net, const unsigned char *input_hwc, float 
 {
     y2_net_rt *rt = y2_rt(net);
     if (rt && rt->pipe_inflight) error("network_detect_batch_u8: batches of the submit/wait pipeline are in flight");
-    submit_common(net, input_hwc, 1, 0, 0, thresh, nms, max_det);
+    submit_common(net, input_hwc, 1, 0, 0, net.batch, NULL, thresh, nms, max_det);
     network_detect_wait(net, dets, counts, max_det);
 }
 
@@ -572,8 +689,9 @@ int network_detect_submit_frames(network net, const unsigned char *frames_hwc, i
 {
     y2_net_rt *rt = y2_rt(net);
     if (!rt) error("network_detect_submit_frames: network has no device plan");
-    if (frames_take_u8(net, frame_w, frame_h)) return submit_common(net, frames_hwc, 1, 0, 0, thresh, nms, max_det);
-    return submit_common(net, frames_hwc, 2, frame_w, frame_h, thresh, nms, max_det);
+    if (frames_take_u8(net, frame_w, frame_h))
+        return submit_common(net, frames_hwc, 1, 0, 0, net.batch, NULL, thresh, nms, max_det);
+    return submit_common(net, frames_hwc, 2, frame_w, frame_h, net.batch, NULL, thresh, nms, max_det);
 }
 
 int network_detect_submit_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
@@ -581,7 +699,7 @@ int network_detect_submit_frame_list(network net, int n, const unsigned char *co
 {
     const frame_list fl = {n, frames, frame_w, frame_h};
     check_frame_list(net, &fl);
-    return submit_common(net, &fl, 4, 0, 0, thresh, nms, max_det);
+    return submit_common(net, &fl, 4, 0, 0, n, NULL, thresh, nms, max_det);
 }
 
 void network_detect_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
@@ -592,6 +710,33 @@ void network_detect_batch_frame_list(network net, int n, const unsigned char *co
     if (rt && rt->pipe_inflight)
         error("network_detect_batch_frame_list: batches of the submit/wait pipeline are in flight");
     network_detect_submit_frame_list(net, n, frames, frame_w, frame_h, thresh, nms, max_det);
+    network_detect_wait(net, dets, counts, max_det);
+}
+
+int network_detect_submit_streams(network net, int n, const int *stream_ids, const unsigned char *const *frames,
+                                  const int *frame_w, const int *frame_h, float thresh, float nms, int max_det)
+{
+    const frame_list fl = {n, frames, frame_w, frame_h};
+    check_frame_list(net, &fl);
+    check_streams(net, n, stream_ids);
+    return submit_common(net, &fl, 4, 0, 0, n, stream_ids, thresh, nms, max_det);
+}
+
+int network_detect_submit_streams_resident(network net, int n, const int *stream_ids, float thresh, float nms,
+                                           int max_det)
+{
+    check_streams(net, n, stream_ids);
+    return submit_common(net, 0, 3, 0, 0, n, stream_ids, thresh, nms, max_det);
+}
+
+void network_detect_batch_streams(network net, int n, const int *stream_ids, const unsigned char *const *frames,
+                                  const int *frame_w, const int *frame_h, float thresh, float nms,
+                                  y2_detection *dets, int *counts, int max_det)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (rt && rt->pipe_inflight)
+        error("network_detect_batch_streams: batches of the submit/wait pipeline are in flight");
+    network_detect_submit_streams(net, n, stream_ids, frames, frame_w, frame_h, thresh, nms, max_det);
     network_detect_wait(net, dets, counts, max_det);
 }
 

@@ -75,8 +75,23 @@ typedef struct y2_layer_rt {
     y2_event_t ev0, ev1;
 } y2_layer_rt;
 
+/* video streams of network_detect_submit_streams (network_streams_open).  They outlive a re-plan
+ * (set_batch_network, resize_network) and are freed with the network. */
+typedef struct y2_streams {
+    int max_streams;
+    int outputs;           /* region outputs per image when opened */
+    float *ring_dev;       /* [max_streams][3][outputs], rows defined once written (y2_stream_plan never reads others) */
+    int *frame_index;      /* [max_streams] ring slot of the stream's next frame */
+    int *frames_seen;      /* [max_streams] frames since open / reset, saturating at 3 */
+    float *mean_dev;       /* [mean_cap][outputs] the means the decode reads */
+    int mean_cap;
+    y2_stream_src *table_pinned[2], *table_dev[2]; /* per pipeline slot, table_cap[slot] records */
+    int table_cap[2];
+} y2_streams;
+
 typedef struct y2_net_rt {
     int device;
+    y2_streams *streams; /* NULL until network_streams_open */
     y2_stream_t stream;
     int cap_batch;       /* batch the buffers were sized for */
     int plan_batch;      /* batch the plans/tensor maps were built for */
@@ -143,6 +158,9 @@ void y2_push_convolutional_layer(layer *l);
 int y2_output_layer_index(network net);
 void y2_run_forward_from(network net, float *in_dev, y2_graph_t *graph, int *graph_valid);
 void y2_pipe_release(y2_net_rt *rt);
+
+/* y2_detect.c */
+void y2_streams_free(y2_net_rt *rt);
 
 /* layer constructors, per-layer forwards and resizes: declared in include/darknet_b200.h */
 void forward_no_cpu_path(layer l, network_state state);

@@ -547,6 +547,7 @@ void y2_unplan_network(network *net)
     y2_host_free(rt->hits_pinned);
     y2_free(rt->export_dev);
     pipe_free(rt);
+    y2_streams_free(rt);
     y2_stream_destroy(rt->stream);
     free(rt);
     net->b200 = 0;
@@ -818,11 +819,19 @@ static void build_plans(network *net, int batch)
 
 void y2_plan_network(network *net)
 {
+    /* the video streams outlive the re-plan (set_batch_network, resize_network) when the device stays the same */
+    y2_streams *streams = NULL;
+    y2_net_rt *old = (y2_net_rt *)net->b200;
+    if (old && old->device == net->gpu_index) {
+        streams = old->streams;
+        old->streams = NULL;
+    }
     if (net->b200) y2_unplan_network(net);
     Y2_CHECK(y2_set_device(net->gpu_index));
     y2_net_rt *rt = (y2_net_rt *)calloc(1, sizeof(y2_net_rt));
     net->b200 = rt;
     rt->device = net->gpu_index;
+    rt->streams = streams;
     Y2_CHECK(y2_stream_create(&rt->stream));
     const int B = net->batch;
     rt->cap_batch = B;
@@ -1849,6 +1858,7 @@ void free_network(network net)
         y2_host_free(rt->hits_pinned);
         y2_free(rt->export_dev);
         pipe_free(rt);
+        y2_streams_free(rt);
         y2_stream_destroy(rt->stream);
         free(rt);
         (void)tmp;

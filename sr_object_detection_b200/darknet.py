@@ -167,6 +167,12 @@ def lib() -> C.CDLL:
         "network_detect_submit_frame_list": (i, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f, i]),
         "network_detect_batch_frame_list": (None, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f,
                                                    C.POINTER(Detection), _ip, i]),
+        "network_streams_open": (None, [Network, i]),
+        "network_stream_reset": (None, [Network, i]),
+        "network_detect_submit_streams": (i, [Network, i, _ip, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f, i]),
+        "network_detect_submit_streams_resident": (i, [Network, i, _ip, f, f, i]),
+        "network_detect_batch_streams": (None, [Network, i, _ip, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f,
+                                                C.POINTER(Detection), _ip, i]),
         "network_classify_submit_frame_list": (i, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i]),
         "network_classify_batch_frame_list": (None, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i,
                                                      C.POINTER(ClassHit)]),
@@ -412,6 +418,49 @@ def network_detect_wait_n(net: Network, n: int, max_det: int = 256):
     counts = (C.c_int * net.batch)()
     lib().network_detect_wait(net, dets, counts, max_det)
     return _det_lists(dets, counts, n, max_det)
+
+
+def network_streams_open(net: Network, max_streams: int) -> None:
+    """Extension: (re)open streams 0 .. max_streams-1 for the 3-frame-mean entries, every one starting over."""
+    lib().network_streams_open(net, max_streams)
+
+
+def network_stream_reset(net: Network, stream: int) -> None:
+    lib().network_stream_reset(net, stream)
+
+
+def _stream_ids(stream_ids, n: int):
+    ids = [int(s) for s in stream_ids]
+    assert len(ids) == n, (len(ids), n)
+    return (C.c_int * max(n, 1))(*ids)
+
+
+def network_detect_streams(net: Network, stream_ids, frames, thresh: float, nms: float, max_det: int = 256):
+    """Extension: detection on a list of decoded frames (uint8 [h][w][3] arrays of their own sizes), frame i from
+    video stream stream_ids[i] and decoded on that stream's 3-frame mean, as Detector::detect(img, thresh,
+    use_mean = true).  Returns (per-image detection arrays, counts) for len(frames) images."""
+    n, ptrs, fw, fh = _frame_list_args(frames)
+    dets = (Detection * (max(n, 1) * max_det))()
+    counts = (C.c_int * max(n, 1))()
+    lib().network_detect_batch_streams(net, n, _stream_ids(stream_ids, n), ptrs, fw, fh, thresh, nms, dets, counts,
+                                       max_det)
+    return _det_lists(dets, counts, n, max_det)
+
+
+def network_detect_submit_streams(net: Network, stream_ids, frames, thresh: float, nms: float,
+                                  max_det: int = 256) -> int:
+    """Queue a streams frame list on the submit/wait pipeline; network_detect_wait_n(net, len(frames), ...) collects
+    it."""
+    n, ptrs, fw, fh = _frame_list_args(frames)
+    return lib().network_detect_submit_streams(net, n, _stream_ids(stream_ids, n), ptrs, fw, fh, thresh, nms, max_det)
+
+
+def network_detect_submit_streams_resident(net: Network, stream_ids, thresh: float, nms: float,
+                                           max_det: int = 256) -> int:
+    """The same with the first len(stream_ids) images already in the slot's device input
+    (network_pipeline_input_device)."""
+    n = len(stream_ids)
+    return lib().network_detect_submit_streams_resident(net, n, _stream_ids(stream_ids, n), thresh, nms, max_det)
 
 
 def network_classify_batch(net: Network, images: np.ndarray | None = None, frames: np.ndarray | None = None,
