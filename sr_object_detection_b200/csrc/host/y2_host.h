@@ -89,6 +89,36 @@ typedef struct y2_streams {
     int table_cap[2];
 } y2_streams;
 
+/* what a batch hands back, each a device buffer with a pinned mirror (y2_pipeline.c) */
+typedef struct y2_results {
+    y2_det *det_dev, *det_pinned;         /* [det_images][det_cap] detection lists */
+    int *cnt_dev, *cnt_pinned;            /* [det_images] detections per image */
+    int det_cap, det_images;
+    y2_class_hit *hits_dev, *hits_pinned; /* [cap_batch][hits_cap] class hits */
+    int hits_cap;
+} y2_results;
+
+/* what a submission feeds the network; y2_pipe_claim completes it */
+typedef enum {
+    Y2_IN_F32,        /* fp32 planar [B][c][h][w] */
+    Y2_IN_U8,         /* uint8 interleaved RGB [B][h][w][3] at the network's resolution */
+    Y2_IN_FRAMES,     /* uint8 interleaved RGB frames [B][fh][fw][3] of any size */
+    Y2_IN_FRAME_LIST, /* 1 .. B frames of their own sizes */
+    Y2_IN_RESIDENT,   /* nothing: the slot's device input already holds the batch */
+} y2_input_kind;
+
+typedef struct {
+    y2_input_kind kind;
+    const void *data;          /* NULL: already in the slot's pinned staging buffer */
+    int fw, fh;                /* Y2_IN_FRAMES */
+    struct y2_frame_list {     /* Y2_IN_FRAME_LIST: n frames of their own sizes */
+        int n;
+        const unsigned char *const *frames;
+        const int *w, *h;
+    } list;
+    int n;                     /* images the batch hands back: the list's length, else the batch */
+} y2_input;
+
 typedef struct y2_net_rt {
     int device;
     y2_streams *streams; /* NULL until network_streams_open */
@@ -96,48 +126,35 @@ typedef struct y2_net_rt {
     int cap_batch;       /* batch the buffers were sized for */
     int plan_batch;      /* batch the plans/tensor maps were built for */
     int plan_w, plan_h;
-    float *in_dev;       /* fp32 NCHW input */
-    float *in_pinned;
-    size_t in_bytes;
+    size_t in_bytes;     /* of a slot's fp32 input */
     float *out_pinned;   /* staging of the network output */
     size_t out_bytes;
-    y2_graph_t graph;
-    int graph_valid;
     int eager;
     int launches;
     int profile;
-    /* detection scratch */
-    y2_det *det_dev, *det_pinned;
-    int *cnt_dev, *cnt_pinned;
-    int det_cap, det_batch;
-    /* class hits of network_classify_device, room for cap_batch x hits_cap */
-    y2_class_hit *hits_dev, *hits_pinned;
-    int hits_cap;
+    y2_results res;      /* of network_detect_device / network_classify_device */
     float *export_dev;   /* fp32 scratch for layer export */
     size_t export_bytes;
-    /* two-deep submit/wait pipeline (network_detect_submit): slot 0 shares in_dev / in_pinned / graph
-     * with the synchronous path, slot 1 has its own input buffers and graph */
+    /* two-deep submit/wait pipeline (y2_pipeline.c).  Slot 0's fp32 input and graph are also the synchronous
+     * path's (network_upload_input, network_forward_device) and exist from plan time on; everything else in a slot
+     * is allocated at first use.  The graphs go when the plans are rebuilt (set_batch_network), the rest with the
+     * network's device plan. */
     struct y2_pipe_slot {
-        float *in_dev, *in_pinned;
+        float *in_dev, *in_pinned; /* fp32 NCHW input */
         y2_graph_t graph;
         int graph_valid;
-        y2_det *det_dev, *det_pinned;
-        int *cnt_dev, *cnt_pinned;
-        int det_cap;
-        y2_event_t ev_h2d, ev_tail, ev_done;
-        int busy;
-        /* raw uint8 HWC input of the same slot (network_detect_submit_u8) */
+        /* raw uint8 HWC input of the same slot (Y2_IN_U8) */
         unsigned char *in_u8_dev, *in_u8_pinned;
         y2_graph_t graph_u8;
         int graph_u8_valid;
-        /* decoded frames of any size (network_detect_submit_frames): resized on the device into in_dev */
+        /* decoded frames of any size or a frame list: resized or letterboxed on the device into in_dev */
         unsigned char *frames_dev, *frames_pinned;
         size_t frames_cap;
+        y2_results res;
+        y2_event_t ev_h2d, ev_tail, ev_done;
         int kind;           /* Y2_PIPE_* of the batch in the slot */
-        int n_images;       /* images the wait hands back: the list length of a frame list, else the batch */
-        /* class hits of a classify batch ([B][hits_top]), room for cap_batch x hits_cap */
-        y2_class_hit *hits_dev, *hits_pinned;
-        int hits_cap, hits_top;
+        int n_images;       /* images the wait hands back */
+        int top;            /* hits per image of a classify batch, 0 for a detection batch */
     } pipe[2];
     y2_stream_t copy_stream; /* host -> device uploads of the pipeline */
     y2_stream_t d2h_stream;  /* detection lists back to the host, under the next batch's forward pass */
@@ -157,7 +174,19 @@ void y2_unplan_network(network *net);
 void y2_push_convolutional_layer(layer *l);
 int y2_output_layer_index(network net);
 void y2_run_forward_from(network net, float *in_dev, y2_graph_t *graph, int *graph_valid);
+
+/* y2_pipeline.c */
 void y2_pipe_release(y2_net_rt *rt);
+void y2_pipe_free(y2_net_rt *rt);
+int y2_pipe_claim(network net, y2_input *in);
+void y2_pipe_submit_input(network net, int s, const y2_input *in, int letterbox);
+void y2_pipe_queue(y2_net_rt *rt, int s, int kind, int n_images, int top);
+int y2_pipe_retire(network net, int kind, int top);
+void y2_results_reserve_dets(y2_net_rt *rt, y2_results *res, int batch, int max_det);
+void y2_results_reserve_hits(y2_net_rt *rt, y2_results *res, int top);
+void y2_results_to_host(const y2_results *res, int n, int top, y2_stream_t stream);
+void y2_results_copy_dets(const y2_results *res, int n, y2_detection *dets, int *counts, int max_det);
+void y2_results_free(y2_results *res);
 
 /* y2_detect.c */
 void y2_streams_free(y2_net_rt *rt);

@@ -526,8 +526,6 @@ static void free_layer_rt(layer *l)
     l->weights_gpu = 0;
 }
 
-static void pipe_free(y2_net_rt *rt);
-
 void y2_unplan_network(network *net)
 {
     y2_net_rt *rt = (y2_net_rt *)net->b200;
@@ -535,18 +533,10 @@ void y2_unplan_network(network *net)
     Y2_CHECK(y2_set_device(rt->device));
     y2_stream_sync(rt->stream);
     for (int i = 0; i < net->n; ++i) free_layer_rt(&net->layers[i]);
-    if (rt->graph) y2_graph_destroy(rt->graph);
-    y2_free(rt->in_dev);
-    y2_host_free(rt->in_pinned);
     y2_host_free(rt->out_pinned);
-    y2_free(rt->det_dev);
-    y2_host_free(rt->det_pinned);
-    y2_free(rt->cnt_dev);
-    y2_host_free(rt->cnt_pinned);
-    y2_free(rt->hits_dev);
-    y2_host_free(rt->hits_pinned);
+    y2_results_free(&rt->res);
     y2_free(rt->export_dev);
-    pipe_free(rt);
+    y2_pipe_free(rt);
     y2_streams_free(rt);
     y2_stream_destroy(rt->stream);
     free(rt);
@@ -809,11 +799,6 @@ static void build_plans(network *net, int batch)
         else if (net->layers[i].type == CONNECTED) build_fc_plan(net, i, batch);
     }
     rt->plan_batch = batch;
-    if (rt->graph) {
-        y2_graph_destroy(rt->graph);
-        rt->graph = 0;
-    }
-    rt->graph_valid = 0;
     y2_pipe_release(rt);
 }
 
@@ -838,8 +823,8 @@ void y2_plan_network(network *net)
     rt->plan_w = net->w;
     rt->plan_h = net->h;
     rt->in_bytes = (size_t)B * net->inputs * sizeof(float);
-    Y2_CHECK(y2_malloc((void **)&rt->in_dev, rt->in_bytes));
-    Y2_CHECK(y2_host_alloc((void **)&rt->in_pinned, rt->in_bytes));
+    Y2_CHECK(y2_malloc((void **)&rt->pipe[0].in_dev, rt->in_bytes)); /* also the synchronous path's input */
+    Y2_CHECK(y2_host_alloc((void **)&rt->pipe[0].in_pinned, rt->in_bytes));
 
     /* pass 1: per-layer storage decisions */
     for (int i = 0; i < net->n; ++i) {
@@ -1477,48 +1462,7 @@ void y2_run_forward_from(network net, float *in_dev, y2_graph_t *graph, int *gra
 static void run_forward(network net)
 {
     y2_net_rt *rt = y2_rt(net);
-    y2_run_forward_from(net, rt->in_dev, &rt->graph, &rt->graph_valid);
-}
-
-/* pipeline state that does not survive a re-plan / batch change */
-void y2_pipe_release(y2_net_rt *rt)
-{
-    if (rt->pipe[1].graph) y2_graph_destroy(rt->pipe[1].graph);
-    rt->pipe[1].graph = 0;
-    rt->pipe[1].graph_valid = 0;
-    for (int s = 0; s < 2; ++s) {
-        if (rt->pipe[s].graph_u8) y2_graph_destroy(rt->pipe[s].graph_u8);
-        rt->pipe[s].graph_u8 = 0;
-        rt->pipe[s].graph_u8_valid = 0;
-    }
-}
-
-static void pipe_free(y2_net_rt *rt)
-{
-    y2_pipe_release(rt);
-    y2_free(rt->pipe[1].in_dev);
-    y2_host_free(rt->pipe[1].in_pinned);
-    for (int s = 0; s < 2; ++s) {
-        y2_free(rt->pipe[s].in_u8_dev);
-        y2_host_free(rt->pipe[s].in_u8_pinned);
-        y2_free(rt->pipe[s].frames_dev);
-        y2_host_free(rt->pipe[s].frames_pinned);
-        y2_free(rt->pipe[s].det_dev);
-        y2_host_free(rt->pipe[s].det_pinned);
-        y2_free(rt->pipe[s].cnt_dev);
-        y2_host_free(rt->pipe[s].cnt_pinned);
-        y2_free(rt->pipe[s].hits_dev);
-        y2_host_free(rt->pipe[s].hits_pinned);
-        if (rt->pipe[s].ev_h2d) y2_event_destroy(rt->pipe[s].ev_h2d);
-        if (rt->pipe[s].ev_done) y2_event_destroy(rt->pipe[s].ev_done);
-        if (rt->pipe[s].ev_tail) y2_event_destroy(rt->pipe[s].ev_tail);
-    }
-    if (rt->copy_stream) y2_stream_destroy(rt->copy_stream);
-    if (rt->d2h_stream) y2_stream_destroy(rt->d2h_stream);
-    memset(rt->pipe, 0, sizeof(rt->pipe));
-    rt->copy_stream = 0;
-    rt->d2h_stream = 0;
-    rt->pipe_ready = 0;
+    y2_run_forward_from(net, rt->pipe[0].in_dev, &rt->pipe[0].graph, &rt->pipe[0].graph_valid);
 }
 
 void network_set_eager(network net, int eager)
@@ -1558,13 +1502,13 @@ void network_sync(network net)
 float *network_input_staging(network net)
 {
     y2_net_rt *rt = y2_rt(net);
-    return rt ? rt->in_pinned : 0;
+    return rt ? rt->pipe[0].in_pinned : 0;
 }
 
 float *network_input_device(network net)
 {
     y2_net_rt *rt = y2_rt(net);
-    return rt ? rt->in_dev : 0;
+    return rt ? rt->pipe[0].in_dev : 0;
 }
 
 void network_upload_input(network net, const float *input)
@@ -1574,11 +1518,11 @@ void network_upload_input(network net, const float *input)
     const size_t bytes = (size_t)net.batch * net.inputs * sizeof(float);
     /* caller memory is pageable in the reference API: stage through the pinned buffer, unless the
      * caller already filled the staging buffer itself (network_input_staging) */
-    if (input && input != rt->in_pinned) {
+    if (input && input != rt->pipe[0].in_pinned) {
         Y2_CHECK(y2_stream_sync(rt->stream));
-        memcpy(rt->in_pinned, input, bytes);
+        memcpy(rt->pipe[0].in_pinned, input, bytes);
     }
-    Y2_CHECK(y2_memcpy_h2d(rt->in_dev, rt->in_pinned, bytes, rt->stream));
+    Y2_CHECK(y2_memcpy_h2d(rt->pipe[0].in_dev, rt->pipe[0].in_pinned, bytes, rt->stream));
 }
 
 /* struct sizes for language bindings that pass network/layer by value (ctypes, cgo ...) */
@@ -1656,7 +1600,8 @@ static float *export_layer(network net, int i)
         d.out = full; d.out_cs = r->cpad; d.out_mode = Y2_OUT_BF16_PADDED;
         y2_conv_plan *plan = 0;
         Y2_CHECK(y2_conv_plan_create(&d, &plan));
-        Y2_CHECK(y2_pack_patches_f32(rt->in_dev, patches, net.batch, l->c, l->h, l->w, l->size, r->kpad, rt->stream));
+        Y2_CHECK(y2_pack_patches_f32(rt->pipe[0].in_dev, patches, net.batch, l->c, l->h, l->w, l->size, r->kpad,
+                                     rt->stream));
         Y2_CHECK(y2_conv_plan_launch(plan, rt->stream));
         Y2_CHECK(y2_unpack_to_nchw_f32(full, rt->export_dev, net.batch, l->out_c, l->out_h, l->out_w, r->cpad,
                                        rt->stream));
@@ -1839,30 +1784,7 @@ void free_layer(layer l)
 
 void free_network(network net)
 {
-    if (net.b200) {
-        y2_net_rt *rt = y2_rt(net);
-        Y2_CHECK(y2_set_device(rt->device));
-        y2_stream_sync(rt->stream);
-        network tmp = net;
-        /* layers are freed below; release the network-level device state first */
-        for (int i = 0; i < net.n; ++i) free_layer_rt(&net.layers[i]);
-        if (rt->graph) y2_graph_destroy(rt->graph);
-        y2_free(rt->in_dev);
-        y2_host_free(rt->in_pinned);
-        y2_host_free(rt->out_pinned);
-        y2_free(rt->det_dev);
-        y2_host_free(rt->det_pinned);
-        y2_free(rt->cnt_dev);
-        y2_host_free(rt->cnt_pinned);
-        y2_free(rt->hits_dev);
-        y2_host_free(rt->hits_pinned);
-        y2_free(rt->export_dev);
-        pipe_free(rt);
-        y2_streams_free(rt);
-        y2_stream_destroy(rt->stream);
-        free(rt);
-        (void)tmp;
-    }
+    y2_unplan_network(&net); /* the network-level device state first, the layers below */
     for (int i = 0; i < net.n; ++i) free_layer(net.layers[i]);
     free(net.layers);
     free(net.seen);
