@@ -449,6 +449,47 @@ int network_detect_submit_streams_resident(network net, int n, const int *stream
 void network_detect_batch_streams(network net, int n, const int *stream_ids, const unsigned char *const *frames,
                                   const int *frame_w, const int *frame_h, float thresh, float nms,
                                   y2_detection *dets, int *counts, int max_det);
+/* ---- tracked streams: per stream the result is bit-identical to Detector::detect(img, thresh, use_mean) followed by
+ * Detector::tracking(result, frames_story) (yolo_v2_class.cpp:173-304) on that stream's frames in order: boxes in the
+ * frame's pixels, each with a track id that stays the same across frames (ids start at 1 per class and stream). */
+#ifndef Y2_BBOX_DEFINED
+#define Y2_BBOX_DEFINED
+typedef struct y2_bbox { /* bbox_t (yolo_v2_class.hpp:27-33) */
+    unsigned int x, y, w, h;
+    float prob;
+    unsigned int obj_id, track_id;
+} y2_bbox;
+#endif
+#ifndef Y2_TRACK_MAX_STORY
+#define Y2_TRACK_MAX_STORY 32
+#endif
+#ifndef Y2_TRACK_MAX_TOTAL
+#define Y2_TRACK_MAX_TOTAL 7168
+#endif
+/* Turns tracking on for the opened streams (1 <= frames_story <= Y2_TRACK_MAX_STORY; the Detector's default is 6) and
+ * starts every track over; refused for a region of more than Y2_TRACK_MAX_TOTAL boxes per image (l.w * l.h * l.n).
+ * The history and ids live on the device.  network_streams_open drops them (call this
+ * again after it); set_batch_network keeps them; network_stream_reset also starts that stream's tracks over.
+ * frames_story is fixed until the next call: a Detector whose story shrinks between calls drops one frame per call,
+ * which is not reproduced. */
+void network_streams_track(network net, int frames_story);
+/* As network_detect_submit_streams, frame i of frame_w[i] x frame_h[i] pixels.  use_mean 1 decodes on the stream's
+ * 3-frame mean and advances its ring; use_mean 0 decodes the plain region output and leaves the ring alone.  Either
+ * way the tracks advance.  Tracking sees every detection; max_det caps only what is copied out, counts hold the full
+ * number.  Collected by network_detect_wait_tracked (n images, boxes [n][max_det]). */
+int network_detect_submit_streams_tracked(network net, int n, const int *stream_ids, const unsigned char *const *frames,
+                                          const int *frame_w, const int *frame_h, float thresh, float nms,
+                                          int use_mean, int max_det);
+/* The same with the batch already in the slot's device input; frame_w / frame_h are the pixel sizes the boxes are
+ * scaled to. */
+int network_detect_submit_streams_tracked_resident(network net, int n, const int *stream_ids, const int *frame_w,
+                                                   const int *frame_h, float thresh, float nms, int use_mean,
+                                                   int max_det);
+void network_detect_batch_streams_tracked(network net, int n, const int *stream_ids,
+                                          const unsigned char *const *frames, const int *frame_w, const int *frame_h,
+                                          float thresh, float nms, int use_mean, y2_bbox *boxes, int *counts,
+                                          int max_det);
+int network_detect_wait_tracked(network net, y2_bbox *boxes, int *counts, int max_det);
 /* ---- batched, device-resident classification: letterbox, forward pass, WordTree products and top-k run on the
  * device and only `top` (index, probability) pairs per image come back, equal to what predict_classifier_image
  * computes on the host (classifier.c:676-730: letterbox_image, network_predict, hierarchy_predictions for a WordTree
@@ -517,7 +558,7 @@ int network_launch_count(network net);
 int network_profile_layers(network net, float *ms_per_layer, int n);
 /* 1 -> run layers eagerly instead of replaying the captured CUDA graph */
 void network_set_eager(network net, int eager);
-/* sizeof(layer|network|network_state|y2_detection|box|y2_class_hit) for what = 0..5: lets a binding that
+/* sizeof(layer|network|network_state|y2_detection|box|y2_class_hit|y2_bbox) for what = 0..6: lets a binding that
  * passes these structs by value check its mirror against the library it loaded. */
 size_t y2_abi_sizeof(int what);
 

@@ -319,6 +319,47 @@ int y2_stream_mean(const float *out, const float *ring, const y2_stream_src *tab
 /* ring[table[i].commit] = out[i] for every committing image; launch after y2_stream_mean of the same table. */
 int y2_stream_commit(const float *out, float *ring, const y2_stream_src *table, int n, int outputs, y2_stream_t s);
 
+/* ---- tracking of video streams (replaces, for many streams in one batch, the pixel conversion of
+ *      yolo_v2_class.cpp:228-236 and Detector::tracking, yolo_v2_class.cpp:251-304) ----------------------------------- */
+#ifndef Y2_BBOX_DEFINED
+#define Y2_BBOX_DEFINED
+typedef struct y2_bbox { /* bbox_t (yolo_v2_class.hpp:27-33): pixels, class, track id */
+    unsigned int x, y, w, h;
+    float prob;
+    unsigned int obj_id, track_id;
+} y2_bbox;
+#endif
+#define Y2_TRACK_MAX_STORY 32
+/* boxes per frame y2_stream_track holds in shared memory (32 bytes each, within the 227 KB of a block) */
+#define Y2_TRACK_MAX_TOTAL 7168
+/* One image of a tracked batch.  Stream s keeps a history ring of `story` frames (slot k holds up to `total` boxes and
+ * their count) and one next-id counter per class.  The host owns the ring position and fill; the device owns the
+ * boxes and the ids. */
+typedef struct y2_track_img {
+    int image;   /* row of the batch's detection lists */
+    int stream;
+    int w, h;    /* frame size in pixels, the boxes are scaled to it */
+    int head;    /* history slot this frame is pushed to; the newest earlier frame is in slot head-1 (mod story) */
+    int len;     /* frames in the history before this one, 0 .. story */
+    int restart; /* 1: the stream's ids restart at 1 before this frame (open, reset) */
+} y2_track_img;
+/* For a list of n images (image i from stream stream_ids[i], frame_w[i] x frame_h[i] pixels): the distinct streams in
+ * order of first appearance, each with its images in list order (records recs[offsets[k] .. offsets[k+1]) for stream k,
+ * offsets[n_streams] = n).  head, len and restart ([max_streams]; 0, 0, 1 for a stream that starts over) are read and
+ * advanced.  Returns n_streams; Y2_EINVAL (nothing changed) for an id outside 0..max_streams-1, a frame size of 0 or
+ * less or a story outside 1..Y2_TRACK_MAX_STORY.  Host only. */
+int y2_track_plan(int n, const int *stream_ids, const int *frame_w, const int *frame_h, int max_streams, int story,
+                  int *head, int *len, int *restart, y2_track_img *recs, int *offsets);
+/* Detector::tracking(to_bbox(detections), story) for every image of the plan, one block per stream walking its images
+ * in order.  det [images][det_stride] / count [images]: the detection lists (count <= min(total, det_stride));
+ * hist [max_streams][story][total], hist_count [max_streams][story], next_id [max_streams][classes] (every
+ * obj_id < classes): the device state, read and advanced; out [images][out_stride] receives the first out_stride
+ * tracked boxes of each image (tracking itself sees all count[image]).  1 <= total <= Y2_TRACK_MAX_TOTAL. */
+struct y2_det; /* below, with the final pick */
+int y2_stream_track(const struct y2_det *det, int det_stride, const int *count, const y2_track_img *recs,
+                    const int *offsets, int n_streams, int total, int classes, int story, y2_bbox *hist, int *hist_count,
+                    unsigned int *next_id, y2_bbox *out, int out_stride, y2_stream_t s);
+
 /* ---- do_nms_sort (replaces box.c:249-277) ------------------------------------------- */
 /* boxes [B][total][4], probs [B][total][classes] updated in place. */
 int y2_nms_sort(const float *boxes, float *probs, int batch, int total, int classes,

@@ -72,6 +72,28 @@ def stream_plan(stream_ids, max_streams: int, frame_index, frames_seen):
     return list(plan)[:n], list(fi), list(seen)
 
 
+class TrackImg(C.Structure):
+    """Mirror of `y2_track_img`: one image of a tracked batch and its stream's history position before it."""
+    _fields_ = [("image", C.c_int), ("stream", C.c_int), ("w", C.c_int), ("h", C.c_int), ("head", C.c_int),
+                ("len", C.c_int), ("restart", C.c_int)]
+
+
+def track_plan(stream_ids, sizes, max_streams: int, story: int, head, length, restart):
+    """y2_track_plan for one list of stream ids with frame sizes [(w, h), ...]: (records, offsets, advanced head,
+    advanced len, advanced restart).  The counter lists are not modified; a bad argument raises Y2Error."""
+    lib = load()
+    n = len(stream_ids)
+    ids = (C.c_int * max(n, 1))(*stream_ids)
+    fw = (C.c_int * max(n, 1))(*[s[0] for s in sizes])
+    fh = (C.c_int * max(n, 1))(*[s[1] for s in sizes])
+    hd, ln, rs = ((C.c_int * max_streams)(*v) for v in (head, length, restart))
+    recs = (TrackImg * max(n, 1))()
+    offsets = (C.c_int * (n + 1))()
+    k = lib.y2_track_plan(n, ids, fw, fh, max_streams, story, hd, ln, rs, recs, offsets)
+    check(0 if k >= 1 else k, "y2_track_plan")
+    return list(recs)[:n], list(offsets)[:k + 1], list(hd), list(ln), list(rs)
+
+
 def lib_path() -> Path:
     return _build.LIB
 
@@ -146,6 +168,9 @@ def _declare(lib: C.CDLL) -> None:
         "y2_stream_plan": (i, [i, C.POINTER(i), i, C.POINTER(i), C.POINTER(i), C.POINTER(StreamSrc)]),
         "y2_stream_mean": (i, [vp, vp, vp, i, i, vp, vp]),
         "y2_stream_commit": (i, [vp, vp, vp, i, i, vp]),
+        "y2_track_plan": (i, [i, C.POINTER(i), C.POINTER(i), C.POINTER(i), i, i, C.POINTER(i), C.POINTER(i),
+                              C.POINTER(i), C.POINTER(TrackImg), C.POINTER(i)]),
+        "y2_stream_track": (i, [vp, i, vp, vp, vp, i, i, i, i, vp, vp, vp, vp, i, vp]),
         "y2_unpack_to_nchw_f32": (i, [vp, vp, i, i, i, i, i, vp]),
         "y2_flat_to_nchw_f32": (i, [vp, vp, i, i, i, i, vp]),
         "y2_nchw_to_flat_f32": (i, [vp, vp, i, i, i, vp]),

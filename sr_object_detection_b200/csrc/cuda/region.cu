@@ -877,6 +877,114 @@ __global__ void __launch_bounds__(STREAM_THREADS) stream_commit_kernel(const flo
     }
 }
 
+// tracking of video streams ----------------------------------------------------------
+// yolo_v2_class.cpp:228-236 (to_bbox) and 251-304 (Detector::tracking) for the images of each stream in order.  One
+// block per stream.  The current frame's boxes live in shared memory next to best[]; every old box of the history
+// (newest frame first, boxes in list order) is one block-wide step, because a match halves the matched box's extent
+// and so moves the centre that later old boxes see.  Thread t alone reads and writes the current boxes m = t (mod
+// TRACK_THREADS), so a step needs one barrier: the reduction of the match and of id_taken, after which the owner of
+// the match applies it.  The match goes through one of three shared slots in turn, so that the slot a step reduces
+// into was reset by thread 0 behind an earlier barrier while no thread could still read it.
+constexpr int TRACK_THREADS = 128;
+
+// float / double -> unsigned as x86-64 compilers convert (through a 64-bit integer): what the host Detector computes
+__device__ __forceinline__ unsigned int track_u32(double v) { return (unsigned int)(long long)v; }
+
+__device__ __forceinline__ y2_bbox track_to_bbox(const y2_det &d, int img_w, int img_h)
+{
+    const double cx = __dmul_rn(__dsub_rn((double)d.x, __ddiv_rn((double)d.w, 2.)), (double)img_w);
+    const double cy = __dmul_rn(__dsub_rn((double)d.y, __ddiv_rn((double)d.h, 2.)), (double)img_h);
+    y2_bbox b;
+    b.x = track_u32(0. < cx ? cx : 0.); // std::max((double)0, v)
+    b.y = track_u32(0. < cy ? cy : 0.);
+    b.w = track_u32((double)__fmul_rn(d.w, (float)img_w));
+    b.h = track_u32((double)__fmul_rn(d.h, (float)img_h));
+    b.prob = d.prob;
+    b.obj_id = (unsigned int)d.obj_id;
+    b.track_id = 0;
+    return b;
+}
+
+__global__ void __launch_bounds__(TRACK_THREADS) stream_track_kernel(const y2_det *__restrict__ det, int det_stride,
+                                                                     const int *__restrict__ count,
+                                                                     const y2_track_img *__restrict__ recs,
+                                                                     const int *__restrict__ offsets, int total,
+                                                                     int classes, int story, y2_bbox *hist,
+                                                                     int *hist_count, unsigned int *next_id,
+                                                                     y2_bbox *__restrict__ out, int out_stride)
+{
+    extern __shared__ __align__(16) unsigned char track_smem[];
+    y2_bbox *cur = (y2_bbox *)track_smem;
+    unsigned int *best = (unsigned int *)(cur + total);
+    __shared__ int s_match[3];
+    const int tid = threadIdx.x;
+    const int first = offsets[blockIdx.x], last = offsets[blockIdx.x + 1];
+    const int s = recs[first].stream;
+    unsigned int *ids = next_id + (size_t)s * classes;
+    if (tid < 3) s_match[tid] = -1;
+    int q = 0; // block-wide steps so far
+    for (int r = first; r < last; ++r) {
+        const y2_track_img rec = recs[r];
+        if (rec.restart)
+            for (int c = tid; c < classes; c += TRACK_THREADS) ids[c] = 1u;
+        const int n = min(max(count[rec.image], 0), min(total, det_stride));
+        const y2_det *d = det + (size_t)rec.image * det_stride;
+        for (int m = tid; m < n; m += TRACK_THREADS) {
+            cur[m] = track_to_bbox(d[m], rec.w, rec.h);
+            best[m] = 0xffffffffu;
+        }
+        __syncthreads();
+        for (int k = 1; k <= rec.len; ++k) {
+            const int slot = (rec.head - k + story) % story;
+            const y2_bbox *frame = hist + ((size_t)s * story + slot) * total;
+            const int on = hist_count[s * story + slot];
+            y2_bbox next = frame[0]; // the next step's old box, loaded a step ahead (unused when the frame is empty)
+            for (int j = 0; j < on; ++j, ++q) {
+                const y2_bbox old = next;
+                if (j + 1 < on) next = frame[j + 1];
+                const float ox = (float)(old.x + old.w / 2), oy = (float)(old.y + old.h / 2);
+                int match = -1;
+                int taken = 0;
+                for (int m = tid; m < n; m += TRACK_THREADS) {
+                    const y2_bbox k = cur[m];
+                    if (k.obj_id != old.obj_id) continue;
+                    taken |= k.track_id == old.track_id;
+                    const float dx = __fsub_rn(ox, (float)(k.x + k.w / 2));
+                    const float dy = __fsub_rn(oy, (float)(k.y + k.h / 2));
+                    const unsigned int dist = track_u32((double)__fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy))));
+                    if (dist < 100 && (k.track_id == 0 || best[m] > dist)) {
+                        best[m] = dist;
+                        match = m; // the last m that qualifies wins, not the nearest
+                    }
+                }
+                match = __reduce_max_sync(0xffffffffu, match);
+                if ((tid & 31) == 0 && match >= 0) atomicMax(&s_match[q % 3], match);
+                taken = __syncthreads_or(taken);
+                const int m = s_match[q % 3];
+                if (tid == 0) s_match[(q + 2) % 3] = -1; // read by every thread before this step's barrier
+                if (m >= 0 && !taken && m % TRACK_THREADS == tid) {
+                    cur[m].track_id = old.track_id;
+                    cur[m].w = (cur[m].w + old.w) / 2;
+                    cur[m].h = (cur[m].h + old.h) / 2;
+                }
+            }
+        }
+        __syncthreads();
+        if (tid == 0)
+            for (int m = 0; m < n; ++m)
+                if (cur[m].track_id == 0) cur[m].track_id = ids[cur[m].obj_id]++;
+        __syncthreads();
+        y2_bbox *push = hist + ((size_t)s * story + rec.head) * total;
+        y2_bbox *dst = out + (size_t)rec.image * out_stride;
+        for (int m = tid; m < n; m += TRACK_THREADS) {
+            push[m] = cur[m];
+            if (m < out_stride) dst[m] = cur[m];
+        }
+        if (tid == 0) hist_count[s * story + rec.head] = n;
+        __syncthreads();
+    }
+}
+
 // classifier tail ------------------------------------------------------------------
 // avgpool_layer.c:40-55: sequential float sum over h*w, then / (h*w).  One thread per
 // (b, c) keeps the reference's summation order; reads are coalesced along c.
@@ -1324,6 +1432,60 @@ extern "C" int y2_stream_plan(int n, const int *stream_ids, int max_streams, int
         if (frames_seen[s] < 3) frames_seen[s]++;
     }
     free(slot);
+    return Y2_OK;
+}
+
+extern "C" int y2_track_plan(int n, const int *stream_ids, const int *frame_w, const int *frame_h, int max_streams,
+                             int story, int *head, int *len, int *restart, y2_track_img *recs, int *offsets)
+{
+    if (n < 1 || !stream_ids || !frame_w || !frame_h || max_streams < 1 || story < 1 || story > Y2_TRACK_MAX_STORY ||
+        !head || !len || !restart || !recs || !offsets)
+        return Y2_EINVAL;
+    for (int i = 0; i < n; ++i)
+        if (stream_ids[i] < 0 || stream_ids[i] >= max_streams || frame_w[i] <= 0 || frame_h[i] <= 0) return Y2_EINVAL;
+    int n_streams = 0, k = 0;
+    for (int i = 0; i < n; ++i) {
+        const int s = stream_ids[i];
+        bool seen = false;
+        for (int q = 0; q < i && !seen; ++q) seen = stream_ids[q] == s;
+        if (seen) continue;
+        offsets[n_streams++] = k;
+        for (int j = i; j < n; ++j) {
+            if (stream_ids[j] != s) continue;
+            recs[k++] = y2_track_img{j, s, frame_w[j], frame_h[j], head[s], len[s], restart[s]};
+            restart[s] = 0;
+            head[s] = (head[s] + 1) % story;
+            if (len[s] < story) len[s]++;
+        }
+    }
+    offsets[n_streams] = n;
+    return n_streams;
+}
+
+extern "C" int y2_stream_track(const y2_det *det, int det_stride, const int *count, const y2_track_img *recs,
+                               const int *offsets, int n_streams, int total, int classes, int story, y2_bbox *hist,
+                               int *hist_count, unsigned int *next_id, y2_bbox *out, int out_stride, y2_stream_t s)
+{
+    if (!det || !count || !recs || !offsets || !hist || !hist_count || !next_id || !out || n_streams < 1 || total < 1 ||
+        total > Y2_TRACK_MAX_TOTAL || det_stride < 1 || out_stride < 1 || classes < 1 || story < 1 ||
+        story > Y2_TRACK_MAX_STORY) {
+        set_error("y2_stream_track: invalid arguments (n_streams=%d total=%d det_stride=%d out_stride=%d classes=%d "
+                  "story=%d)", n_streams, total, det_stride, out_stride, classes, story);
+        return Y2_EINVAL;
+    }
+    const size_t smem = (size_t)total * (sizeof(y2_bbox) + sizeof(unsigned int));
+    static bool attr_done[64] = {};
+    int dev = 0;
+    Y2_CUDA_CHECK(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64 || !attr_done[dev]) { /* once per device, for the largest list the ABI takes */
+        Y2_CUDA_CHECK(cudaFuncSetAttribute(stream_track_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)((size_t)Y2_TRACK_MAX_TOTAL * (sizeof(y2_bbox) + sizeof(unsigned int)))));
+        if (dev >= 0 && dev < 64) attr_done[dev] = true;
+    }
+    stream_track_kernel<<<n_streams, TRACK_THREADS, smem, to_stream(s)>>>(det, det_stride, count, recs, offsets, total,
+                                                                         classes, story, hist, hist_count, next_id,
+                                                                         out, out_stride);
+    Y2_LAUNCH_CHECK();
     return Y2_OK;
 }
 

@@ -210,7 +210,7 @@ void network_detect_device(network net, float thresh, float nms, y2_detection *d
     y2_results *res = &rt->res;
     y2_results_reserve_dets(rt, res, B, max_det);
     detect_tail(rt, l, net.layers[net.n - 2].b200, (float *)((y2_layer_rt *)l->b200)->out, B, thresh, nms, res);
-    y2_results_to_host(res, B, 0, rt->stream);
+    y2_results_to_host(res, Y2_PIPE_DETECT, B, 0, rt->stream);
     Y2_CHECK(y2_stream_sync(rt->stream));
     y2_results_copy_dets(res, B, dets, counts, max_det);
 }
@@ -233,14 +233,17 @@ static layer *streams_region(network net)
     return l;
 }
 
-/* the stream ids of a streams batch, one per image */
+/* the stream ids of a streams batch, one per image; a tracked batch also has the frame sizes in pixels */
 typedef struct {
     int n;
     const int *ids;
+    int tracked;
+    int use_mean;     /* decoded on the 3-frame means (always, untracked) */
+    const int *w, *h; /* tracked */
 } stream_list;
 
 /* the refusals of every streams submission, after the pipeline's and the frame list's, before anything is staged */
-static void check_streams(network net, int n, const int *stream_ids)
+static void check_streams(network net, const stream_list *sl)
 {
     y2_net_rt *rt = y2_rt(net);
     const layer *l = streams_region(net);
@@ -249,17 +252,39 @@ static void check_streams(network net, int n, const int *stream_ids)
     if (l->outputs != st->outputs)
         error("network streams: the region output size differs from the one the streams were opened with (after "
               "resize_network, open them again)");
-    if (n < 1 || n > net.batch) error("network streams: the list must hold 1 .. batch images");
-    if (!stream_ids) error("network streams: NULL stream id array");
-    for (int i = 0; i < n; ++i)
-        if (stream_ids[i] < 0 || stream_ids[i] >= st->max_streams)
+    if (sl->n < 1 || sl->n > net.batch) error("network streams: the list must hold 1 .. batch images");
+    if (!sl->ids) error("network streams: NULL stream id array");
+    for (int i = 0; i < sl->n; ++i)
+        if (sl->ids[i] < 0 || sl->ids[i] >= st->max_streams)
             error("network streams: a stream id outside 0 .. max_streams-1");
+    if (!sl->tracked) return;
+    if (!st->story) error("network streams tracked: tracking not enabled, call network_streams_track");
+    if (sl->use_mean != 0 && sl->use_mean != 1) error("network streams tracked: use_mean must be 0 or 1");
+    if (!sl->w || !sl->h) error("network streams tracked: NULL frame width or height array");
+    for (int i = 0; i < sl->n; ++i)
+        if (sl->w[i] <= 0 || sl->h[i] <= 0) error("network streams tracked: a frame size of 0 or less");
+}
+
+static void track_free(y2_streams *st)
+{
+    y2_free(st->hist_dev);
+    y2_free(st->hist_cnt_dev);
+    y2_free(st->next_id_dev);
+    free(st->track_head);
+    free(st->track_len);
+    free(st->track_restart);
+    st->hist_dev = NULL;
+    st->hist_cnt_dev = NULL;
+    st->next_id_dev = NULL;
+    st->track_head = st->track_len = st->track_restart = NULL;
+    st->story = 0;
 }
 
 void y2_streams_free(y2_net_rt *rt)
 {
     y2_streams *st = rt->streams;
     if (!st) return;
+    track_free(st);
     y2_free(st->ring_dev);
     y2_free(st->mean_dev);
     for (int s = 0; s < 2; ++s) {
@@ -303,13 +328,55 @@ void network_stream_reset(network net, int stream)
     /* host only: batches already submitted keep the table they were given */
     st->frame_index[stream] = 0;
     st->frames_seen[stream] = 0;
+    if (st->story) { /* an empty history; the stream's next tracked image restarts its ids on the device */
+        st->track_head[stream] = 0;
+        st->track_len[stream] = 0;
+        st->track_restart[stream] = 1;
+    }
 }
 
-/* A streams batch into slot s: its ring plan in the slot's table, copied on the copy stream (ahead of the slot's
- * input copies, so the slot's ev_h2d covers it) */
-static void streams_stage(y2_net_rt *rt, int s, int n, const int *stream_ids, int batch)
+void network_streams_track(network net, int frames_story)
+{
+    y2_net_rt *rt = y2_rt(net);
+    if (!rt) error("network_streams_track: network has no device plan");
+    y2_streams *st = rt->streams;
+    if (!st) error("network_streams_track: streams not opened, call network_streams_open");
+    if (frames_story < 1 || frames_story > Y2_TRACK_MAX_STORY)
+        error("network_streams_track: frames_story must be in 1 .. Y2_TRACK_MAX_STORY");
+    const layer *l = streams_region(net);
+    if (l->w * l->h * l->n > Y2_TRACK_MAX_TOTAL)
+        error("network_streams_track: more region boxes per image than Y2_TRACK_MAX_TOTAL (the tracking kernel holds a "
+              "frame's boxes in shared memory)");
+    Y2_CHECK(y2_set_device(rt->device));
+    Y2_CHECK(y2_stream_sync(rt->stream)); /* batches in flight read and write the old history */
+    track_free(st);
+    const int S = st->max_streams, total = l->w * l->h * l->n;
+    st->track_head = (int *)calloc((size_t)S, sizeof(int));
+    st->track_len = (int *)calloc((size_t)S, sizeof(int));
+    st->track_restart = (int *)malloc((size_t)S * sizeof(int));
+    if (!st->track_head || !st->track_len || !st->track_restart) error("network_streams_track: out of host memory");
+    for (int s = 0; s < S; ++s) st->track_restart[s] = 1;
+    /* not cleared: a history slot is read only below its fill, ids only after the restart that sets them */
+    Y2_CHECK(y2_malloc((void **)&st->hist_dev, (size_t)S * frames_story * total * sizeof(y2_bbox)));
+    Y2_CHECK(y2_malloc((void **)&st->hist_cnt_dev, (size_t)S * frames_story * sizeof(int)));
+    Y2_CHECK(y2_malloc((void **)&st->next_id_dev, (size_t)S * l->classes * sizeof(unsigned int)));
+    st->story = frames_story;
+    st->total = total;
+    st->classes = l->classes;
+}
+
+/* where the parts of a slot's stream table sit for a batch of n images */
+static size_t track_recs_at(int n) { return (size_t)n * sizeof(y2_stream_src); }
+static size_t track_offsets_at(int n) { return track_recs_at(n) + (size_t)n * sizeof(y2_track_img); }
+static size_t table_bytes(int n) { return track_offsets_at(n) + (size_t)(n + 1) * sizeof(int); }
+
+/* A streams batch into slot s: its ring plan (decoded on the means) and its tracking plan (tracked) in the slot's
+ * table, copied in one piece on the copy stream (ahead of the slot's input copies, so the slot's ev_h2d covers it).
+ * Returns the number of distinct streams of a tracked batch. */
+static int streams_stage(y2_net_rt *rt, int s, const stream_list *sl, int batch)
 {
     y2_streams *st = rt->streams;
+    const int n = sl->n;
     const int cap_b = batch > rt->cap_batch ? batch : rt->cap_batch;
     if (st->mean_cap < batch) {
         Y2_CHECK(y2_stream_sync(rt->stream)); /* the other slot's decode may still read the means */
@@ -320,20 +387,32 @@ static void streams_stage(y2_net_rt *rt, int s, int n, const int *stream_ids, in
     if (st->table_cap[s] < batch) {
         y2_free(st->table_dev[s]);
         y2_host_free(st->table_pinned[s]);
-        Y2_CHECK(y2_malloc((void **)&st->table_dev[s], (size_t)cap_b * sizeof(y2_stream_src)));
-        Y2_CHECK(y2_host_alloc((void **)&st->table_pinned[s], (size_t)cap_b * sizeof(y2_stream_src)));
+        Y2_CHECK(y2_malloc((void **)&st->table_dev[s], table_bytes(cap_b)));
+        Y2_CHECK(y2_host_alloc((void **)&st->table_pinned[s], table_bytes(cap_b)));
         st->table_cap[s] = cap_b;
     }
-    Y2_CHECK(y2_stream_plan(n, stream_ids, st->max_streams, st->frame_index, st->frames_seen, st->table_pinned[s]));
-    Y2_CHECK(y2_memcpy_h2d(st->table_dev[s], st->table_pinned[s], (size_t)n * sizeof(y2_stream_src), rt->copy_stream));
+    unsigned char *tab = st->table_pinned[s];
+    if (sl->use_mean)
+        Y2_CHECK(y2_stream_plan(n, sl->ids, st->max_streams, st->frame_index, st->frames_seen, (y2_stream_src *)tab));
+    int n_streams = 0;
+    if (sl->tracked) {
+        n_streams = y2_track_plan(n, sl->ids, sl->w, sl->h, st->max_streams, st->story, st->track_head, st->track_len,
+                                  st->track_restart, (y2_track_img *)(tab + track_recs_at(n)),
+                                  (int *)(tab + track_offsets_at(n)));
+        Y2_CHECK(n_streams < 1 ? Y2_EINVAL : Y2_OK);
+    }
+    const size_t from = sl->use_mean ? 0 : track_recs_at(n), to = sl->tracked ? table_bytes(n) : track_recs_at(n);
+    Y2_CHECK(y2_memcpy_h2d(st->table_dev[s] + from, tab + from, to - from, rt->copy_stream));
+    return n_streams;
 }
 
-/* A detection batch into the pipeline.  With streams it is a streams batch: decoded on the 3-frame means, streams->n
- * images come back; otherwise (NULL) the tail runs on the region output of all B images and in.n come back. */
+/* A detection batch into the pipeline.  With streams it is a streams batch: decoded on the 3-frame means (or, tracked
+ * without use_mean, on the region output), streams->n images come back, tracked as pixel boxes with track ids;
+ * otherwise (NULL) the tail runs on the region output of all B images and in.n come back. */
 static int detect_submit(network net, y2_input in, const stream_list *streams, float thresh, float nms, int max_det)
 {
     const int s = y2_pipe_claim(net, &in);
-    if (streams) check_streams(net, streams->n, streams->ids);
+    if (streams) check_streams(net, streams);
     y2_net_rt *rt = y2_rt(net);
     struct y2_pipe_slot *ps = &rt->pipe[s];
     layer *l = region_of(net);
@@ -341,8 +420,15 @@ static int detect_submit(network net, y2_input in, const stream_list *streams, f
     void *head_rt = net.layers[net.n - 2].b200;
     const int B = net.batch;
     const int n = streams ? streams->n : in.n;
-    y2_results_reserve_dets(rt, &ps->res, B, max_det);
-    if (streams) streams_stage(rt, s, n, streams->ids, B);
+    const int tracked = streams && streams->tracked;
+    const int total = l->w * l->h * l->n;
+    /* tracking sees every detection of a frame: the lists hold all `total` boxes, max_det cuts only the copy out */
+    y2_results_reserve_dets(rt, &ps->res, B, tracked ? total : max_det);
+    if (tracked) {
+        y2_results_reserve_boxes(rt, &ps->res, B, total);
+        ps->res.box_stride = max_det < total ? max_det : total; /* rows of the copy back */
+    }
+    const int n_streams = streams ? streams_stage(rt, s, streams, B) : 0;
     y2_pipe_submit_input(net, s, &in, 0);
     if (streams) {
         y2_streams *st = rt->streams;
@@ -350,14 +436,23 @@ static int detect_submit(network net, y2_input in, const stream_list *streams, f
             Y2_CHECK(y2_event_record(ps->ev_h2d, rt->copy_stream));
             Y2_CHECK(y2_stream_wait_event(rt->stream, ps->ev_h2d));
         }
-        Y2_CHECK(y2_stream_mean((const float *)r->out, st->ring_dev, st->table_dev[s], n, st->outputs, st->mean_dev,
-                                rt->stream));
-        Y2_CHECK(y2_stream_commit((const float *)r->out, st->ring_dev, st->table_dev[s], n, st->outputs, rt->stream));
-        detect_tail(rt, l, head_rt, st->mean_dev, n, thresh, nms, &ps->res);
+        const y2_stream_src *ring_plan = (const y2_stream_src *)st->table_dev[s];
+        if (streams->use_mean) {
+            Y2_CHECK(y2_stream_mean((const float *)r->out, st->ring_dev, ring_plan, n, st->outputs, st->mean_dev,
+                                    rt->stream));
+            Y2_CHECK(y2_stream_commit((const float *)r->out, st->ring_dev, ring_plan, n, st->outputs, rt->stream));
+        }
+        detect_tail(rt, l, head_rt, streams->use_mean ? st->mean_dev : (float *)r->out, n, thresh, nms, &ps->res);
+        if (tracked)
+            Y2_CHECK(y2_stream_track((const y2_det *)ps->res.det_dev, ps->res.det_cap, ps->res.cnt_dev,
+                                     (const y2_track_img *)(st->table_dev[s] + track_recs_at(n)),
+                                     (const int *)(st->table_dev[s] + track_offsets_at(n)), n_streams, total,
+                                     st->classes, st->story, st->hist_dev, st->hist_cnt_dev, st->next_id_dev,
+                                     ps->res.box_dev, ps->res.box_stride, rt->stream));
     } else {
         detect_tail(rt, l, head_rt, (float *)r->out, B, thresh, nms, &ps->res);
     }
-    y2_pipe_queue(rt, s, Y2_PIPE_DETECT, n, 0);
+    y2_pipe_queue(rt, s, tracked ? Y2_PIPE_TRACK : Y2_PIPE_DETECT, n, 0);
     return s;
 }
 
@@ -369,14 +464,24 @@ int network_detect_wait(network net, y2_detection *dets, int *counts, int max_de
     return s;
 }
 
-/* the detection *_batch_* entries: one submission and its wait, refused while batches of the pipeline are in flight */
+int network_detect_wait_tracked(network net, y2_bbox *boxes, int *counts, int max_det)
+{
+    const int s = y2_pipe_retire(net, Y2_PIPE_TRACK, 0);
+    const struct y2_pipe_slot *ps = &y2_rt(net)->pipe[s];
+    y2_results_copy_boxes(&ps->res, ps->n_images, boxes, counts, max_det);
+    return s;
+}
+
+/* the detection *_batch_* entries: one submission and its wait, refused while batches of the pipeline are in flight.
+ * A tracked batch hands out boxes, every other one dets. */
 static void detect_batch(network net, const char *in_flight, y2_input in, const stream_list *streams, float thresh,
-                         float nms, y2_detection *dets, int *counts, int max_det)
+                         float nms, y2_detection *dets, y2_bbox *boxes, int *counts, int max_det)
 {
     y2_net_rt *rt = y2_rt(net);
     if (rt && rt->pipe_inflight) error(in_flight);
     detect_submit(net, in, streams, thresh, nms, max_det);
-    network_detect_wait(net, dets, counts, max_det);
+    if (streams && streams->tracked) network_detect_wait_tracked(net, boxes, counts, max_det);
+    else network_detect_wait(net, dets, counts, max_det);
 }
 
 int network_detect_submit(network net, const float *input, float thresh, float nms, int max_det)
@@ -393,7 +498,7 @@ void network_detect_batch_u8(network net, const unsigned char *input_hwc, float 
                              int *counts, int max_det)
 {
     detect_batch(net, "network_detect_batch_u8: batches of the submit/wait pipeline are in flight",
-                 (y2_input){.kind = Y2_IN_U8, .data = input_hwc}, NULL, thresh, nms, dets, counts, max_det);
+                 (y2_input){.kind = Y2_IN_U8, .data = input_hwc}, NULL, thresh, nms, dets, NULL, counts, max_det);
 }
 
 /* The batch is already in the slot's device input (network_pipeline_input_device(net, slot), e.g. written by another
@@ -419,7 +524,7 @@ void network_detect_batch_frames(network net, const unsigned char *frames_hwc, i
 {
     const y2_input in = {.kind = Y2_IN_FRAMES, .data = frames_hwc, .fw = frame_w, .fh = frame_h};
     detect_batch(net, "network_detect_batch_frames: batches of the submit/wait pipeline are in flight", in, NULL,
-                 thresh, nms, dets, counts, max_det);
+                 thresh, nms, dets, NULL, counts, max_det);
 }
 
 int network_detect_submit_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
@@ -435,20 +540,20 @@ void network_detect_batch_frame_list(network net, int n, const unsigned char *co
 {
     const y2_input in = {.kind = Y2_IN_FRAME_LIST, .list = {n, frames, frame_w, frame_h}};
     detect_batch(net, "network_detect_batch_frame_list: batches of the submit/wait pipeline are in flight", in,
-                 NULL, thresh, nms, dets, counts, max_det);
+                 NULL, thresh, nms, dets, NULL, counts, max_det);
 }
 
 int network_detect_submit_streams(network net, int n, const int *stream_ids, const unsigned char *const *frames,
                                   const int *frame_w, const int *frame_h, float thresh, float nms, int max_det)
 {
     const y2_input in = {.kind = Y2_IN_FRAME_LIST, .list = {n, frames, frame_w, frame_h}};
-    return detect_submit(net, in, &(stream_list){n, stream_ids}, thresh, nms, max_det);
+    return detect_submit(net, in, &(stream_list){n, stream_ids, 0, 1}, thresh, nms, max_det);
 }
 
 int network_detect_submit_streams_resident(network net, int n, const int *stream_ids, float thresh, float nms,
                                            int max_det)
 {
-    return detect_submit(net, (y2_input){.kind = Y2_IN_RESIDENT}, &(stream_list){n, stream_ids}, thresh, nms,
+    return detect_submit(net, (y2_input){.kind = Y2_IN_RESIDENT}, &(stream_list){n, stream_ids, 0, 1}, thresh, nms,
                          max_det);
 }
 
@@ -458,7 +563,34 @@ void network_detect_batch_streams(network net, int n, const int *stream_ids, con
 {
     const y2_input in = {.kind = Y2_IN_FRAME_LIST, .list = {n, frames, frame_w, frame_h}};
     detect_batch(net, "network_detect_batch_streams: batches of the submit/wait pipeline are in flight", in,
-                 &(stream_list){n, stream_ids}, thresh, nms, dets, counts, max_det);
+                 &(stream_list){n, stream_ids, 0, 1}, thresh, nms, dets, NULL, counts, max_det);
+}
+
+int network_detect_submit_streams_tracked(network net, int n, const int *stream_ids, const unsigned char *const *frames,
+                                          const int *frame_w, const int *frame_h, float thresh, float nms,
+                                          int use_mean, int max_det)
+{
+    const y2_input in = {.kind = Y2_IN_FRAME_LIST, .list = {n, frames, frame_w, frame_h}};
+    return detect_submit(net, in, &(stream_list){n, stream_ids, 1, use_mean, frame_w, frame_h}, thresh, nms, max_det);
+}
+
+int network_detect_submit_streams_tracked_resident(network net, int n, const int *stream_ids, const int *frame_w,
+                                                   const int *frame_h, float thresh, float nms, int use_mean,
+                                                   int max_det)
+{
+    return detect_submit(net, (y2_input){.kind = Y2_IN_RESIDENT},
+                         &(stream_list){n, stream_ids, 1, use_mean, frame_w, frame_h}, thresh, nms, max_det);
+}
+
+void network_detect_batch_streams_tracked(network net, int n, const int *stream_ids,
+                                          const unsigned char *const *frames, const int *frame_w, const int *frame_h,
+                                          float thresh, float nms, int use_mean, y2_bbox *boxes, int *counts,
+                                          int max_det)
+{
+    const y2_input in = {.kind = Y2_IN_FRAME_LIST, .list = {n, frames, frame_w, frame_h}};
+    detect_batch(net, "network_detect_batch_streams_tracked: batches of the submit/wait pipeline are in flight", in,
+                 &(stream_list){n, stream_ids, 1, use_mean, frame_w, frame_h}, thresh, nms, NULL, boxes, counts,
+                 max_det);
 }
 
 /* ---- batched, device-resident classification (extension) --------------------------------------- */
@@ -498,7 +630,7 @@ void network_classify_device(network net, int top, y2_class_hit *hits)
     Y2_CHECK(y2_set_device(rt->device));
     y2_results_reserve_hits(rt, &rt->res, top);
     classify_tail(rt, net, l, top, rt->res.hits_dev);
-    y2_results_to_host(&rt->res, net.batch, top, rt->stream);
+    y2_results_to_host(&rt->res, Y2_PIPE_CLASSIFY, net.batch, top, rt->stream);
     Y2_CHECK(y2_stream_sync(rt->stream));
     memcpy(hits, rt->res.hits_pinned, (size_t)net.batch * top * sizeof(y2_class_hit));
 }

@@ -20,7 +20,7 @@ void y2_fatal(const char *where, int rc);
     } while (0)
 
 enum { Y2_KIND_BF16_PADDED = 0, Y2_KIND_F32_FLAT = 1, Y2_KIND_F32_VEC = 2, Y2_KIND_NONE = 3 };
-enum { Y2_PIPE_DETECT = 0, Y2_PIPE_CLASSIFY = 1 }; /* what a pipeline slot's batch computes */
+enum { Y2_PIPE_DETECT = 0, Y2_PIPE_CLASSIFY = 1, Y2_PIPE_TRACK = 2 }; /* what a pipeline slot's batch computes */
 
 /* per-layer device plan, owned by net.layers[i].b200 */
 typedef struct y2_layer_rt {
@@ -85,8 +85,17 @@ typedef struct y2_streams {
     int *frames_seen;      /* [max_streams] frames since open / reset, saturating at 3 */
     float *mean_dev;       /* [mean_cap][outputs] the means the decode reads */
     int mean_cap;
-    y2_stream_src *table_pinned[2], *table_dev[2]; /* per pipeline slot, table_cap[slot] records */
+    /* per pipeline slot, for table_cap[slot] images: the ring plan (y2_stream_src[n]), then the tracking plan
+     * (y2_track_img[n], int offsets[n + 1]); one host -> device copy a batch */
+    unsigned char *table_pinned[2], *table_dev[2];
     int table_cap[2];
+    /* tracking (network_streams_track), story 0 when off.  The device holds the boxes and ids, the host the ring
+     * position, fill and start-over flag of each stream (y2_track_plan). */
+    int story, total, classes;
+    y2_bbox *hist_dev;          /* [max_streams][story][total] */
+    int *hist_cnt_dev;          /* [max_streams][story] */
+    unsigned int *next_id_dev;  /* [max_streams][classes] */
+    int *track_head, *track_len, *track_restart; /* [max_streams] */
 } y2_streams;
 
 /* what a batch hands back, each a device buffer with a pinned mirror (y2_pipeline.c) */
@@ -96,6 +105,8 @@ typedef struct y2_results {
     int det_cap, det_images;
     y2_class_hit *hits_dev, *hits_pinned; /* [cap_batch][hits_cap] class hits */
     int hits_cap;
+    y2_bbox *box_dev, *box_pinned;        /* [box_images][box_cap] tracked boxes; a batch uses rows of box_stride */
+    int box_cap, box_images, box_stride;
 } y2_results;
 
 /* what a submission feeds the network; y2_pipe_claim completes it */
@@ -184,8 +195,10 @@ void y2_pipe_queue(y2_net_rt *rt, int s, int kind, int n_images, int top);
 int y2_pipe_retire(network net, int kind, int top);
 void y2_results_reserve_dets(y2_net_rt *rt, y2_results *res, int batch, int max_det);
 void y2_results_reserve_hits(y2_net_rt *rt, y2_results *res, int top);
-void y2_results_to_host(const y2_results *res, int n, int top, y2_stream_t stream);
+void y2_results_reserve_boxes(y2_net_rt *rt, y2_results *res, int batch, int total);
+void y2_results_to_host(const y2_results *res, int kind, int n, int top, y2_stream_t stream);
 void y2_results_copy_dets(const y2_results *res, int n, y2_detection *dets, int *counts, int max_det);
+void y2_results_copy_boxes(const y2_results *res, int n, y2_bbox *boxes, int *counts, int max_det);
 void y2_results_free(y2_results *res);
 
 /* y2_detect.c */

@@ -1535,6 +1535,7 @@ size_t y2_abi_sizeof(int what)
     case 3: return sizeof(y2_detection);
     case 4: return sizeof(box);
     case 5: return sizeof(y2_class_hit);
+    case 6: return sizeof(y2_bbox);
     default: return 0;
     }
 }

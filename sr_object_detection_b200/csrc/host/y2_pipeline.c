@@ -39,16 +39,32 @@ void y2_results_reserve_hits(y2_net_rt *rt, y2_results *res, int top)
     res->hits_cap = top;
 }
 
-/* queues the device -> host copies of n images' results on `stream`: top class hits each, or (top 0) the detection
- * counts and lists */
-void y2_results_to_host(const y2_results *res, int n, int top, y2_stream_t stream)
+/* grows the tracked boxes to `total` per image for at least `batch` (and cap_batch) images */
+void y2_results_reserve_boxes(y2_net_rt *rt, y2_results *res, int batch, int total)
 {
-    if (top) {
+    if (res->box_cap >= total && res->box_images >= batch) return;
+    y2_free(res->box_dev);
+    y2_host_free(res->box_pinned);
+    res->box_cap = total;
+    res->box_images = batch > rt->cap_batch ? batch : rt->cap_batch;
+    const size_t nb = (size_t)res->box_images * total;
+    Y2_CHECK(y2_malloc((void **)&res->box_dev, nb * sizeof(y2_bbox)));
+    Y2_CHECK(y2_host_alloc((void **)&res->box_pinned, nb * sizeof(y2_bbox)));
+}
+
+/* queues the device -> host copies of n images' results of a Y2_PIPE_* kind on `stream`: top class hits each, the
+ * detection counts and lists, or the counts and tracked boxes */
+void y2_results_to_host(const y2_results *res, int kind, int n, int top, y2_stream_t stream)
+{
+    if (kind == Y2_PIPE_CLASSIFY) {
         Y2_CHECK(y2_memcpy_d2h(res->hits_pinned, res->hits_dev, (size_t)n * top * sizeof(y2_class_hit), stream));
         return;
     }
     Y2_CHECK(y2_memcpy_d2h(res->cnt_pinned, res->cnt_dev, (size_t)n * sizeof(int), stream));
-    Y2_CHECK(y2_memcpy_d2h(res->det_pinned, res->det_dev, (size_t)n * res->det_cap * sizeof(y2_det), stream));
+    if (kind == Y2_PIPE_TRACK)
+        Y2_CHECK(y2_memcpy_d2h(res->box_pinned, res->box_dev, (size_t)n * res->box_stride * sizeof(y2_bbox), stream));
+    else
+        Y2_CHECK(y2_memcpy_d2h(res->det_pinned, res->det_dev, (size_t)n * res->det_cap * sizeof(y2_det), stream));
 }
 
 /* the first n images' detection lists out of the pinned mirror, each cut to max_det; counts keep the full number */
@@ -63,6 +79,18 @@ void y2_results_copy_dets(const y2_results *res, int n, y2_detection *dets, int 
     }
 }
 
+/* the same for the tracked boxes */
+void y2_results_copy_boxes(const y2_results *res, int n, y2_bbox *boxes, int *counts, int max_det)
+{
+    for (int b = 0; b < n; ++b) {
+        int c = res->cnt_pinned[b];
+        counts[b] = c;
+        if (c > max_det) c = max_det;
+        if (c > res->box_stride) c = res->box_stride;
+        memcpy(boxes + (size_t)b * max_det, res->box_pinned + (size_t)b * res->box_stride, (size_t)c * sizeof(y2_bbox));
+    }
+}
+
 void y2_results_free(y2_results *res)
 {
     y2_free(res->det_dev);
@@ -71,6 +99,8 @@ void y2_results_free(y2_results *res)
     y2_host_free(res->cnt_pinned);
     y2_free(res->hits_dev);
     y2_host_free(res->hits_pinned);
+    y2_free(res->box_dev);
+    y2_host_free(res->box_pinned);
 }
 
 /* ---- slot lifecycle ------------------------------------------------------------------------------ */
@@ -339,7 +369,7 @@ void y2_pipe_queue(y2_net_rt *rt, int s, int kind, int n_images, int top)
     struct y2_pipe_slot *ps = &rt->pipe[s];
     Y2_CHECK(y2_event_record(ps->ev_tail, rt->stream));
     Y2_CHECK(y2_stream_wait_event(rt->d2h_stream, ps->ev_tail));
-    y2_results_to_host(&ps->res, n_images, top, rt->d2h_stream);
+    y2_results_to_host(&ps->res, kind, n_images, top, rt->d2h_stream);
     Y2_CHECK(y2_event_record(ps->ev_done, rt->d2h_stream));
     ps->kind = kind;
     ps->n_images = n_images;
@@ -352,15 +382,23 @@ void y2_pipe_queue(y2_net_rt *rt, int s, int kind, int n_images, int top)
 int y2_pipe_retire(network net, int kind, int top)
 {
     static const char *const nothing[] = {"network_detect_wait: nothing in flight",
-                                          "network_classify_wait: nothing in flight"};
-    static const char *const other[] = {
-        "network_detect_wait: the oldest batch in flight is a classify batch, call network_classify_wait",
-        "network_classify_wait: the oldest batch in flight is a detection batch, call network_detect_wait"};
+                                          "network_classify_wait: nothing in flight",
+                                          "network_detect_wait_tracked: nothing in flight"};
+    /* [wait's kind][kind of the oldest batch] */
+    static const char *const other[3][3] = {
+        {NULL, "network_detect_wait: the oldest batch in flight is a classify batch, call network_classify_wait",
+         "network_detect_wait: the oldest batch in flight is a tracked batch, call network_detect_wait_tracked"},
+        {"network_classify_wait: the oldest batch in flight is a detection batch, call network_detect_wait", NULL,
+         "network_classify_wait: the oldest batch in flight is a tracked batch, call network_detect_wait_tracked"},
+        {"network_detect_wait_tracked: the oldest batch in flight is an untracked detection batch, call "
+         "network_detect_wait",
+         "network_detect_wait_tracked: the oldest batch in flight is a classify batch, call network_classify_wait",
+         NULL}};
     y2_net_rt *rt = y2_rt(net);
     if (!rt || !rt->pipe_ready || rt->pipe_inflight <= 0) error(nothing[kind]);
     const int s = rt->pipe_head;
     struct y2_pipe_slot *ps = &rt->pipe[s];
-    if (ps->kind != kind) error(other[kind]);
+    if (ps->kind != kind) error(other[kind][ps->kind]);
     if (top != ps->top) error("network_classify_wait: top differs from the one the batch was submitted with");
     Y2_CHECK(y2_event_sync(ps->ev_done));
     rt->pipe_head ^= 1;

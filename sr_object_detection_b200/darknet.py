@@ -102,6 +102,12 @@ class ClassHit(C.Structure):
     _fields_ = [("index", C.c_int), ("prob", C.c_float)]
 
 
+class BBox(C.Structure):
+    """Mirror of `y2_bbox` (bbox_t): a tracked box in frame pixels."""
+    _fields_ = [("x", C.c_uint), ("y", C.c_uint), ("w", C.c_uint), ("h", C.c_uint), ("prob", C.c_float),
+                ("obj_id", C.c_uint), ("track_id", C.c_uint)]
+
+
 class Image(C.Structure):
     _fields_ = [("h", C.c_int), ("w", C.c_int), ("c", C.c_int), ("data", _fp)]
 
@@ -173,6 +179,13 @@ def lib() -> C.CDLL:
         "network_detect_submit_streams_resident": (i, [Network, i, _ip, f, f, i]),
         "network_detect_batch_streams": (None, [Network, i, _ip, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f,
                                                 C.POINTER(Detection), _ip, i]),
+        "network_streams_track": (None, [Network, i]),
+        "network_detect_submit_streams_tracked": (i, [Network, i, _ip, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f, f,
+                                                       i, i]),
+        "network_detect_submit_streams_tracked_resident": (i, [Network, i, _ip, _ip, _ip, f, f, i, i]),
+        "network_detect_batch_streams_tracked": (None, [Network, i, _ip, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, f,
+                                                        f, i, C.POINTER(BBox), _ip, i]),
+        "network_detect_wait_tracked": (i, [Network, C.POINTER(BBox), _ip, i]),
         "network_classify_submit_frame_list": (i, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i]),
         "network_classify_batch_frame_list": (None, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i,
                                                      C.POINTER(ClassHit)]),
@@ -238,6 +251,7 @@ def lib() -> C.CDLL:
     assert l.y2_abi_sizeof(2) == C.sizeof(NetworkState)
     assert l.y2_abi_sizeof(3) == C.sizeof(Detection)
     assert l.y2_abi_sizeof(5) == C.sizeof(ClassHit)
+    assert l.y2_abi_sizeof(6) == C.sizeof(BBox)
     _declared = True
     return l
 
@@ -461,6 +475,52 @@ def network_detect_submit_streams_resident(net: Network, stream_ids, thresh: flo
     (network_pipeline_input_device)."""
     n = len(stream_ids)
     return lib().network_detect_submit_streams_resident(net, n, _stream_ids(stream_ids, n), thresh, nms, max_det)
+
+
+def network_streams_track(net: Network, frames_story: int = 6) -> None:
+    """Extension: turn tracking on for the opened streams (Detector::tracking's frames_story), every track over."""
+    lib().network_streams_track(net, frames_story)
+
+
+def network_detect_streams_tracked(net: Network, stream_ids, frames, thresh: float, nms: float, use_mean: bool = True,
+                                   max_det: int = 256):
+    """Extension: as network_detect_streams, then tracked per stream as Detector::detect(img, thresh, use_mean) and
+    Detector::tracking(boxes, frames_story) would.  Returns (per-image arrays with fields x, y, w, h (pixels), prob,
+    obj_id, track_id; full counts) for len(frames) images."""
+    n, ptrs, fw, fh = _frame_list_args(frames)
+    boxes = (BBox * (max(n, 1) * max_det))()
+    counts = (C.c_int * max(n, 1))()
+    lib().network_detect_batch_streams_tracked(net, n, _stream_ids(stream_ids, n), ptrs, fw, fh, thresh, nms,
+                                               int(use_mean), boxes, counts, max_det)
+    return _det_lists(boxes, counts, n, max_det)
+
+
+def network_detect_submit_streams_tracked(net: Network, stream_ids, frames, thresh: float, nms: float,
+                                          use_mean: bool = True, max_det: int = 256) -> int:
+    """Queue a tracked streams frame list; network_detect_wait_tracked(net, len(frames), ...) collects it."""
+    n, ptrs, fw, fh = _frame_list_args(frames)
+    return lib().network_detect_submit_streams_tracked(net, n, _stream_ids(stream_ids, n), ptrs, fw, fh, thresh, nms,
+                                                       int(use_mean), max_det)
+
+
+def network_detect_submit_streams_tracked_resident(net: Network, stream_ids, sizes, thresh: float, nms: float,
+                                                   use_mean: bool = True, max_det: int = 256) -> int:
+    """The same with the first len(stream_ids) images already in the slot's device input; sizes [(w, h), ...] are
+    the frame sizes in pixels the boxes are scaled to."""
+    n = len(stream_ids)
+    assert len(sizes) == n, (len(sizes), n)
+    fw = (C.c_int * max(n, 1))(*[int(s[0]) for s in sizes])
+    fh = (C.c_int * max(n, 1))(*[int(s[1]) for s in sizes])
+    return lib().network_detect_submit_streams_tracked_resident(net, n, _stream_ids(stream_ids, n), fw, fh, thresh,
+                                                                nms, int(use_mean), max_det)
+
+
+def network_detect_wait_tracked(net: Network, n: int, max_det: int = 256):
+    """network_detect_wait_tracked for the oldest batch in flight, a tracked batch of n images"""
+    boxes = (BBox * (net.batch * max_det))()
+    counts = (C.c_int * net.batch)()
+    lib().network_detect_wait_tracked(net, boxes, counts, max_det)
+    return _det_lists(boxes, counts, n, max_det)
 
 
 def network_classify_batch(net: Network, images: np.ndarray | None = None, frames: np.ndarray | None = None,

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Developer tool (GPU box): device-memory leak check - parse / predict / detect / resize / free in a loop,
 parse / classify / change the batch / free for a classifier, frame lists whose packed size grows and shrinks, and
-video streams (open, submit with repeats, reset, reopen larger, change the batch, free)."""
+video streams (open, submit with repeats, reset, reopen larger, change the batch, free) and tracked video streams
+(enable tracking, submit with repeats, reset, reopen and enable again, change the batch, free)."""
 import sys
 import tempfile
 from pathlib import Path
@@ -111,9 +112,35 @@ def streams_cycle(name, side, batch):
     dn.free_network(net)
 
 
+def tracked_cycle(name, side, batch):
+    text = synth.CFGS[name](batch=batch, w=side, h=side)
+    (tmp / "t.cfg").write_text(text)
+    w = tmp / f"{name}.weights"
+    if not w.exists():
+        synth.write_weights(w, text, seed=1)
+    net = dn.parse_network_cfg(tmp / "t.cfg")
+    dn.load_weights(net, w)
+    rng = np.random.default_rng(4)
+    frames = [rng.integers(0, 256, size=(375, 500, 3), dtype=np.uint8) for _ in range(batch)]
+    dn.network_streams_open(net, 4)
+    dn.network_streams_track(net, 6)
+    ids = [i % 3 for i in range(batch)]
+    dn.network_detect_submit_streams_tracked(net, ids, frames, 0.02, 0.4, True, 64)
+    dn.network_detect_submit_streams_tracked(net, ids[::-1], frames, 0.02, 0.4, False, 64)
+    dn.network_stream_reset(net, 1)
+    dn.network_detect_wait_tracked(net, batch, 64)
+    dn.network_detect_wait_tracked(net, batch, 64)
+    dn.network_streams_open(net, 64)  # reopen larger: tracking is dropped, enable it again with a longer story
+    dn.network_streams_track(net, 32)
+    dn.network_detect_streams_tracked(net, list(range(batch)), frames, 0.02, 0.4, True, 64)
+    dn.set_batch_network(net, batch * 2)  # a re-plan that keeps the tracks
+    dn.network_detect_streams_tracked(net, [5] * batch, frames, 0.02, 0.4, False, 64)
+    dn.free_network(net)
+
+
 for fn, name, side, batch in ((cycle, "tiny-yolo-voc", 416, 8), (cycle, "yolo-voc", 416, 64),
                               (classify_cycle, "darknet19_448", 448, 16), (frame_list_cycle, "tiny-yolo-voc", 416, 16),
-                              (streams_cycle, "tiny-yolo-voc", 416, 16)):
+                              (streams_cycle, "tiny-yolo-voc", 416, 16), (tracked_cycle, "tiny-yolo-voc", 416, 16)):
     fn(name, side, batch)  # warm: allocator pools, per-device scratch
     torch.cuda.synchronize()
     free0, _ = torch.cuda.mem_get_info()
