@@ -100,8 +100,7 @@ __device__ __forceinline__ void slab_store_f32_staged(const SlabParams &prm, uin
             if (ch + 4 <= prm.cout) {
                 // streaming store: 2 GB of head output per yolo9000 step must not push the 58 MB weight matrix (read
                 // again for every position tile) out of the L2
-                if (prm.dbg & 16) *reinterpret_cast<uint4 *>(o) = q;
-                else __stcs(reinterpret_cast<uint4 *>(o), q);
+                __stcs(reinterpret_cast<uint4 *>(o), q);
             } else {  // the last filters of a head whose count is not a multiple of 4
                 o[0] = __uint_as_float(q.x);
                 if (ch + 1 < prm.cout) o[1] = __uint_as_float(q.y);
@@ -141,7 +140,7 @@ __device__ __forceinline__ void slab_affine_pack(const uint32_t (&v)[32], const 
 // copy engine writes full 128-byte lines, the LSU sees 8 shared-memory stores per thread instead of 8
 // global stores that touch 32 different lines each.
 __device__ __forceinline__ void slab_store_tma(const void *tm_out, uint4 *stage, const uint4 (&w)[8], int lane,
-                                               int p_first, int ch0, bool issue = true)
+                                               int p_first, int ch0)
 {
     // the previous box of this warp must have been read out of the staging tile
     if (lane == 0) tma_store_wait_read();
@@ -150,7 +149,7 @@ __device__ __forceinline__ void slab_store_tma(const void *tm_out, uint4 *stage,
     for (int c = 0; c < 8; ++c) stage[lane * 8 + (c ^ (lane & 7))] = w[c];
     fence_proxy_async();
     __syncwarp();
-    if (lane == 0 && issue) {
+    if (lane == 0) {
         tma_store_2d(tm_out, stage, ch0, p_first);
         tma_store_commit();
     }

@@ -88,7 +88,7 @@ template <int TAPS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kPairThreads, 1)
 conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
                  const __grid_constant__ CUtensorMap tm_b32, const __grid_constant__ CUtensorMap tm_out,
-                 const SlabParams prm)
+                 const __grid_constant__ SlabParams prm)
 {
     extern __shared__ uint8_t smem_raw[];
     // identical carve-up in both CTAs: descriptors and barrier offsets name the peer's memory too
@@ -175,21 +175,6 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
         // ===================== weight producer (both CTAs, own half of the piece's filters) =====
         int stage = 0;
         uint32_t phase = 0;
-        int issued = 0;
-        if (TAPS == 1 && prm.b_resident) {
-            // 1x1 layer whose whole weight half fits: stage nt * cblocks + cb holds channel block cb of filter tile nt
-            // for the lifetime of the CTA (loaded under the previous layer's tail, never released)
-            if (elect_one_sync()) {
-                for (int nt = 0; nt < prm.tiles_n; ++nt)
-                    for (int cb = 0; cb < cblocks; ++cb) {
-                        const int st = nt * cblocks + cb;
-                        if (leader) mbar_expect_tx(&b_full[st], 2u * kPairBHalfBytes);
-                        tma_load_2d_pair(&tm_b, &b_full[st], smem_b + (size_t)st * kPairBHalfBytes, cb * kPairBK,
-                                         nt * kPairN + (int)rank * 128);
-                    }
-            }
-            __syncwarp();
-        } else
         while (sched.next(seg)) {
             const int half_rows = seg.ncols >> 1;  // 32, 64, 96 or 128 filters per CTA
             const int n0 = seg.n0 + (int)rank * half_rows;
@@ -198,21 +183,15 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
 #pragma unroll 1
                 for (int tap = 0; tap < TAPS; ++tap) {
                     mbar_wait(&b_empty[stage], phase ^ 1, 2);
-                    const bool skip = (prm.dbg & 1) && (tap & 1) && issued >= 2 * stages_b;
-                    ++issued;
                     if (elect_one_sync()) {
                         uint8_t *sb = smem_b + (size_t)stage * kPairBHalfBytes;
                         const int k0 = (tap * cblocks + cb) * kPairBK;
-                        if (skip) {  // timing experiment: the stage "completes" with stale bytes
-                            if (leader) mbar_arrive(&b_full[stage]);
-                        } else {
-                            if (leader) mbar_expect_tx(&b_full[stage], tx);
-                            if (half_rows == 128) {
-                                tma_load_2d_pair(&tm_b, &b_full[stage], sb, k0, n0);
-                            } else {  // narrow piece: 32-filter boxes, only the rows the MMA reads
-                                for (int r = 0; r < half_rows; r += 32)
-                                    tma_load_2d_pair(&tm_b32, &b_full[stage], sb + r * kPairRowBytes, k0, n0 + r);
-                            }
+                        if (leader) mbar_expect_tx(&b_full[stage], tx);
+                        if (half_rows == 128) {
+                            tma_load_2d_pair(&tm_b, &b_full[stage], sb, k0, n0);
+                        } else {  // narrow piece: 32-filter boxes, only the rows the MMA reads
+                            for (int r = 0; r < half_rows; r += 32)
+                                tma_load_2d_pair(&tm_b32, &b_full[stage], sb + r * kPairRowBytes, k0, n0 + r);
                         }
                     }
                     __syncwarp();
@@ -224,7 +203,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
         // ===================== MMA issuer (leader CTA only) =====================
         if (leader) {
             int sa_i = 0, sb_i = 0;
-            uint32_t pa = 0, pb = 0, b_seen = 0;
+            uint32_t pa = 0, pb = 0;
             int it = 0;
             const uint32_t a_lo0 = ((smem_u32(smem_a) & 0x3FFFFu) >> 4) | (1u << 16);
             const uint32_t b_lo0 = ((smem_u32(smem_b) & 0x3FFFFu) >> 4) | (1u << 16);
@@ -244,16 +223,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                     const uint32_t acc_first = cb != 0;
 #pragma unroll
                     for (int tap = 0; tap < TAPS; ++tap) {
-                        const bool resident = TAPS == 1 && prm.b_resident;
-                        if (resident) {  // the stage never changes: wait for its one and only fill, once
-                            sb_i = (seg.n0 >> 8) * cblocks + cb;
-                            if (!((b_seen >> sb_i) & 1u)) {
-                                mbar_wait(&b_full[sb_i], 0, 5);
-                                b_seen |= 1u << sb_i;
-                            }
-                        } else {
-                            mbar_wait(&b_full[sb_i], pb, 5);
-                        }
+                        mbar_wait(&b_full[sb_i], pb, 5);
                         tc_fence_after();
                         if (elect_one_sync()) {
                             const uint32_t b_lo = b_lo0 + (uint32_t)sb_i * (kPairBHalfBytes >> 4);
@@ -263,14 +233,14 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                                 umma_bf16_pair(d0, ((uint64_t)kPairDescHi << 32) | (uint64_t)(a_tap + (uint32_t)(k * 2)),
                                                ((uint64_t)kPairDescHi << 32) | (uint64_t)(b_lo + (uint32_t)(k * 2)),
                                                idesc, (tap == 0 && k == 0) ? acc_first : 1u);
-                            if (!resident) umma_commit_pair(&b_empty[sb_i]);
+                            umma_commit_pair(&b_empty[sb_i]);
                             if (tap == TAPS - 1) {
                                 umma_commit_pair(&a_empty[sa_i]);
                                 if (cb == cblocks - 1) umma_commit_pair(&tfull_bar[buf]);
                             }
                         }
                         __syncwarp();
-                        if (!resident && ++sb_i == stages_b) { sb_i = 0; pb ^= 1; }
+                        if (++sb_i == stages_b) { sb_i = 0; pb ^= 1; }
                     }
                     if (++sa_i == stages_a) { sa_i = 0; pa ^= 1; }
                 }
@@ -379,20 +349,13 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
 // -------------------------------------------------------------------------------------
 // ---- work lists ------------------------------------------------------------------------
 // Cost of one piece of n 64-filter units, in units of a quarter of a full 256-filter piece.  Measured on B200
-// (yolo-voc L23 at batch 64 with every piece forced to one width, Y2_PAIR_FORCE_UNITS, profiles/r2k_pair_balance.txt):
+// (yolo-voc L23 at batch 64 with every piece forced to one width, profiles/r2k_pair_balance.txt; the switch that
+// forced the width was removed later and is in the history):
 // a tcgen05.mma.cta_group::2 of M = 256, K = 16 takes ~95 / 105 / 115 / 128 clk at N = 64 / 128 / 192 / 256, i.e. it
 // has a floor of ~90 clk whatever N is - each SM fetches its 4 KB A operand (and N/2 rows of B) from shared memory at
 // ~64 B/clk, which at N = 256 (8 KB) is exactly the 128 clk the tensor pipe needs.  Narrow pieces are therefore
 // expensive and the balanced cut only uses them where they shorten the longest list (the 13x13 layers: -1.3 %).
-// Y2_PAIR_COST=c1,c2,c3 overrides the table.
-static void pair_piece_costs(double c[5])
-{
-    c[0] = 0.0; c[1] = 2.97; c[2] = 3.28; c[3] = 3.6; c[4] = 4.0;
-    if (const char *e = getenv("Y2_PAIR_COST")) {
-        double a, b, cc;
-        if (sscanf(e, "%lf,%lf,%lf", &a, &b, &cc) == 3) { c[1] = a; c[2] = b; c[3] = cc; }
-    }
-}
+static constexpr double kPairPieceCost[5] = {0.0, 2.97, 3.28, 3.6, 4.0};
 
 // rows = position tiles, U = 64-filter units per row (a multiple of 4), P pairs.
 // balanced: the row-major unit sequence is cut into P contiguous ranges of minimal largest cost (binary search on
@@ -403,8 +366,7 @@ static void pair_schedule(int rows, int U, int P, bool balanced, std::vector<int
     std::vector<std::vector<int4>> lists(P);
     const long long T = (long long)rows * U;
     if (balanced && rows * (U / 4) > P) {
-        double c[5];
-        pair_piece_costs(c);
+        const double *c = kPairPieceCost;
         std::vector<double> g(U + 1, 0.0);   // cheapest split of r units of one row
         std::vector<int> first(U + 1, 0);    // size of the first piece of that split
         for (int r = 1; r <= U; ++r) {
@@ -467,15 +429,9 @@ static void pair_schedule(int rows, int U, int P, bool balanced, std::vector<int
     bool any = false;
     for (const auto &l : lists) any = any || !l.empty();
     if (!any) {
-        // Y2_PAIR_FORCE_UNITS=1..3: pieces of that many units round-robin (measures the cost table above)
-        int wu = 4;
-        if (const char *e = getenv("Y2_PAIR_FORCE_UNITS")) wu = atoi(e) >= 1 && atoi(e) <= 4 ? atoi(e) : 4;
         long long t = 0;
         for (int row = 0; row < rows; ++row)
-            for (int j = 0; j < U; j += wu, ++t) {
-                const int n = U - j < wu ? U - j : wu;
-                lists[(size_t)(t % P)].push_back(make_int4(row, j * 64, n * 64, 0));
-            }
+            for (int j = 0; j < U; j += 4, ++t) lists[(size_t)(t % P)].push_back(make_int4(row, j * 64, 256, 0));
     }
     size_t longest = 0;
     for (const auto &l : lists) longest = l.size() > longest ? l.size() : longest;
@@ -485,7 +441,7 @@ static void pair_schedule(int rows, int U, int P, bool balanced, std::vector<int
         for (size_t i = 0; i < lists[q].size(); ++i) work[(size_t)q * stride + i] = lists[q][i];
 }
 
-int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
+int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d, ConvChoice choice)
 {
     if ((d->ksize != 3 && d->ksize != 1) || d->block_k != kPairBK || d->block_n != 256 || d->npad % kPairN ||
         d->cin % kPairBK)
@@ -496,21 +452,16 @@ int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     // wide fp32 heads (yolo9000: 28 269 filters over 1024 channels, a third of that network's step): one-tap form
     // with the staged row-contiguous fp32 stores of conv_epilogue.cuh
     const bool f32_head = taps == 1 && d->out_mode == Y2_OUT_F32_FLAT && d->cout >= 512 && d->out_cs % 4 == 0 &&
-                          ((uintptr_t)d->out & 15) == 0 && !getenv("Y2_SLAB_NO_F32_STAGE") && !getenv("Y2_PAIR_NO_F32_HEAD");
+                          ((uintptr_t)d->out & 15) == 0;
     // other 1x1 layers: only bf16 tensors through the TMA-store epilogue
     if (taps == 1 && !f32_head && (d->out_mode != Y2_OUT_BF16_PADDED || d->cout % 64)) return Y2_EINVAL;
     // 1x1 layers: the one-tap form of this kernel measured 21.0 us (L19, 1024 -> 512) against 20.1 of the slab kernel,
-    // so it is only used when asked for (Y2_CONV_VARIANT=pair; tests).  Y2_PAIR_RESIDENT=1 additionally keeps the CTA's
-    // half of the WHOLE weight matrix in shared memory when it fits next to two activation stages (npad * cin <= 8
-    // stages of 16 KB: yolo-voc L13 / L15, 512 -> 256): that halves the L2 -> shared traffic (ncu: 106 -> 68 MB) and
-    // still loses, 18.2 us against 16.5 of the slab kernel (profiles/r2o_resident.txt) - with three activation stages
-    // left the K loop of a 1x1 layer (8 steps of 512 clk per tile) is latency-bound, not traffic-bound.
-    const int resident_stages = (d->npad / kPairN) * (d->cin / kPairBK);
-    const char *forced = getenv("Y2_CONV_VARIANT");
-    const bool forced_pair = forced && !strcmp(forced, "pair");
-    const char *res_env = getenv("Y2_PAIR_RESIDENT");
-    const bool resident = taps == 1 && resident_stages <= 8 && res_env && atoi(res_env) != 0;
-    if (taps == 1 && !forced_pair && !f32_head && !(resident && total >= 2ll * 256 * (sm_count() / 2))) return Y2_EINVAL;
+    // so it is only used when asked for (Y2_CONV_VARIANT=pair; tests).  Keeping the CTA's half of the WHOLE weight
+    // matrix in shared memory (yolo-voc L13 / L15, 512 -> 256) halves the L2 -> shared traffic (ncu: 106 -> 68 MB) and
+    // still loses, 18.2 us against 16.5 of the slab kernel (profiles/r2o_resident.txt; that resident-weights form was
+    // removed later and is in the history) - with three activation stages left the K loop of a 1x1 layer (8 steps of
+    // 512 clk per tile) is latency-bound, not traffic-bound.
+    if (taps == 1 && choice != kChoosePair && !f32_head) return Y2_EINVAL;
     const int halo = taps == 9 ? wp + 1 : 0;
     const int slab_rows = 128 + 2 * halo;
     const int loads = (slab_rows + 255) / 256;
@@ -520,18 +471,10 @@ int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     const int slab_bytes = loads * box_rows * kPairRowBytes;
     const int aux = ((2 * kPairN * 8 + 512 + 1023) / 1024) * 1024 + 8 * 4096;  // alpha/beta, barriers | store staging
     const int budget = 227 * 1024 - 1024 - aux;
-    int stages_a = taps == 9 ? 2 : kPairMaxStagesA;  // 1x1: a fresh A tile every K step
-    int stages_b;
-    if (resident) {
-        stages_b = resident_stages;
-        stages_a = (budget - stages_b * kPairBHalfBytes) / slab_bytes;
-        if (stages_a > kPairMaxStagesA) stages_a = kPairMaxStagesA;
-        if (stages_a < 2) return Y2_EINVAL;
-    } else {
-        stages_b = (budget - stages_a * slab_bytes) / kPairBHalfBytes;
-        if (stages_b > kPairMaxStagesB) stages_b = kPairMaxStagesB;
-        if (stages_b < 4) return Y2_EINVAL;
-    }
+    const int stages_a = taps == 9 ? 2 : kPairMaxStagesA;  // 1x1: a fresh A tile every K step
+    int stages_b = (budget - stages_a * slab_bytes) / kPairBHalfBytes;
+    if (stages_b > kPairMaxStagesB) stages_b = kPairMaxStagesB;
+    if (stages_b < 4) return Y2_EINVAL;
     const int sms = sm_count();
     if (sms < 2) return Y2_EINVAL;
     const int ktot = taps * d->cin;
@@ -562,10 +505,8 @@ int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     p.out_cs = d->out_cs;
     p.couple = 0;
     p.tma_store = 0;
-    p.dbg = getenv("Y2_PAIR_DBG") ? atoi(getenv("Y2_PAIR_DBG")) : 0;
-    p.b_resident = resident ? 1 : 0;
     memset(&pl->tm_out, 0, sizeof(pl->tm_out));
-    if (d->out_mode == Y2_OUT_BF16_PADDED && d->cout % 64 == 0 && !getenv("Y2_SLAB_NO_TMA_STORE")) {
+    if (d->out_mode == Y2_OUT_BF16_PADDED && d->cout % 64 == 0) {
         rc = encode_2d_bf16(&pl->tm_out, d->out, (uint64_t)d->cout, (uint64_t)total, (uint64_t)d->out_cs * 2, 64u, 32u, 64);
         if (rc != Y2_OK) return rc;
         p.tma_store = 1;
@@ -588,8 +529,7 @@ int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     std::vector<int4> work;
     int stride = 0;
     const char *bal = getenv("Y2_PAIR_BALANCE");
-    // resident weights are laid out per 256-filter tile: whole tiles only
-    pair_schedule(p.tiles_m, d->npad / 64, pairs, !(bal && atoi(bal) == 0) && !resident, work, stride);
+    pair_schedule(p.tiles_m, d->npad / 64, pairs, !(bal && atoi(bal) == 0), work, stride);
     Y2_CUDA_CHECK(cudaMalloc(&pl->work_buf, work.size() * sizeof(int4)));
     Y2_CUDA_CHECK(cudaMemcpy(pl->work_buf, work.data(), work.size() * sizeof(int4), cudaMemcpyHostToDevice));
     p.work = (const int4 *)pl->work_buf;

@@ -28,6 +28,9 @@ struct ConvParams {
 };
 
 // ---- slab kernel (conv_slab.cu) ------------------------------------------------------
+// The slab and pair kernels take it __grid_constant__, so its fields are read from the parameter bank where they
+// are used.  Without the qualifier the 128-byte struct is copied into registers up front, and the CTA-pair 3x3
+// kernel spills more.
 struct SlabParams {
     int cblocks;           // cin / BLOCK_K
     int wp, hp, h, w;
@@ -44,9 +47,6 @@ struct SlabParams {
     int reverse;           // slab kernel: walk the position tiles last-to-first (see slab_plan_init)
     const int4 *work;      // pair kernel: per-pair lists of pieces (m_tile, n0, ncols, -), ncols == 0 terminates
     int work_stride;       // entries per pair in `work`
-    int b_resident;        // pair kernel, 1x1: the CTA's half of the whole weight matrix stays in shared memory
-    int dbg;               // timing experiments only, WRONG results (Y2_PAIR_DBG / Y2_SLAB_DBG): 1 = pair kernel skips the weight
-                           // loads of odd taps, 2 = slab kernel skips the epilogue math and stores, 4 = slab kernel issues no MMAs
     const float *alpha;
     const float *beta;
     void *out;
@@ -70,6 +70,10 @@ struct PoolParams {
 };
 
 enum { kVariantPerTap = 0, kVariantSlab = 1, kVariantPair = 2, kVariantPool = 3 };
+
+// Y2_CONV_VARIANT, read once per plan by y2_conv_plan_create: unset = auto, pertap | slab | pair restrict the
+// choice (an unknown value is pertap)
+enum ConvChoice { kChooseAuto, kChoosePerTap, kChooseSlab, kChoosePair };
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *,
                                   const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
@@ -100,10 +104,10 @@ struct y2_conv_plan {
 namespace y2 {
 // conv_slab.cu: returns Y2_OK and fills the plan when the layer fits the slab kernel, Y2_EINVAL
 // (without touching the error string) when it does not and the per-tap kernel must be used
-int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d);
+int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d, ConvChoice choice);
 int slab_plan_launch(const y2_conv_plan *pl, cudaStream_t st);
 // conv_pair.cu: the CTA-pair (cta_group::2) kernel for wide 3x3 layers, same contract
-int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d);
+int pair_plan_init(y2_conv_plan *pl, const y2_conv_desc *d, ConvChoice choice);
 int pair_plan_launch(const y2_conv_plan *pl, cudaStream_t st);
 // conv_pool.cu: 3x3 convolution fused with the following 2x2/2 maxpool (out_mode Y2_OUT_BF16_POOLED)
 int pool_plan_init(y2_conv_plan *pl, const y2_conv_desc *d);

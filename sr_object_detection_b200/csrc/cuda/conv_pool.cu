@@ -24,8 +24,6 @@
 // the epilogue is a long dependent chain per thread, so it is spread over many warps.
 #include "conv_plan.cuh"
 
-#include <stdlib.h>
-
 namespace y2 {
 
 constexpr int kPoolThreads = 608;  // 3 producer / MMA warps + 16 epilogue warps
@@ -427,7 +425,6 @@ int pool_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     p.out_cs = d->out_cs;
     // start with the part of a large input that is still in the L2 (see conv_slab.cu, `reverse`)
     p.reverse = (double)d->batch * (d->h + 1) * (d->w + 1) * d->in_cs * 2.0 > 64e6 && !d->in_order;
-    if (const char *e = getenv("Y2_SLAB_REVERSE")) p.reverse = atoi(e) != 0;
     pl->variant = kVariantPool;
     pl->block_n = bn;
     pl->block_k = bk;

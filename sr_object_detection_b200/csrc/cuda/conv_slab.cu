@@ -29,7 +29,6 @@
 // elect one lane per issue (see elect_one_sync in y2_common.cuh).
 #include "conv_epilogue.cuh"
 
-#include <stdlib.h>
 #include <string.h>
 
 namespace y2 {
@@ -67,7 +66,7 @@ __device__ __forceinline__ uint64_t slab_desc(uint32_t hi, uint32_t lo)
 template <int BLOCK_N, int BLOCK_K, int ACCS, int TPS, int TAPS>
 __global__ void __launch_bounds__(kSlabThreads, 1)
 conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
-                 const __grid_constant__ CUtensorMap tm_out, const SlabParams prm)
+                 const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ SlabParams prm)
 {
     using Cfg = SlabCfg<BLOCK_N, BLOCK_K, ACCS, TPS, TAPS>;
     constexpr int kTileM = Cfg::kTileM;
@@ -122,7 +121,8 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    // the TMEM base is read from *tmem_slot where it is used rather than held in a register for the whole kernel:
+    // the epilogue warps run at the 168-register cap
 
     pdl_launch_dependents();
     if (warp == 0) {
@@ -191,7 +191,7 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
             const uint32_t buf_phase = (it >> 1) & 1;
             mbar_wait(&tempty_bar[buf], buf_phase ^ 1, 3);
             tc_fence_after();
-            const uint32_t d0 = tmem_base + (uint32_t)(buf * ACCS * BLOCK_N);
+            const uint32_t d0 = *tmem_slot + (uint32_t)(buf * ACCS * BLOCK_N);
             for (int cb = 0; cb < cblocks; ++cb) {
                 mbar_wait(&a_full[sa_i], pa, 4);
                 const uint32_t a_lo = a_lo0 + (uint32_t)sa_i * slab16;
@@ -208,7 +208,6 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                         const uint32_t a_tap = a_lo + (uint32_t)(tap / 3) * wp16 + (uint32_t)(tap % 3) * kRow16;
 #pragma unroll
                         for (int a = 0; a < ACCS; ++a) {
-                            if (prm.dbg & 4) break;  // timing experiment: no tensor work
 #pragma unroll
                             for (int k = 0; k < BLOCK_K / 16; ++k)
                                 umma_bf16(d0 + (uint32_t)(a * BLOCK_N),
@@ -271,7 +270,7 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
             const int y = rem / prm.wp;
             const int x = rem - y * prm.wp;
             const bool valid = in_range && (y < prm.h) && (x < prm.w);
-            const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) +
+            const uint32_t taddr = *tmem_slot + ((uint32_t)(quarter * 32) << 16) +
                                    (uint32_t)((buf * ACCS + acc) * BLOCK_N + col0);
 
             mbar_wait(&tfull_bar[buf], buf_phase, 6);
@@ -286,10 +285,6 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                     if (c + 64 >= kSpan) {  // accumulator drained into registers: hand it back to the MMA warp
                         tc_fence_before();
                         mbar_arrive(&tempty_bar[buf]);
-                    }
-                    if (prm.dbg & 2) {  // timing experiment: no epilogue math, no stores (keeps the loads alive)
-                        if (v0[0] == 0x7fc12345u && v1[31] == 0x7fc54321u) s_ab[0].x = 1.f;
-                        continue;
                     }
                     if (prm.tma_store == 2) {  // fp32 flat head: staged, row-contiguous 16-byte stores
                         const long long fr = valid ? ((long long)b * prm.h + y) * prm.w + x : -1ll;
@@ -316,7 +311,7 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                             slab_affine_pack<Y2_ACT_LOGISTIC>(v0, sab, col0 + c, valid, w);
                             slab_affine_pack<Y2_ACT_LOGISTIC>(v1, sab, col0 + c + 32, valid, w + 4);
                         }
-                        slab_store_tma(&tm_out, s_stage + (warp - 3) * 256, w, lane, p - lane, n0 + col0 + c, !(prm.dbg & 8));
+                        slab_store_tma(&tm_out, s_stage + (warp - 3) * 256, w, lane, p - lane, n0 + col0 + c);
                     } else if (prm.act == Y2_ACT_LEAKY) {
                         slab_epilogue_chunk<Y2_ACT_LEAKY>(prm, v0, sab, col0 + c, n0, p, b, y, x, in_range, valid);
                         slab_epilogue_chunk<Y2_ACT_LEAKY>(prm, v1, sab, col0 + c + 32, n0, p, b, y, x, in_range, valid);
@@ -349,7 +344,7 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
     tc_fence_before();
     __syncthreads();
     if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base),
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*tmem_slot),
                      "r"((uint32_t)Cfg::kTmemCols)
                      : "memory");
     }
@@ -387,7 +382,7 @@ static int slab_prepare_cfg()
     return Y2_OK;
 }
 
-int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
+int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d, ConvChoice choice)
 {
     const int taps = d->ksize * d->ksize;
     const int bn = d->block_n;
@@ -435,7 +430,7 @@ int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     // positions, SWIZZLE_128B): pad positions are stored as zeros like before, rows past the tensor are clipped
     p.tma_store = 0;
     memset(&pl->tm_out, 0, sizeof(pl->tm_out));
-    if (d->out_mode == Y2_OUT_BF16_PADDED && bn >= 64 && d->cout % 64 == 0 && !getenv("Y2_SLAB_NO_TMA_STORE")) {
+    if (d->out_mode == Y2_OUT_BF16_PADDED && bn >= 64 && d->cout % 64 == 0) {
         rc = encode_2d_bf16(&pl->tm_out, d->out, (uint64_t)d->cout, (uint64_t)total, (uint64_t)d->out_cs * 2, 64u, 32u, 64);
         if (rc != Y2_OK) return rc;
         p.tma_store = 1;
@@ -443,7 +438,7 @@ int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     // fp32 heads with 16-byte aligned rows: staged row-contiguous stores (conv_epilogue.cuh) instead of 32 scalar
     // stores per lane and chunk
     const bool f32_staged = d->out_mode == Y2_OUT_F32_FLAT && bn >= 128 && d->out_cs % 4 == 0 &&
-                            ((uintptr_t)d->out & 15) == 0 && !getenv("Y2_SLAB_NO_F32_STAGE");
+                            ((uintptr_t)d->out & 15) == 0;
     if (f32_staged) p.tma_store = 2;
     p.cblocks = d->cin / bk;
     p.wp = wp;
@@ -466,7 +461,6 @@ int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     p.alpha = d->alpha;
     p.beta = d->beta;
     p.out = d->out;
-    p.dbg = getenv("Y2_SLAB_DBG") ? atoi(getenv("Y2_SLAB_DBG")) : 0;  // timing experiments (wrong results)
     // measured on B200: lock-stepped epilogue warps write 128-byte rows (<= 64 filters) 10% faster, wider
     // rows prefer free-running warps
     p.couple = bn <= 64;
@@ -478,7 +472,6 @@ int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     // threshold.
     // The producer may itself have walked last-to-first (in_order 1): then the resident end is the front.
     p.reverse = (double)d->batch * hp * wp * d->in_cs * 2.0 > 64e6 && !d->in_order;
-    if (const char *e = getenv("Y2_SLAB_REVERSE")) p.reverse = atoi(e) != 0;
     pl->variant = kVariantSlab;
     pl->block_n = bn;
     pl->block_k = bk;
@@ -488,9 +481,7 @@ int slab_plan_init(y2_conv_plan *pl, const y2_conv_desc *d)
     // 1x1 layers: the 256-position tiles pay off only while every SM still gets two or more of them and
     // the output is the bf16 tensor (measured on B200: L5/L9/L13 +5..15%, the 13x13 layers and the fp32
     // head are faster on the per-tap kernel's 128-position tiles)
-    int min_tiles = 2 * sms;
-    if (const char *e = getenv("Y2_SLAB_1X1_MIN_TILES")) min_tiles = atoi(e);
-    if (taps == 1 && !f32_staged && (tiles < min_tiles || d->out_mode != Y2_OUT_BF16_PADDED) && !getenv("Y2_CONV_VARIANT"))
+    if (taps == 1 && !f32_staged && (tiles < 2 * sms || d->out_mode != Y2_OUT_BF16_PADDED) && choice == kChooseAuto)
         return Y2_EINVAL;
     pl->grid = tiles < sms ? tiles : sms;
     pl->taps = taps;

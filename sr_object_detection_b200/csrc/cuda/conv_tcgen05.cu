@@ -374,7 +374,8 @@ extern "C" int y2_conv_plan_create(const y2_conv_desc *d, y2_conv_plan **out_pla
     const int ktot = taps * d->cin;
     // kernel choice: CTA-pair kernel for wide 3x3 layers, halo-slab kernel for the other 3x3 layers, this
     // file's per-tap kernel for 1x1 layers and whatever does not fit.  Y2_CONV_VARIANT=pertap|slab|pair
-    // restricts the choice (tests, A/B timing).
+    // restricts the choice (tests, A/B timing); slab and pair also lift the slab kernel's 1x1 preference, pair
+    // admits 1x1 layers to the one-tap pair kernel.
     if (d->out_mode == Y2_OUT_BF16_POOLED) {
         const int rc = pool_plan_init(pl, d);
         if (rc != Y2_OK) {
@@ -385,13 +386,15 @@ extern "C" int y2_conv_plan_create(const y2_conv_desc *d, y2_conv_plan **out_pla
         return Y2_OK;
     }
     const char *forced = getenv("Y2_CONV_VARIANT");
-    const bool allow_pair = !forced || !strcmp(forced, "pair");
-    const bool allow_slab = !forced || !strcmp(forced, "slab") || !strcmp(forced, "pair");
-    if (allow_pair && pair_plan_init(pl, d) == Y2_OK) {
+    const ConvChoice choice = !forced                  ? kChooseAuto
+                              : !strcmp(forced, "slab") ? kChooseSlab
+                              : !strcmp(forced, "pair") ? kChoosePair
+                                                        : kChoosePerTap;
+    if ((choice == kChooseAuto || choice == kChoosePair) && pair_plan_init(pl, d, choice) == Y2_OK) {
         *out_plan = pl;
         return Y2_OK;
     }
-    if (allow_slab && slab_plan_init(pl, d) == Y2_OK) {
+    if (choice != kChoosePerTap && slab_plan_init(pl, d, choice) == Y2_OK) {
         *out_plan = pl;
         return Y2_OK;
     }

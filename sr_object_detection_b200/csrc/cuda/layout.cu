@@ -944,7 +944,7 @@ extern "C" int y2_gather_rows_f32(const float *src, void *dst, int batch, int c,
     const int rows = batch * (oh + 1);
     const int cap = sm_count() * 8;
     const size_t smem = (size_t)c * ksize * (w | 1) * sizeof(float);
-    if (smem <= 48 * 1024 && !getenv("Y2_GATHER_DIRECT"))
+    if (smem <= 48 * 1024)
         gather_rows_f32_smem_kernel<<<rows < cap ? rows : cap, 512, smem, to_stream(s)>>>(
             src, (__nv_bfloat16 *)dst, batch, c, h, w, ksize, stride, pad, oh, ow, kpad);
     else

@@ -21,75 +21,12 @@ __device__ __forceinline__ float logistic_ref(float x)
 }
 
 // ---------------------------------------------------------------------------------
-// region forward: one warp per softmax group of one box.
-//   out[0..3] = in[0..3];  out[4] = logistic(in[4]);
-//   out[5+g..] = softmax over the group (blas.c:205-221): the exps are evaluated by the
-//   lanes in parallel (double exp, rounded to float), the float sum is then accumulated in
-//   index order by shuffling the terms through lane 0's order, so it is the same sequence
-//   of roundings as the reference's serial loop.
-// ---------------------------------------------------------------------------------
-__global__ void region_forward_kernel(const float *in, int in_cs, int anchors, float *out,
-                                      long long boxes, int classes, int softmax, int n_groups,
-                                      const int *__restrict__ group_size,
-                                      const int *__restrict__ group_offset)
-{
-    const int lane = threadIdx.x & 31;
-    const long long warp_global = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
-    const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
-    const int size = classes + 5;
-    const int groups = n_groups > 0 ? n_groups : 1;
-    const long long work = boxes * groups;
-    for (long long wi = warp_global; wi < work; wi += nwarps) {
-        const long long box = wi / groups;
-        const int g = (int)(wi - box * groups);
-        const float *x = in + (box / anchors) * in_cs + (box % anchors) * size;
-        float *o = out + box * size;
-        if (g == 0 && lane < 5) o[lane] = (lane == 4) ? logistic_ref(x[4]) : x[lane];
-        int off = 0, n = classes;
-        if (n_groups > 0) {
-            off = group_offset[g];
-            n = group_size[g];
-        }
-        const float *xi = x + 5 + off;
-        float *oi = o + 5 + off;
-        if (!softmax) {
-            for (int i = lane; i < n; i += 32) oi[i] = xi[i];
-            continue;
-        }
-        float largest = -FLT_MAX;
-        for (int i = lane; i < n; i += 32) {
-            const float v = xi[i];
-            if (v > largest) largest = v;
-        }
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            const float other = __shfl_xor_sync(0xffffffffu, largest, d);
-            if (other > largest) largest = other;
-        }
-        // temp == 1: input[i]/temp - largest/temp is a float expression
-        float sum = 0.f;
-        for (int base = 0; base < n; base += 32) {
-            const int i = base + lane;
-            float e = 0.f;
-            if (i < n) {
-                const float arg = xi[i] / 1.f - largest / 1.f;
-                e = (float)exp((double)arg);
-                oi[i] = e;
-            }
-            const int cnt = (n - base) < 32 ? (n - base) : 32;
-            for (int j = 0; j < cnt; ++j) sum = sum + __shfl_sync(0xffffffffu, e, j);
-        }
-        for (int i = lane; i < n; i += 32) oi[i] = oi[i] / sum;
-    }
-}
-
-// ---------------------------------------------------------------------------------
 // region forward, WordTree softmax (softmax_tree, softmax_layer.c:35-47): one LANE per (box, group).
 // The groups of a WordTree are small (9k.tree: 1723 groups, median 3, 99th percentile 28 classes), so a
-// warp per group (region_forward_kernel above) wastes 29 of 32 lanes on 26 million warp tasks at
-// yolo9000 batch 16 (8 ms).  Here every lane runs the reference's three serial loops over its own
-// group; the few groups wider than a warp are then finished by the whole warp, lanes over classes, the
-// float sum still accumulated in class order.
+// warp per group wastes 29 of 32 lanes on 26 million warp tasks at yolo9000 batch 16 (8 ms; that
+// warp-per-group kernel was removed later and is in the history).  Here every lane runs the
+// reference's three serial loops over its own group; the few groups wider than a warp are then
+// finished by the whole warp, lanes over classes, the float sum still accumulated in class order.
 // ---------------------------------------------------------------------------------
 __global__ void region_forward_tree_kernel(const float *__restrict__ in, int in_cs, int anchors, float *__restrict__ out, long long boxes,
                                            int classes, int softmax, int n_groups,
@@ -181,7 +118,7 @@ __global__ void region_forward_tree_kernel(const float *__restrict__ in, int in_
 
 // ---------------------------------------------------------------------------------
 // region forward, flat softmax (no tree): FOUR lanes per box, eight boxes per warp.
-// The warp-per-group kernel above spends a whole warp on 20 classes plus a serial logistic in one
+// A warp per box spends a whole warp on 20 classes plus a serial logistic in one
 // lane and is issue-bound (54 080 boxes x ~250 warp instructions at yolo-voc b64).  Here lane q of
 // a box evaluates the double-precision exps of classes q, q+4, ... and one of the pass-through /
 // objectness values; the float sum still runs in class order: round k hands the four terms of
@@ -1297,16 +1234,9 @@ extern "C" int y2_region_forward_strided(const float *in, int in_cs, float *out,
         return Y2_OK;
     }
     const long long work = boxes * n_groups;
-    if (!getenv("Y2_REGION_WARP_PER_GROUP")) {
-        const int grid = grid_cap((work + threads - 1) / threads, 8);
-        region_forward_tree_kernel<<<grid, threads, 0, to_stream(s)>>>(in, in_cs, n, out, boxes, classes, softmax, n_groups,
-                                                                       d_group_size, d_group_offset);
-        Y2_LAUNCH_CHECK();
-        return Y2_OK;
-    }
-    const int grid = grid_cap((work * 32 + threads - 1) / threads, 8);
-    region_forward_kernel<<<grid, threads, 0, to_stream(s)>>>(in, in_cs, n, out, boxes, classes, softmax, n_groups,
-                                                              d_group_size, d_group_offset);
+    const int grid = grid_cap((work + threads - 1) / threads, 8);
+    region_forward_tree_kernel<<<grid, threads, 0, to_stream(s)>>>(in, in_cs, n, out, boxes, classes, softmax, n_groups,
+                                                                   d_group_size, d_group_offset);
     Y2_LAUNCH_CHECK();
     return Y2_OK;
 }

@@ -23,13 +23,6 @@ void set_error(const char *fmt, ...)
     va_end(ap);
 }
 
-bool pdl_enabled()
-{
-    static int cached = -1;
-    if (cached < 0) cached = getenv("Y2_NO_PDL") ? 0 : 1;
-    return cached != 0;
-}
-
 int sm_count()
 {
     static int cached[64] = {0};
@@ -141,8 +134,7 @@ extern "C" int y2_host_alloc(void **hptr, size_t bytes)
     if (bytes >= (1u << 20) && !getenv("Y2_NO_NUMA_BIND") && cudaGetDevice(&dev) == cudaSuccess &&
         sched_getaffinity(0, sizeof(saved), &saved) == 0 && device_local_cpus(dev, &local))
         moved = sched_setaffinity(0, sizeof(local), &local) == 0;
-    const unsigned flags = getenv("Y2_STAGING_WC") && bytes >= (1u << 20) ? cudaHostAllocWriteCombined : cudaHostAllocDefault;
-    const cudaError_t e = cudaHostAlloc(hptr, bytes ? bytes : 16, flags);
+    const cudaError_t e = cudaHostAlloc(hptr, bytes ? bytes : 16, cudaHostAllocDefault);
     if (moved) sched_setaffinity(0, sizeof(saved), &saved);
     Y2_CUDA_CHECK(e);
     return Y2_OK;

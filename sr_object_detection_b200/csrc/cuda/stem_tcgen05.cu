@@ -33,7 +33,6 @@
 // x -> leaky(fma(alpha, x, beta)) is then non-decreasing in fp32, so it commutes with max.
 #include "conv_plan.cuh"
 
-#include <stdlib.h>
 #include <string.h>
 
 namespace y2 {
@@ -501,8 +500,8 @@ static int stem_launch(const void *in, bool u8, int batch, int c, int h, int w, 
         p.use_tma = 2;
     } else {
         p.boxw = p.wt + 8;  // image columns x0 - 4 .. x0 + wt + 3
-        if (enc && w % 4 == 0 && ((uintptr_t)in & 15) == 0 && p.boxw <= kStemBoxW && p.boxw <= w && kStemRows + 2 <= h &&
-            !getenv("Y2_STEM_NO_TMA")) {  // a box never exceeds the tensor it slides over
+        // a box never exceeds the tensor it slides over
+        if (enc && w % 4 == 0 && ((uintptr_t)in & 15) == 0 && p.boxw <= kStemBoxW && p.boxw <= w && kStemRows + 2 <= h) {
             cuuint64_t gdim[3] = {(cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)batch * c};
             cuuint64_t gstr[2] = {(cuuint64_t)w * 4, (cuuint64_t)w * h * 4};
             cuuint32_t box[3] = {(cuuint32_t)p.boxw, (cuuint32_t)(kStemRows + 2), (cuuint32_t)c};

@@ -42,13 +42,12 @@ int sm_count();
 // CTAs of layer i+1 are scheduled on an SM as soon as layer i's CTA there has finished: they set up their barriers,
 // allocate TMEM and prefetch WEIGHT tiles (which do not depend on layer i) while layer i's last wave drains, and
 // only the warp that loads ACTIVATIONS blocks in pdl_wait() until layer i has completed and its stores are visible.
-// Without the attribute both instructions are no-ops.  Y2_NO_PDL=1 launches everything the plain way.
+// Without the attribute both instructions are no-ops.
 // Only the persistent convolution kernels use it.  Measured (profiles/r2q_pdl_small.txt, A/B in one box): with the
 // pool / reorg / shortcut / region / NMS kernels launched the same way the step gets SLOWER (yolo-voc 1.655 -> 1.68 ms,
 // resnet50 2.51 -> 2.60, tiny-yolo-voc 0.673 -> 0.698): once all blocks of such a grid have started, the next
 // convolution's CTAs (227 KB of shared memory, 59 k registers each) take over the SMs one by one and sit in
 // griddepcontrol.wait while the small kernel's tail runs on what is left.
-bool pdl_enabled();
 template <typename... KArgs, typename... Args>
 static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                                      Args... args)
@@ -63,7 +62,7 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -179,7 +179,7 @@ static void detect_tail(y2_net_rt *rt, layer *l, void *head_rt, float *pred, int
 {
     y2_layer_rt *r = (y2_layer_rt *)l->b200;
     const int total = l->w * l->h * l->n;
-    if (l->softmax_tree && rt->defer_region) {
+    if (l->softmax_tree) {
         /* softmax tree: only the groups on the path of classes above .5 are evaluated, straight from the head's
          * raw output; NMS and the pick work on one (class, value) record per box (2 launches) */
         y2_layer_rt *hr = (y2_layer_rt *)head_rt;
@@ -191,9 +191,8 @@ static void detect_tail(y2_net_rt *rt, layer *l, void *head_rt, float *pred, int
         return;
     }
     Y2_CHECK(y2_region_boxes_counted(pred, r->biases_dev, r->boxes_dev, r->probs_dev, B, l->w, l->h, l->n,
-                                     l->classes, 1.f, 1.f, thresh, 0, l->classfix,
-                                     l->softmax_tree ? l->softmax_tree->n : 0, r->tree_parent_dev, 0, 0,
-                                     r->nms_cnt_dev, rt->stream));
+                                     l->classes, 1.f, 1.f, thresh, 0, l->classfix, 0, 0, 0, 0, r->nms_cnt_dev,
+                                     rt->stream));
     if (nms > 0)
         Y2_CHECK(y2_nms_mark(r->boxes_dev, r->probs_dev, r->nms_cnt_dev, B, total, l->classes, nms, rt->stream));
     Y2_CHECK(y2_collect_ws(r->boxes_dev, r->probs_dev, B, total, l->classes, thresh, res->det_dev, res->cnt_dev,
@@ -227,7 +226,7 @@ void network_detect_batch(network net, const float *input, float thresh, float n
 static layer *streams_region(network net)
 {
     layer *l = region_of(net);
-    if (l->softmax_tree || y2_rt(net)->defer_region)
+    if (y2_rt(net)->defer_region)
         error("network streams: needs a flat-softmax region head (a softmax tree defers the region forward, so there "
               "is no dense region output to average)");
     return l;

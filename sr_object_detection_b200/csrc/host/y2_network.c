@@ -650,7 +650,7 @@ static int feeds_only_pool2x2(network *net, int i)
 /* layer 0 over <= 3 channels with <= 32 filters: conv + pool run as the fused first-layer kernel */
 static int stem_fusable(network *net, int i)
 {
-    if (i != 0 || getenv("Y2_NO_STEM_FUSION")) return 0;
+    if (i != 0) return 0;
     layer *l = &net->layers[0];
     if (l->c > 3 || l->n > 32) return 0;
     return feeds_only_pool2x2(net, 0);
@@ -660,7 +660,7 @@ static int stem_fusable(network *net, int i)
  * maxpool runs in the convolution's epilogue (conv_pool.cu) */
 static int pool_fusable(network *net, int i, int cin_pad)
 {
-    if (i == 0 || getenv("Y2_NO_POOL_FUSION")) return 0;
+    if (i == 0) return 0;
     layer *l = &net->layers[i];
     if (cin_pad != 32 && cin_pad != 64) return 0;
     if (l->n != 64 && l->n != 128) return 0;
@@ -1193,7 +1193,7 @@ void y2_plan_network(network *net)
                 free(cgrp);
                 free(fill);
                 Y2_CHECK(y2_malloc(&r->tree_rec_dev, (size_t)B * total * y2_tree_rec_bytes()));
-                rt->defer_region = !getenv("Y2_TREE_DENSE");
+                rt->defer_region = 1;
             }
             if (l->map) r->map_dev = (int *)dev_upload(l->map, 200 * sizeof(int));
         }

@@ -1,7 +1,6 @@
 #!/bin/bash
 # Developer tool (GPU box): tree-softmax parity tests + where the yolo9000 step goes (launch list of the tail).
 python -m pytest tests/test_golden_gpu.py tests/test_network_gpu.py -q -x -k "decode_nms or toy or yolo9000" 2>&1 | tail -3
-Y2_REGION_WARP_PER_GROUP=1 python -m pytest tests/test_golden_gpu.py -q -x -k "decode_nms" 2>&1 | tail -2
 timeout 200 python tools/throughput.py yolo9000 544 16 --layers 2>&1 | tail -3
 ncu --metrics gpu__time_duration.sum --clock-control none -c 60 --csv --log-file gpurun_out/y9k_launches.csv python tools/throughput.py yolo9000 544 16 1 > /dev/null 2>&1
 python - <<PY
