@@ -426,6 +426,44 @@ int network_detect_submit_frame_list(network net, int n, const unsigned char *co
 void network_detect_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
                                      const int *frame_h, float thresh, float nms, y2_detection *dets, int *counts,
                                      int max_det);
+/* ---- frames as decoders deliver them: interleaved RGB or BGR, or NV12, with a row pitch, in host memory or in memory
+ * of the network's GPU (a hardware decoder's surface, a torch or cupy tensor).  Host and device frames and the formats
+ * may be mixed in one list.  Per frame, the result is bit-identical to the frame-list entry fed with the frame
+ * converted to tight RGB bytes: BGR with its channels swapped, NV12 with OpenCV's COLOR_YUV2RGB_NV12 (BT.601 limited
+ * range, fixed point).  The conversion runs on the device, inside the resize or letterbox launch.
+ * Host frames are staged and uploaded as frame-list frames (NV12 at half the bytes of RGB) and are free when the
+ * submit returns.  Device frames are read in place: only the table of records crosses PCIe.  They must stay unchanged
+ * until the wait that returns their batch.
+ * ready: a cudaEvent_t of the network's device (or NULL); the network's stream waits for it before it reads any
+ * device frame, so a decoder or another stream can hand over frames without a host synchronise.
+ * Refused through error(), before anything is staged: what the frame-list entries refuse, a NULL descs, an unknown
+ * format, an odd NV12 size, a row of more than INT_MAX bytes, a pitch or uv_pitch smaller than the row, a device frame
+ * that is not device or managed memory of the network's GPU over all its rows inside one allocation (one cudaMalloc,
+ * or one mapped chunk of a virtual-memory allocator), and a host frame in device memory. */
+#ifndef Y2_FRAME_DESC_DEFINED
+#define Y2_FRAME_DESC_DEFINED
+enum { Y2_FRAME_RGB24 = 0, Y2_FRAME_BGR24 = 1, Y2_FRAME_NV12 = 2 };
+typedef struct y2_frame_desc {
+    const void *data;  /* RGB24/BGR24: first row of interleaved pixels; NV12: first row of the Y plane */
+    const void *uv;    /* NV12: first row of the interleaved U,V plane (NULL: data + h * pitch); else unused */
+    int w, h;          /* pixels; NV12 needs both even */
+    int pitch;         /* bytes from one row to the next; 0 = tight (3w, or w for NV12) */
+    int uv_pitch;      /* NV12: bytes between UV rows; 0 = pitch */
+    int format;        /* Y2_FRAME_* */
+    int on_device;     /* 0: host memory, staged and uploaded like a frame-list frame; 1: memory of the network's GPU,
+                        * read in place */
+} y2_frame_desc;
+#endif
+/* The slot's pinned buffer laid out for this list (only w, h, format and on_device are read): its base, and in
+ * offsets[n] each host frame's place in it ((size_t)-1 for a device frame).  A host frame whose data (and NV12 uv)
+ * already points at its place, tight, is not copied again on the host.  The buffer moves when a later call needs it
+ * larger. */
+unsigned char *network_pipeline_staging_frame_descs(network net, int slot, int n, const y2_frame_desc *descs,
+                                                    size_t *offsets);
+int network_detect_submit_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, float thresh,
+                                      float nms, int max_det);
+void network_detect_batch_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, float thresh,
+                                      float nms, y2_detection *dets, int *counts, int max_det);
 /* ---- many video streams in one batch, each frame detected on the 3-frame mean of its stream: per stream the
  * result is bit-identical to Detector::detect(img, thresh, use_mean = true) (yolo_v2_class.cpp:206-216) on that
  * stream's frames in order.  A stream is a ring of the last 3 region outputs, all zero at the start, and a
@@ -490,6 +528,18 @@ void network_detect_batch_streams_tracked(network net, int n, const int *stream_
                                           float thresh, float nms, int use_mean, y2_bbox *boxes, int *counts,
                                           int max_det);
 int network_detect_wait_tracked(network net, y2_bbox *boxes, int *counts, int max_det);
+/* The streams and tracked-streams entries fed with frame descriptors (see network_detect_submit_frame_descs); tracked
+ * boxes are scaled to each descriptor's w x h. */
+int network_detect_submit_streams_descs(network net, int n, const int *stream_ids, const y2_frame_desc *descs,
+                                        void *ready, float thresh, float nms, int max_det);
+void network_detect_batch_streams_descs(network net, int n, const int *stream_ids, const y2_frame_desc *descs,
+                                        void *ready, float thresh, float nms, y2_detection *dets, int *counts,
+                                        int max_det);
+int network_detect_submit_streams_tracked_descs(network net, int n, const int *stream_ids, const y2_frame_desc *descs,
+                                                void *ready, float thresh, float nms, int use_mean, int max_det);
+void network_detect_batch_streams_tracked_descs(network net, int n, const int *stream_ids,
+                                                const y2_frame_desc *descs, void *ready, float thresh, float nms,
+                                                int use_mean, y2_bbox *boxes, int *counts, int max_det);
 /* ---- batched, device-resident classification: letterbox, forward pass, WordTree products and top-k run on the
  * device and only `top` (index, probability) pairs per image come back, equal to what predict_classifier_image
  * computes on the host (classifier.c:676-730: letterbox_image, network_predict, hierarchy_predictions for a WordTree
@@ -528,6 +578,11 @@ int network_classify_submit_frame_list(network net, int n, const unsigned char *
                                        const int *frame_h, int top);
 void network_classify_batch_frame_list(network net, int n, const unsigned char *const *frames, const int *frame_w,
                                        const int *frame_h, int top, y2_class_hit *hits);
+/* A list of n frame descriptors (see network_detect_submit_frame_descs), each letterboxed on the device:
+ * hits [n][top]. */
+int network_classify_submit_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, int top);
+void network_classify_batch_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, int top,
+                                        y2_class_hit *hits);
 /* ---- the same over several GPUs of one box from ONE caller (one replica and one host thread per GPU; idiom of
  * train_networks, network_kernels.cu:346-376).  Replica i owns the next nets[i].batch images of the global batch;
  * detections land in the caller's arrays in image order - nothing else crosses GPUs. ------------------------- */
@@ -558,8 +613,8 @@ int network_launch_count(network net);
 int network_profile_layers(network net, float *ms_per_layer, int n);
 /* 1 -> run layers eagerly instead of replaying the captured CUDA graph */
 void network_set_eager(network net, int eager);
-/* sizeof(layer|network|network_state|y2_detection|box|y2_class_hit|y2_bbox) for what = 0..6: lets a binding that
- * passes these structs by value check its mirror against the library it loaded. */
+/* sizeof(layer|network|network_state|y2_detection|box|y2_class_hit|y2_bbox|y2_frame_desc) for what = 0..7: lets a
+ * binding that passes these structs by value check its mirror against the library it loaded. */
 size_t y2_abi_sizeof(int what);
 
 #ifdef __cplusplus

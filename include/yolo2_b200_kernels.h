@@ -222,6 +222,70 @@ size_t y2_frame_list_layout(int n, const int *frame_w, const int *frame_h, int w
 int y2_frames_u8_to_f32(const unsigned char *packed, const y2_frame_window *table, int n, float *dst, int batch,
                         int w, int h, y2_stream_t s);
 
+/* Frames as video decoders and capture libraries deliver them (the descriptor is also declared in darknet_b200.h):
+ * interleaved RGB or BGR bytes, or NV12 (a Y plane of w x h bytes, then an interleaved U,V plane of w x h/2 bytes),
+ * with a row pitch, in host memory or in memory of the network's GPU. */
+#ifndef Y2_FRAME_DESC_DEFINED
+#define Y2_FRAME_DESC_DEFINED
+enum { Y2_FRAME_RGB24 = 0, Y2_FRAME_BGR24 = 1, Y2_FRAME_NV12 = 2 };
+typedef struct y2_frame_desc {
+    const void *data;  /* RGB24/BGR24: first row of interleaved pixels; NV12: first row of the Y plane */
+    const void *uv;    /* NV12: first row of the interleaved U,V plane (NULL: data + h * pitch); else unused */
+    int w, h;          /* pixels; NV12 needs both even */
+    int pitch;         /* bytes from one row to the next; 0 = tight (3w, or w for NV12) */
+    int uv_pitch;      /* NV12: bytes between UV rows; 0 = pitch */
+    int format;        /* Y2_FRAME_* */
+    int on_device;     /* 0: host memory, staged and uploaded like a frame-list frame; 1: memory of the network's GPU,
+                        * read in place */
+} y2_frame_desc;
+#endif
+/* Where one such frame is read on the device: the y2_frame_window geometry with win.offset the absolute device
+ * address of the first row (NV12: of the Y plane), the device address of the first UV row (NV12), both pitches and
+ * the format. */
+typedef struct y2_frame_src {
+    y2_frame_window win;
+    unsigned long long uv;
+    int pitch, uv_pitch;
+    int format;
+    int reserved;
+} y2_frame_src;
+/* The rules of one descriptor, in one place: its size, format and pitches, the defaults applied.  Returns Y2_FRAME_OK
+ * and fills *rows, or the first rule it breaks: a size <= 0, an unknown format, an odd NV12 size, a row of more than
+ * INT_MAX bytes, a pitch below the row, a uv_pitch below the row (NV12).  data is not read, only added to. */
+enum {
+    Y2_FRAME_OK = 0,
+    Y2_FRAME_BAD_SIZE = 1,
+    Y2_FRAME_BAD_FORMAT = 2,
+    Y2_FRAME_BAD_NV12_SIZE = 3,
+    Y2_FRAME_BAD_ROW = 4,
+    Y2_FRAME_BAD_PITCH = 5,
+    Y2_FRAME_BAD_UV_PITCH = 6
+};
+typedef struct y2_frame_rows {
+    size_t row;               /* bytes of one row: 3w, or w for NV12 (both planes) */
+    size_t pitch;             /* bytes between rows, the default applied */
+    size_t uv_pitch;          /* NV12: bytes between UV rows, the default applied; else 0 */
+    const unsigned char *uv;  /* NV12: the first UV row, the default applied; else NULL */
+} y2_frame_rows;
+int y2_frame_desc_rows(const y2_frame_desc *d, y2_frame_rows *rows);
+/* The staged layout of a descriptor list for a w x h network: host frames in list order, each tight (3w bytes a row;
+ * NV12 the Y plane then the UV plane, w bytes a row) at a 16-byte-aligned offset, device frames taking no space, then
+ * the table of n records (at *table_offset, 16-byte aligned).  recs (may be NULL) receives the records: a host frame's
+ * win.offset and uv are offsets into the staged buffer (the caller adds the buffer's device address) with tight
+ * pitches; a device frame's are its own addresses and pitches, the defaults of y2_frame_desc applied.  letterbox as
+ * for y2_frame_list_layout.  Returns the staged size in bytes, or 0 when n < 1, descs is NULL, or a descriptor breaks
+ * a rule of y2_frame_desc_rows. */
+size_t y2_frame_desc_layout(int n, const y2_frame_desc *descs, int w, int h, int letterbox, y2_frame_src *recs,
+                            size_t *table_offset);
+/* y2_frames_u8_to_f32 over a table of frame sources (a device pointer): image i < n is converted to RGB bytes (BGR:
+ * channels swapped; NV12: BT.601 limited range in the fixed point of OpenCV's COLOR_YUV2RGB_NV12), then byte/255. +
+ * resize_image into its window, bit-identical to y2_frames_u8_to_f32 on the converted tight RGB frame; images
+ * n..batch-1 are all .5f.  Every address in the table must be readable device memory over its frame's rows. */
+int y2_frames_src_to_f32(const y2_frame_src *table, int n, float *dst, int batch, int w, int h, y2_stream_t s);
+/* The device ordinal of the device or managed allocation that holds all of [p, p + bytes), or -1 when p is host or
+ * unknown memory or the range leaves its allocation. */
+int y2_pointer_device(const void *p, size_t bytes);
+
 /* bf16 padded NHWC slice -> fp32 NCHW [B][C][H][W] (host-visible l.output layout). */
 int y2_unpack_to_nchw_f32(const void *src, float *dst, int batch, int c, int h, int w,
                           int cs, y2_stream_t s);

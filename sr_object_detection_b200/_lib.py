@@ -54,6 +54,35 @@ def frame_list_layout(sizes, w: int, h: int, letterbox: bool):
     return list(win)[:n], toff.value, total
 
 
+class FrameDesc(C.Structure):
+    """Mirror of `y2_frame_desc`: a frame as a decoder delivers it (darknet.frame_desc builds one from an array)."""
+    _fields_ = [("data", C.c_void_p), ("uv", C.c_void_p), ("w", C.c_int), ("h", C.c_int), ("pitch", C.c_int),
+                ("uv_pitch", C.c_int), ("format", C.c_int), ("on_device", C.c_int)]
+
+
+class FrameSrc(C.Structure):
+    """Mirror of `y2_frame_src`: where the conversion kernel reads one frame, and the window it fills."""
+    _fields_ = [("win", FrameWindow), ("uv", C.c_ulonglong), ("pitch", C.c_int), ("uv_pitch", C.c_int),
+                ("format", C.c_int), ("reserved", C.c_int)]
+
+
+class FrameRows(C.Structure):
+    """Mirror of `y2_frame_rows`: a descriptor's row bytes, pitches and UV address with the defaults applied."""
+    _fields_ = [("row", C.c_size_t), ("pitch", C.c_size_t), ("uv_pitch", C.c_size_t), ("uv", C.c_void_p)]
+
+
+def frame_desc_layout(descs, w: int, h: int, letterbox: bool):
+    """y2_frame_desc_layout for a list of FrameDesc on a w x h network: (records, table offset, staged size in
+    bytes)."""
+    lib = load()
+    n = len(descs)
+    arr = (FrameDesc * max(n, 1))(*descs)
+    recs = (FrameSrc * max(n, 1))()
+    toff = C.c_size_t()
+    total = lib.y2_frame_desc_layout(n, arr, w, h, int(letterbox), recs, C.byref(toff))
+    return list(recs)[:n], toff.value, total
+
+
 class StreamSrc(C.Structure):
     """Mirror of `y2_stream_src`: where the 3 ring slots of an image's stream come from, and the ring row it commits."""
     _fields_ = [("src", C.c_int * 3), ("commit", C.c_int)]
@@ -165,6 +194,11 @@ def _declare(lib: C.CDLL) -> None:
         "y2_frame_list_layout": (C.c_size_t, [i, C.POINTER(i), C.POINTER(i), i, i, i, C.POINTER(FrameWindow),
                                               C.POINTER(C.c_size_t)]),
         "y2_frames_u8_to_f32": (i, [vp, vp, i, vp, i, i, i, vp]),
+        "y2_frame_desc_layout": (C.c_size_t, [i, C.POINTER(FrameDesc), i, i, i, C.POINTER(FrameSrc),
+                                              C.POINTER(C.c_size_t)]),
+        "y2_frame_desc_rows": (i, [C.POINTER(FrameDesc), C.POINTER(FrameRows)]),
+        "y2_frames_src_to_f32": (i, [vp, i, vp, i, i, i, vp]),
+        "y2_pointer_device": (i, [vp, C.c_size_t]),
         "y2_stream_plan": (i, [i, C.POINTER(i), i, C.POINTER(i), C.POINTER(i), C.POINTER(StreamSrc)]),
         "y2_stream_mean": (i, [vp, vp, vp, i, i, vp, vp]),
         "y2_stream_commit": (i, [vp, vp, vp, i, i, vp]),

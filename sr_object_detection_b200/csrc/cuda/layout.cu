@@ -5,6 +5,7 @@
 #include "y2_common.cuh"
 
 #include <float.h>
+#include <limits.h>
 
 namespace y2 {
 
@@ -275,38 +276,23 @@ __global__ void gather_patches_bf16_kernel(const __nv_bfloat16 *__restrict__ in,
 // Quirk kept: the last target row takes only the (1-dy) term (image.c:1985 `continue`).
 // ---------------------------------------------------------------------------------
 
-// The resized image fills the window [dx, dx+nw) x [dy, dy+nh) of the w x h canvas and the rest is .5f: the whole
-// canvas for resize_image, the centred window of letterbox_image (image.c:1624-1644: fill_image(.5) + embed_image).
-// Image b = blockIdx.y reads its record once: table[b], or for a uniform batch (table == NULL) the by-value record
-// with the frame at uni.offset + b * stride.  One thread per output pixel writes all three planes from the same
-// 3-byte taps.  Images b >= n are the .5f canvas.
-__global__ void frames_u8_to_f32_kernel(const unsigned char *__restrict__ packed,
-                                        const y2_frame_window *__restrict__ table, y2_frame_window uni,
-                                        unsigned long long stride, int n, float *__restrict__ dst, int w, int h)
+// One source pixel's three bytes, R G B, already loaded (the tap of a converted format).
+struct px3 {
+    unsigned char v[3];
+    __device__ __forceinline__ unsigned char operator[](int k) const { return v[k]; }
+};
+
+// resize_image's taps for canvas pixel (c, r) inside window f, all three planes from the same taps: out[k * hw] =
+// plane k.  src.row(y) gives source row y and src.at(row, x) the tap of its pixel x, whose tap[k] is byte k (R G B);
+// an interleaved tap is a pointer, so its bytes are loaded channel by channel next to the arithmetic that uses them.
+// All four taps are formed, also where the edge column or the last row does not use them: every tap has
+// 0 <= x <= src_w - 1 and 0 <= y <= src_h - 1 (ix is below src_w - 1 off the edge column, ix1, iy and iy1 are
+// clamped), so it stays inside its frame's rows.  Shared by every frame kernel, so they agree bit for bit.
+template <class Src>
+__device__ __forceinline__ void resize_taps(const y2_frame_window &f, int c, int r, const float *lut, const Src &src,
+                                            float *out, int hw)
 {
-    __shared__ float lut[256];
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = (float)((double)(float)i / 255.);
-    __syncthreads();
-    const int b = blockIdx.y;
-    const int hw = w * h;
-    const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= hw) return;
-    float *out = dst + (size_t)b * 3 * hw + p;
-    const int y = p / w;
-    y2_frame_window f = uni;
-    if (b < n) {
-        if (table) f = table[b];
-        else f.offset += (unsigned long long)b * stride;
-    }
-    const int c = p - y * w - f.dx, r = y - f.dy;
-    if (b >= n || c < 0 || c >= f.new_w || r < 0 || r >= f.new_h) {
-        out[0] = .5f;
-        out[hw] = .5f;
-        out[2 * hw] = .5f;
-        return;
-    }
     const int sw = f.src_w, sh = f.src_h;
-    const unsigned char *img = packed + f.offset;
     // horizontal taps of resize_part: the edge column, or ix / ix1 with weight dx
     const bool edge = c == f.new_w - 1 || sw == 1;
     int ix = sw - 1, ix1 = sw - 1;
@@ -325,8 +311,8 @@ __global__ void frames_u8_to_f32_kernel(const unsigned char *__restrict__ packed
     const bool two_rows = !(r == f.new_h - 1 || sh == 1); // image.c:1985: the last row takes the (1-dy) term only
     int iy1 = iy + 1;
     if (iy1 > sh - 1) iy1 = sh - 1;
-    const unsigned char *r0 = img + (size_t)iy * sw * 3, *r1 = img + (size_t)iy1 * sw * 3;
-    const unsigned char *a0 = r0 + ix * 3, *b0 = r0 + ix1 * 3, *a1 = r1 + ix * 3, *b1 = r1 + ix1 * 3;
+    const auto r0 = src.row(iy), r1 = src.row(iy1);
+    const auto a0 = src.at(r0, ix), b0 = src.at(r0, ix1), a1 = src.at(r1, ix), b1 = src.at(r1, ix1);
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
         float part0 = lut[a0[k]];
@@ -339,6 +325,137 @@ __global__ void frames_u8_to_f32_kernel(const unsigned char *__restrict__ packed
         }
         out[(size_t)k * hw] = val;
     }
+}
+
+// Interleaved 3-byte pixels, rows `pitch` bytes apart; SWAP: stored B G R.  A tap is the pixel's address.
+template <bool SWAP>
+struct Interleaved {
+    const unsigned char *data;
+    size_t pitch;
+    struct Tap {
+        const unsigned char *q;
+        __device__ __forceinline__ unsigned char operator[](int k) const { return q[SWAP ? 2 - k : k]; }
+    };
+    __device__ __forceinline__ const unsigned char *row(int y) const { return data + (size_t)y * pitch; }
+    __device__ __forceinline__ Tap at(const unsigned char *row, int x) const { return Tap{row + x * 3}; }
+};
+
+// A packed frame-list frame: tight RGB rows of 3 * sw bytes, each row's address computed as (size_t)y * sw * 3.
+struct PackedRGB {
+    const unsigned char *data;
+    int sw;
+    __device__ __forceinline__ const unsigned char *row(int y) const { return data + (size_t)y * sw * 3; }
+    __device__ __forceinline__ Interleaved<false>::Tap at(const unsigned char *row, int x) const
+    {
+        return Interleaved<false>::Tap{row + x * 3};
+    }
+};
+
+// The (float)(byte / 255.) table of load_image_stb, in shared memory.
+__device__ __forceinline__ void fill_lut(float *lut)
+{
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = (float)((double)(float)i / 255.);
+    __syncthreads();
+}
+
+// The resized image fills the window [dx, dx+nw) x [dy, dy+nh) of the w x h canvas and the rest is .5f: the whole
+// canvas for resize_image, the centred window of letterbox_image (image.c:1624-1644: fill_image(.5) + embed_image).
+// Image b = blockIdx.y reads its record once: table[b], or for a uniform batch (table == NULL) the by-value record
+// with the frame at uni.offset + b * stride.  One thread per output pixel writes all three planes from the same
+// 3-byte taps.  Images b >= n are the .5f canvas.
+__global__ void frames_u8_to_f32_kernel(const unsigned char *__restrict__ packed,
+                                        const y2_frame_window *__restrict__ table, y2_frame_window uni,
+                                        unsigned long long stride, int n, float *__restrict__ dst, int w, int h)
+{
+    __shared__ float lut[256];
+    fill_lut(lut);
+    const int b = blockIdx.y;
+    const int hw = w * h;
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= hw) return;
+    float *out = dst + (size_t)b * 3 * hw + p;
+    const int y = p / w;
+    y2_frame_window f = uni;
+    if (b < n) {
+        if (table) f = table[b];
+        else f.offset += (unsigned long long)b * stride;
+    }
+    const int c = p - y * w - f.dx, r = y - f.dy;
+    if (b >= n || c < 0 || c >= f.new_w || r < 0 || r >= f.new_h) {
+        out[0] = .5f;
+        out[hw] = .5f;
+        out[2 * hw] = .5f;
+        return;
+    }
+    resize_taps(f, c, r, lut, PackedRGB{packed + f.offset, f.src_w}, out, hw);
+}
+
+// NV12 -> RGB as OpenCV's cvtColor(COLOR_YUV2RGB_NV12): BT.601 limited range in 20-bit fixed point.  Exact in int32:
+// every intermediate stays within +-6e8.
+__device__ __forceinline__ px3 nv12_rgb(int Y, int U, int V)
+{
+    const int y = max(Y - 16, 0) * 1220542, half = 1 << 19, u = U - 128, v = V - 128;
+    const int r = (y + half + 1673527 * v) >> 20;
+    const int g = (y + half - 852492 * v - 409993 * u) >> 20;
+    const int bl = (y + half + 2116026 * u) >> 20;
+    return px3{{(unsigned char)min(max(r, 0), 255), (unsigned char)min(max(g, 0), 255),
+                (unsigned char)min(max(bl, 0), 255)}};
+}
+
+// NV12: a Y plane and an interleaved U,V plane at half the rows; pixel x of row y takes the pair at (x & ~1) of UV
+// row y >> 1.
+struct Nv12 {
+    const unsigned char *y, *uv;
+    size_t pitch, uv_pitch;
+    struct Row {
+        const unsigned char *y, *uv;
+    };
+    __device__ __forceinline__ Row row(int yy) const
+    {
+        return Row{y + (size_t)yy * pitch, uv + (size_t)(yy >> 1) * uv_pitch};
+    }
+    __device__ __forceinline__ px3 at(const Row &r, int x) const
+    {
+        const unsigned char *q = r.uv + (x & ~1);
+        return nv12_rgb(r.y[x], q[0], q[1]);
+    }
+};
+
+// frames_u8_to_f32_kernel over frame sources: each record names its frame's device address, pitch and format, and
+// the format is uniform per block (one image per blockIdx.y), so the switch does not diverge.  Bounds: a fetch has
+// 0 <= x <= src_w - 1 and 0 <= y <= src_h - 1 (resize_taps), so an RGB/BGR fetch reads inside
+// [data, data + (src_h-1)*pitch + 3*src_w) and an NV12 fetch inside [data, data + (src_h-1)*pitch + src_w) and, with
+// src_w and src_h even, (y>>1) <= src_h/2 - 1 and (x&~1) + 1 <= src_w - 1, inside
+// [uv, uv + (src_h/2-1)*uv_pitch + src_w).  The host checks those ranges before it launches.
+__global__ void frames_src_to_f32_kernel(const y2_frame_src *__restrict__ table, int n, float *__restrict__ dst, int w,
+                                         int h)
+{
+    __shared__ float lut[256];
+    fill_lut(lut);
+    const int b = blockIdx.y;
+    const int hw = w * h;
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= hw) return;
+    float *out = dst + (size_t)b * 3 * hw + p;
+    const int y = p / w;
+    y2_frame_src s = {};
+    if (b < n) s = table[b];
+    const y2_frame_window &f = s.win;
+    const int c = p - y * w - f.dx, r = y - f.dy;
+    if (b >= n || c < 0 || c >= f.new_w || r < 0 || r >= f.new_h) {
+        out[0] = .5f;
+        out[hw] = .5f;
+        out[2 * hw] = .5f;
+        return;
+    }
+    const unsigned char *img = (const unsigned char *)f.offset;
+    const size_t pitch = (size_t)s.pitch;
+    if (s.format == Y2_FRAME_NV12)
+        resize_taps(f, c, r, lut, Nv12{img, (const unsigned char *)s.uv, pitch, (size_t)s.uv_pitch}, out, hw);
+    else if (s.format == Y2_FRAME_BGR24)
+        resize_taps(f, c, r, lut, Interleaved<true>{img, pitch}, out, hw);
+    else
+        resize_taps(f, c, r, lut, Interleaved<false>{img, pitch}, out, hw);
 }
 
 // ---------------------------------------------------------------------------------
@@ -1027,6 +1144,74 @@ extern "C" int y2_frames_u8_to_f32(const unsigned char *packed, const y2_frame_w
     }
     const y2_frame_window none = {};
     return launch_frames(packed, table, none, 0, n, dst, batch, w, h, s);
+}
+
+extern "C" int y2_frame_desc_rows(const y2_frame_desc *d, y2_frame_rows *rows)
+{
+    if (d->w <= 0 || d->h <= 0) return Y2_FRAME_BAD_SIZE;
+    if (d->format != Y2_FRAME_RGB24 && d->format != Y2_FRAME_BGR24 && d->format != Y2_FRAME_NV12)
+        return Y2_FRAME_BAD_FORMAT;
+    const bool nv12 = d->format == Y2_FRAME_NV12;
+    if (nv12 && (d->w % 2 || d->h % 2)) return Y2_FRAME_BAD_NV12_SIZE;
+    const size_t row = (size_t)d->w * (nv12 ? 1 : 3);
+    if (row > (size_t)INT_MAX) return Y2_FRAME_BAD_ROW; // the record and the kernel's byte offsets are int
+    const size_t pitch = d->pitch ? (size_t)d->pitch : row;
+    if (d->pitch < 0 || pitch < row) return Y2_FRAME_BAD_PITCH;
+    const size_t uv_pitch = d->uv_pitch ? (size_t)d->uv_pitch : pitch;
+    if (nv12 && (d->uv_pitch < 0 || uv_pitch < row)) return Y2_FRAME_BAD_UV_PITCH;
+    rows->row = row;
+    rows->pitch = pitch;
+    rows->uv_pitch = nv12 ? uv_pitch : 0;
+    rows->uv = !nv12 ? nullptr
+                     : d->uv ? (const unsigned char *)d->uv : (const unsigned char *)d->data + (size_t)d->h * pitch;
+    return Y2_FRAME_OK;
+}
+
+extern "C" size_t y2_frame_desc_layout(int n, const y2_frame_desc *descs, int w, int h, int letterbox,
+                                       y2_frame_src *recs, size_t *table_offset)
+{
+    if (n < 1 || !descs || w <= 0 || h <= 0) return 0;
+    size_t off = 0;
+    for (int i = 0; i < n; ++i) {
+        const y2_frame_desc &d = descs[i];
+        y2_frame_rows fr;
+        if (y2_frame_desc_rows(&d, &fr) != Y2_FRAME_OK) return 0;
+        const bool nv12 = d.format == Y2_FRAME_NV12;
+        y2_frame_src r = {};
+        r.win = frame_window(d.w, d.h, w, h, letterbox);
+        r.format = d.format;
+        if (d.on_device) {
+            r.win.offset = (unsigned long long)(uintptr_t)d.data;
+            r.uv = (unsigned long long)(uintptr_t)fr.uv;
+            r.pitch = (int)fr.pitch;
+            r.uv_pitch = (int)fr.uv_pitch;
+        } else { // staged tight: NV12 as the Y plane then the UV plane
+            const size_t plane = fr.row * d.h;
+            r.win.offset = off;
+            r.uv = nv12 ? off + plane : 0;
+            r.pitch = (int)fr.row;
+            r.uv_pitch = nv12 ? (int)fr.row : 0;
+            off += (plane + (nv12 ? plane / 2 : 0) + 15) & ~(size_t)15;
+        }
+        if (recs) recs[i] = r;
+    }
+    if (table_offset) *table_offset = off;
+    return off + (size_t)n * sizeof(y2_frame_src);
+}
+
+extern "C" int y2_frames_src_to_f32(const y2_frame_src *table, int n, float *dst, int batch, int w, int h,
+                                    y2_stream_t s)
+{
+    const long long hw = (long long)w * h;
+    if (!table || !dst || n < 1 || n > batch || w <= 0 || h <= 0 || batch > 65535 ||
+        hw > 0x7fffffffLL - FRAMES_THREADS) {
+        set_error("y2_frames_src_to_f32: invalid arguments (n=%d batch=%d %dx%d)", n, batch, w, h);
+        return Y2_EINVAL;
+    }
+    const dim3 grid((unsigned)((hw + FRAMES_THREADS - 1) / FRAMES_THREADS), (unsigned)batch);
+    frames_src_to_f32_kernel<<<grid, FRAMES_THREADS, 0, to_stream(s)>>>(table, n, dst, w, h);
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
 }
 
 // a uniform batch: one record passed by value, frame b at b * src_h * src_w * 3

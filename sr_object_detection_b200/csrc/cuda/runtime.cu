@@ -113,6 +113,37 @@ extern "C" int y2_malloc(void **dptr, size_t bytes)
     Y2_CUDA_CHECK(cudaMalloc(dptr, bytes ? bytes : 16));
     return Y2_OK;
 }
+// cudaPointerGetAttributes tells device, managed and host memory apart; the driver's cuMemGetAddressRange gives the
+// allocation around the address, so a range that runs past its allocation is refused too.
+extern "C" int y2_pointer_device(const void *p, size_t bytes)
+{
+    typedef int (*AddressRangeFn)(unsigned long long *base, size_t *size, unsigned long long ptr);
+    static AddressRangeFn range_fn = nullptr;
+    if (!p || !bytes) return -1;
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        return -1;
+    }
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return -1;
+    if (!range_fn) {
+        void *fn = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &fn, cudaEnableDefault, &q) != cudaSuccess ||
+            q != cudaDriverEntryPointSuccess || !fn) {
+            cudaGetLastError();
+            return -1;
+        }
+        range_fn = (AddressRangeFn)fn;
+    }
+    unsigned long long base = 0;
+    size_t size = 0;
+    const unsigned long long at = (unsigned long long)(uintptr_t)p;
+    if (range_fn(&base, &size, at) != 0) return -1;
+    if (at < base || bytes > size - (at - base)) return -1;
+    return a.device;
+}
+
 extern "C" int y2_free(void *dptr)
 {
     if (dptr) Y2_CUDA_CHECK(cudaFree(dptr));

@@ -592,6 +592,76 @@ void network_detect_batch_streams_tracked(network net, int n, const int *stream_
                  max_det);
 }
 
+/* ---- frame descriptors: the entries above fed with RGB, BGR or NV12 frames in host or device memory ------------ */
+static y2_input descs_input(int n, const y2_frame_desc *descs, void *ready)
+{
+    return (y2_input){.kind = Y2_IN_FRAME_DESCS, .descs = {n, descs, ready}};
+}
+
+int network_detect_submit_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, float thresh,
+                                      float nms, int max_det)
+{
+    return detect_submit(net, descs_input(n, descs, ready), NULL, thresh, nms, max_det);
+}
+
+void network_detect_batch_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, float thresh,
+                                      float nms, y2_detection *dets, int *counts, int max_det)
+{
+    detect_batch(net, "network_detect_batch_frame_descs: batches of the submit/wait pipeline are in flight",
+                 descs_input(n, descs, ready), NULL, thresh, nms, dets, NULL, counts, max_det);
+}
+
+int network_detect_submit_streams_descs(network net, int n, const int *stream_ids, const y2_frame_desc *descs,
+                                        void *ready, float thresh, float nms, int max_det)
+{
+    return detect_submit(net, descs_input(n, descs, ready), &(stream_list){n, stream_ids, 0, 1}, thresh, nms,
+                         max_det);
+}
+
+void network_detect_batch_streams_descs(network net, int n, const int *stream_ids, const y2_frame_desc *descs,
+                                        void *ready, float thresh, float nms, y2_detection *dets, int *counts,
+                                        int max_det)
+{
+    detect_batch(net, "network_detect_batch_streams_descs: batches of the submit/wait pipeline are in flight",
+                 descs_input(n, descs, ready), &(stream_list){n, stream_ids, 0, 1}, thresh, nms, dets, NULL, counts,
+                 max_det);
+}
+
+/* the frame widths then heights of a descriptor list, for the tracking plan (NULL for a list the pipeline refuses) */
+static int *desc_sizes(network net, int n, const y2_frame_desc *descs)
+{
+    if (!descs || n < 1 || n > net.batch) return NULL;
+    int *wh = (int *)malloc((size_t)2 * n * sizeof(int));
+    if (!wh) error("network streams tracked: out of host memory");
+    for (int i = 0; i < n; ++i) {
+        wh[i] = descs[i].w;
+        wh[n + i] = descs[i].h;
+    }
+    return wh;
+}
+
+int network_detect_submit_streams_tracked_descs(network net, int n, const int *stream_ids, const y2_frame_desc *descs,
+                                                void *ready, float thresh, float nms, int use_mean, int max_det)
+{
+    int *wh = desc_sizes(net, n, descs);
+    const int s = detect_submit(net, descs_input(n, descs, ready),
+                                &(stream_list){n, stream_ids, 1, use_mean, wh, wh ? wh + n : NULL}, thresh, nms,
+                                max_det);
+    free(wh);
+    return s;
+}
+
+void network_detect_batch_streams_tracked_descs(network net, int n, const int *stream_ids,
+                                                const y2_frame_desc *descs, void *ready, float thresh, float nms,
+                                                int use_mean, y2_bbox *boxes, int *counts, int max_det)
+{
+    int *wh = desc_sizes(net, n, descs);
+    detect_batch(net, "network_detect_batch_streams_tracked_descs: batches of the submit/wait pipeline are in flight",
+                 descs_input(n, descs, ready), &(stream_list){n, stream_ids, 1, use_mean, wh, wh ? wh + n : NULL},
+                 thresh, nms, NULL, boxes, counts, max_det);
+    free(wh);
+}
+
 /* ---- batched, device-resident classification (extension) --------------------------------------- */
 /* the output layer the classify entries read, after the checks every entry makes */
 static layer *classify_layer(network net, int top)
@@ -714,4 +784,16 @@ void network_classify_batch_frame_list(network net, int n, const unsigned char *
     const y2_input in = {.kind = Y2_IN_FRAME_LIST, .list = {n, frames, frame_w, frame_h}};
     classify_batch(net, "network_classify_batch_frame_list: batches of the submit/wait pipeline are in flight", in,
                    top, hits);
+}
+
+int network_classify_submit_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, int top)
+{
+    return classify_submit(net, descs_input(n, descs, ready), top);
+}
+
+void network_classify_batch_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, int top,
+                                        y2_class_hit *hits)
+{
+    classify_batch(net, "network_classify_batch_frame_descs: batches of the submit/wait pipeline are in flight",
+                   descs_input(n, descs, ready), top, hits);
 }

@@ -115,6 +115,7 @@ typedef enum {
     Y2_IN_U8,         /* uint8 interleaved RGB [B][h][w][3] at the network's resolution */
     Y2_IN_FRAMES,     /* uint8 interleaved RGB frames [B][fh][fw][3] of any size */
     Y2_IN_FRAME_LIST, /* 1 .. B frames of their own sizes */
+    Y2_IN_FRAME_DESCS, /* 1 .. B frame descriptors: RGB, BGR or NV12 with a pitch, in host or device memory */
     Y2_IN_RESIDENT,   /* nothing: the slot's device input already holds the batch */
 } y2_input_kind;
 
@@ -127,6 +128,11 @@ typedef struct {
         const unsigned char *const *frames;
         const int *w, *h;
     } list;
+    struct y2_frame_descs {    /* Y2_IN_FRAME_DESCS */
+        int n;
+        const y2_frame_desc *d;
+        void *ready;           /* cudaEvent_t the compute stream waits for before it reads device frames, or NULL */
+    } descs;
     int n;                     /* images the batch hands back: the list's length, else the batch */
 } y2_input;
 

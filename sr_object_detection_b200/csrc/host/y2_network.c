@@ -1536,6 +1536,7 @@ size_t y2_abi_sizeof(int what)
     case 4: return sizeof(box);
     case 5: return sizeof(y2_class_hit);
     case 6: return sizeof(y2_bbox);
+    case 7: return sizeof(y2_frame_desc);
     default: return 0;
     }
 }

@@ -1,8 +1,9 @@
 /*
  * The two-deep submit/wait pipeline: the H2D copy of batch i+1 overlaps the forward pass of batch i, and the results
  * of batch i return under the forward pass of batch i+1.  This file owns the slots (creating them, growing their
- * buffers, releasing them on a re-plan, freeing them), the staging getters, the input half of a submission, and
- * claiming and retiring a slot.  The detection and classify tails and their entry points are in y2_detect.c.
+ * buffers, releasing them on a re-plan, freeing them), the staging getters, the frame-list and frame-descriptor
+ * checks and staging, the input half of a submission, and claiming and retiring a slot.  The detection and classify
+ * tails and their entry points are in y2_detect.c.
  */
 #include "y2_host.h"
 
@@ -202,18 +203,64 @@ static void check_frame_list(network net, const struct y2_frame_list *fl)
     }
 }
 
+/* the bytes a frame's rows span from its first row: (h - 1) pitches and one row */
+static size_t span(int rows, size_t pitch, size_t row) { return (size_t)(rows - 1) * pitch + row; }
+
+/* The refusals of every descriptor entry, before anything is staged: the frame list's, then each descriptor's
+ * (y2_frame_desc_rows: size, format and pitches), then where its memory is.  A device frame must be memory of the
+ * network's GPU over every row the conversion kernel can read, within one allocation; a host frame must not be
+ * device memory. */
+static void check_frame_descs(network net, const struct y2_frame_descs *fd)
+{
+    static const char *const broken[] = {
+        [Y2_FRAME_BAD_SIZE] = "network frame list: a frame size of 0 or less",
+        [Y2_FRAME_BAD_FORMAT] = "network frame descs: unknown format (Y2_FRAME_RGB24, Y2_FRAME_BGR24 or Y2_FRAME_NV12)",
+        [Y2_FRAME_BAD_NV12_SIZE] = "network frame descs: an NV12 frame needs an even width and height",
+        [Y2_FRAME_BAD_ROW] = "network frame descs: a row of more than INT_MAX bytes",
+        [Y2_FRAME_BAD_PITCH] = "network frame descs: a pitch smaller than the row's bytes",
+        [Y2_FRAME_BAD_UV_PITCH] = "network frame descs: a uv_pitch smaller than the row's bytes"};
+    if (!y2_rt(net)) error("network frame list: network has no device plan");
+    if (net.c != 3) error("network frame list: needs a network with 3 input channels");
+    if (fd->n < 1 || fd->n > net.batch) error("network frame list: the list must hold 1 .. batch frames");
+    if (!fd->d) error("network frame descs: NULL descriptor array");
+    for (int i = 0; i < fd->n; ++i) {
+        y2_frame_rows fr;
+        if (!fd->d[i].data) error("network frame list: NULL frame pointer");
+        const int rc = y2_frame_desc_rows(&fd->d[i], &fr);
+        if (rc != Y2_FRAME_OK) error(broken[rc]);
+    }
+    y2_net_rt *rt = y2_rt(net);
+    Y2_CHECK(y2_set_device(rt->device));
+    for (int i = 0; i < fd->n; ++i) {
+        const y2_frame_desc *d = &fd->d[i];
+        const int nv12 = d->format == Y2_FRAME_NV12;
+        y2_frame_rows fr;
+        y2_frame_desc_rows(d, &fr);
+        if (d->on_device) {
+            if (y2_pointer_device(d->data, span(d->h, fr.pitch, fr.row)) != rt->device ||
+                (nv12 && y2_pointer_device(fr.uv, span(d->h / 2, fr.uv_pitch, fr.row)) != rt->device))
+                error("network frame descs: a device frame that is not device or managed memory of the network's GPU "
+                      "over all its rows, or whose rows leave their allocation (one cudaMalloc, or one mapped chunk of "
+                      "a virtual-memory allocator)");
+        } else if (y2_pointer_device(d->data, 1) >= 0 || (nv12 && d->uv && y2_pointer_device(d->uv, 1) >= 0)) {
+            error("network frame descs: a host frame (on_device 0) in device memory");
+        }
+    }
+}
+
 /* The one place an input is decided: frames at the network's resolution become uint8 input when the network has the
  * first-layer kernel for it; each kind's refusals and lazy set-up; in.n. */
 static y2_input pipe_input(network net, y2_input in)
 {
     if (in.kind == Y2_IN_FRAME_LIST) check_frame_list(net, &in.list);
+    if (in.kind == Y2_IN_FRAME_DESCS) check_frame_descs(net, &in.descs);
     if (!y2_rt(net)) error("network submit: network has no device plan");
     if (in.kind == Y2_IN_FRAMES && in.fw == net.w && in.fh == net.h && takes_u8(net)) in.kind = Y2_IN_U8;
     pipe_init(y2_rt(net));
     if (in.kind == Y2_IN_U8) pipe_init_u8(net);
     if (in.kind == Y2_IN_FRAMES && (net.c != 3 || in.fw <= 0 || in.fh <= 0))
         error("network submit of frames: needs 3-channel input and a frame size");
-    in.n = in.kind == Y2_IN_FRAME_LIST ? in.list.n : net.batch;
+    in.n = in.kind == Y2_IN_FRAME_LIST ? in.list.n : in.kind == Y2_IN_FRAME_DESCS ? in.descs.n : net.batch;
     return in;
 }
 
@@ -273,6 +320,27 @@ unsigned char *network_pipeline_staging_frame_list(network net, int slot, int n,
     return rt->pipe[slot].frames_pinned;
 }
 
+unsigned char *network_pipeline_staging_frame_descs(network net, int slot, int n, const y2_frame_desc *descs,
+                                                    size_t *offsets)
+{
+    if (!y2_rt(net)) error("network_pipeline_staging_frame_descs: network has no device plan");
+    y2_net_rt *rt = staging_rt(net, slot, n >= 1 && n <= net.batch && descs && offsets,
+                               "network_pipeline_staging_frame_descs: bad slot, descs or offsets, or a list not of "
+                               "1 .. batch frames");
+    const size_t bytes = y2_frame_desc_layout(n, descs, net.w, net.h, 0, NULL, NULL);
+    if (!bytes)
+        error("network_pipeline_staging_frame_descs: a frame size of 0 or less, an unknown format, an odd NV12 size "
+              "or a pitch smaller than the row");
+    Y2_CHECK(y2_set_device(rt->device));
+    pipe_reserve_frames(rt, slot, bytes, NULL);
+    y2_frame_src *rec = (y2_frame_src *)calloc((size_t)n, sizeof(y2_frame_src));
+    if (!rec) error("network_pipeline_staging_frame_descs: out of host memory");
+    y2_frame_desc_layout(n, descs, net.w, net.h, 0, rec, NULL);
+    for (int i = 0; i < n; ++i) offsets[i] = descs[i].on_device ? (size_t)-1 : (size_t)rec[i].win.offset;
+    free(rec);
+    return rt->pipe[slot].frames_pinned;
+}
+
 int network_pipeline_next_slot(network net)
 {
     y2_net_rt *rt = y2_rt(net);
@@ -297,6 +365,46 @@ static size_t stage_frame_list(network net, int s, const struct y2_frame_list *f
     for (int i = 0; i < fl->n; ++i) {
         unsigned char *dst = ps->frames_pinned + win[i].offset;
         if (fl->frames[i] != dst) memcpy(dst, fl->frames[i], (size_t)fl->w[i] * fl->h[i] * 3);
+    }
+    Y2_CHECK(y2_host_free(old));
+    Y2_CHECK(y2_memcpy_h2d(ps->frames_dev, ps->frames_pinned, bytes, rt->copy_stream));
+    return table_off;
+}
+
+/* rows of `row` bytes, `pitch` apart at src, tight at dst; nothing when they are already there */
+static void copy_rows(unsigned char *dst, const unsigned char *src, int rows, size_t row, size_t pitch)
+{
+    if (src == dst && pitch == row) return;
+    if (pitch == row) {
+        memcpy(dst, src, (size_t)rows * row);
+        return;
+    }
+    for (int y = 0; y < rows; ++y) memcpy(dst + (size_t)y * row, src + (size_t)y * pitch, row);
+}
+
+/* A descriptor list into slot s: the host frames (tight) and the record table behind them in the slot's pinned buffer,
+ * each host record pointed at the frame's place in the device buffer, then one H2D copy of the whole region on the
+ * copy stream (the table alone when every frame is on the device).  Returns the table's offset in the region. */
+static size_t stage_frame_descs(network net, int s, const struct y2_frame_descs *fd, int letterbox)
+{
+    y2_net_rt *rt = y2_rt(net);
+    struct y2_pipe_slot *ps = &rt->pipe[s];
+    size_t table_off = 0;
+    const size_t bytes = y2_frame_desc_layout(fd->n, fd->d, net.w, net.h, letterbox, NULL, &table_off);
+    unsigned char *old = NULL;
+    pipe_reserve_frames(rt, s, bytes, &old);
+    y2_frame_src *rec = (y2_frame_src *)(ps->frames_pinned + table_off);
+    y2_frame_desc_layout(fd->n, fd->d, net.w, net.h, letterbox, rec, NULL);
+    for (int i = 0; i < fd->n; ++i) {
+        const y2_frame_desc *d = &fd->d[i];
+        if (d->on_device) continue;
+        y2_frame_rows fr;
+        y2_frame_desc_rows(d, &fr);
+        copy_rows(ps->frames_pinned + rec[i].win.offset, (const unsigned char *)d->data, d->h, fr.row, fr.pitch);
+        if (d->format == Y2_FRAME_NV12)
+            copy_rows(ps->frames_pinned + rec[i].uv, fr.uv, d->h / 2, fr.row, fr.uv_pitch);
+        rec[i].win.offset += (unsigned long long)(uintptr_t)ps->frames_dev;
+        if (d->format == Y2_FRAME_NV12) rec[i].uv += (unsigned long long)(uintptr_t)ps->frames_dev;
     }
     Y2_CHECK(y2_host_free(old));
     Y2_CHECK(y2_memcpy_h2d(ps->frames_dev, ps->frames_pinned, bytes, rt->copy_stream));
@@ -333,6 +441,8 @@ void y2_pipe_submit_input(network net, int s, const y2_input *in, int letterbox)
     size_t table_off = 0;
     if (in->kind == Y2_IN_FRAME_LIST) {
         table_off = stage_frame_list(net, s, &in->list, letterbox);
+    } else if (in->kind == Y2_IN_FRAME_DESCS) {
+        table_off = stage_frame_descs(net, s, &in->descs, letterbox);
     } else if (in->kind == Y2_IN_FRAMES) {
         const size_t bytes = (size_t)B * in->fh * in->fw * 3;
         pipe_reserve_frames(rt, s, bytes, NULL);
@@ -346,9 +456,14 @@ void y2_pipe_submit_input(network net, int s, const y2_input *in, int letterbox)
         Y2_CHECK(y2_event_record(ps->ev_h2d, rt->copy_stream));
         Y2_CHECK(y2_stream_wait_event(rt->stream, ps->ev_h2d));
     }
+    if (in->kind == Y2_IN_FRAME_DESCS && in->descs.ready) /* the producer of the device frames */
+        Y2_CHECK(y2_stream_wait_event(rt->stream, in->descs.ready));
     if (in->kind == Y2_IN_FRAME_LIST) /* byte/255. + resize_image or letterbox_image per frame, .5f behind the list */
         Y2_CHECK(y2_frames_u8_to_f32(ps->frames_dev, (const y2_frame_window *)(ps->frames_dev + table_off), in->n,
                                      ps->in_dev, B, net.w, net.h, rt->stream));
+    else if (in->kind == Y2_IN_FRAME_DESCS) /* to RGB, then as the frame list */
+        Y2_CHECK(y2_frames_src_to_f32((const y2_frame_src *)(ps->frames_dev + table_off), in->n, ps->in_dev, B, net.w,
+                                      net.h, rt->stream));
     else if (in->kind == Y2_IN_FRAMES && letterbox) /* byte/255. + letterbox_image, into the slot's fp32 input */
         Y2_CHECK(y2_letterbox_u8_to_f32(ps->frames_dev, ps->in_dev, B, in->fw, in->fh, net.w, net.h, rt->stream));
     else if (in->kind == Y2_IN_FRAMES) /* byte/255. + resize_image, into the slot's fp32 input */

@@ -108,6 +108,10 @@ class BBox(C.Structure):
                 ("obj_id", C.c_uint), ("track_id", C.c_uint)]
 
 
+FrameDesc = _lib.FrameDesc
+FRAME_RGB24, FRAME_BGR24, FRAME_NV12 = 0, 1, 2  # y2_frame_desc.format
+
+
 class Image(C.Structure):
     _fields_ = [("h", C.c_int), ("w", C.c_int), ("c", C.c_int), ("data", _fp)]
 
@@ -189,6 +193,21 @@ def lib() -> C.CDLL:
         "network_classify_submit_frame_list": (i, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i]),
         "network_classify_batch_frame_list": (None, [Network, i, C.POINTER(C.POINTER(C.c_ubyte)), _ip, _ip, i,
                                                      C.POINTER(ClassHit)]),
+        "network_pipeline_staging_frame_descs": (C.POINTER(C.c_ubyte), [Network, i, i, C.POINTER(FrameDesc),
+                                                                         C.POINTER(C.c_size_t)]),
+        "network_detect_submit_frame_descs": (i, [Network, i, C.POINTER(FrameDesc), C.c_void_p, f, f, i]),
+        "network_detect_batch_frame_descs": (None, [Network, i, C.POINTER(FrameDesc), C.c_void_p, f, f,
+                                                    C.POINTER(Detection), _ip, i]),
+        "network_detect_submit_streams_descs": (i, [Network, i, _ip, C.POINTER(FrameDesc), C.c_void_p, f, f, i]),
+        "network_detect_batch_streams_descs": (None, [Network, i, _ip, C.POINTER(FrameDesc), C.c_void_p, f, f,
+                                                      C.POINTER(Detection), _ip, i]),
+        "network_detect_submit_streams_tracked_descs": (i, [Network, i, _ip, C.POINTER(FrameDesc), C.c_void_p, f, f,
+                                                             i, i]),
+        "network_detect_batch_streams_tracked_descs": (None, [Network, i, _ip, C.POINTER(FrameDesc), C.c_void_p, f,
+                                                              f, i, C.POINTER(BBox), _ip, i]),
+        "network_classify_submit_frame_descs": (i, [Network, i, C.POINTER(FrameDesc), C.c_void_p, i]),
+        "network_classify_batch_frame_descs": (None, [Network, i, C.POINTER(FrameDesc), C.c_void_p, i,
+                                                      C.POINTER(ClassHit)]),
         "network_classify_device": (None, [Network, i, C.POINTER(ClassHit)]),
         "network_classify_batch": (None, [Network, fp, i, C.POINTER(ClassHit)]),
         "network_classify_batch_frames": (None, [Network, C.POINTER(C.c_ubyte), i, i, i, C.POINTER(ClassHit)]),
@@ -252,6 +271,7 @@ def lib() -> C.CDLL:
     assert l.y2_abi_sizeof(3) == C.sizeof(Detection)
     assert l.y2_abi_sizeof(5) == C.sizeof(ClassHit)
     assert l.y2_abi_sizeof(6) == C.sizeof(BBox)
+    assert l.y2_abi_sizeof(7) == C.sizeof(FrameDesc), (l.y2_abi_sizeof(7), C.sizeof(FrameDesc))
     _declared = True
     return l
 
@@ -521,6 +541,186 @@ def network_detect_wait_tracked(net: Network, n: int, max_det: int = 256):
     counts = (C.c_int * net.batch)()
     lib().network_detect_wait_tracked(net, boxes, counts, max_det)
     return _det_lists(boxes, counts, n, max_det)
+
+
+def _rows(obj, ndim_shapes):
+    """(address, shape, byte strides, on_device) of a uint8 array: a numpy array (host) or any object with
+    __cuda_array_interface__ (device), e.g. a torch or cupy tensor"""
+    cai = getattr(obj, "__cuda_array_interface__", None)
+    if cai is not None:
+        if cai["typestr"] not in ("|u1", "<u1", ">u1"):
+            raise ValueError(f"frame_desc: a uint8 array is needed, got typestr {cai['typestr']}")
+        shape = tuple(int(v) for v in cai["shape"])
+        strides = cai.get("strides")
+        if strides is None:  # C-contiguous
+            strides, step = [], 1
+            for d in reversed(shape):
+                strides.insert(0, step)
+                step *= d
+        addr, on_device = int(cai["data"][0]), 1
+    elif isinstance(obj, np.ndarray):
+        if obj.dtype != np.uint8:
+            raise ValueError(f"frame_desc: a uint8 array is needed, got {obj.dtype}")
+        shape, strides, addr, on_device = obj.shape, obj.strides, obj.ctypes.data, 0
+    else:
+        raise TypeError("frame_desc: a numpy array or an object with __cuda_array_interface__ is needed")
+    shape, strides = tuple(shape), tuple(int(v) for v in strides)
+    if len(shape) not in ndim_shapes or any(v <= 0 for v in shape) or any(v < 0 for v in strides):
+        raise ValueError(f"frame_desc: an array of {' or '.join(map(str, ndim_shapes))} dimensions with positive "
+                         f"extents and strides is needed, got shape {shape} strides {strides}")
+    return addr, shape, strides, on_device
+
+
+def _pitch(shape, strides, row_elems: int, what: str) -> int:
+    """the row pitch of rows of row_elems interleaved bytes (the trailing axes must be dense); whether it is wide
+    enough is the library's rule (y2_frame_desc_rows)"""
+    dense = 1
+    for d, st in zip(reversed(shape[1:]), reversed(strides[1:])):
+        if d > 1 and st != dense:
+            raise ValueError(f"frame_desc: {what} rows are not interleaved bytes (shape {shape}, strides {strides})")
+        dense *= d
+    return strides[0] if shape[0] > 1 else row_elems
+
+
+# what y2_frame_desc_rows refuses, by its Y2_FRAME_BAD_* code
+_FRAME_RULES = {1: "a size of 0 or less", 2: "an unknown format", 3: "NV12 needs an even width and height",
+                4: "a row of more than INT_MAX bytes", 5: "rows overlap (pitch below the row's bytes)",
+                6: "UV rows overlap (uv_pitch below the row's bytes)"}
+
+
+def frame_desc(obj, fmt: int) -> FrameDesc:
+    """A y2_frame_desc for a frame held in a numpy array (host memory) or in an object with __cuda_array_interface__
+    (memory of the network's GPU, read in place).  fmt FRAME_RGB24 / FRAME_BGR24: a uint8 [h][w][3] array whose rows
+    may be pitched; FRAME_NV12: one uint8 [h*3/2][w] array (the Y plane, then the interleaved UV plane) or a pair
+    (y [h][w], uv [h/2][w] or [h/2][w/2][2]) on the same side.  The pitch comes from the row stride.  The descriptor
+    keeps a reference to the array(s); device frames must stay unchanged until the wait that returns their batch."""
+    d = FrameDesc()
+    if fmt in (FRAME_RGB24, FRAME_BGR24):
+        addr, shape, strides, on_device = _rows(obj, (3,))
+        if shape[2] != 3:
+            raise ValueError(f"frame_desc: RGB/BGR frames are [h][w][3], got shape {shape}")
+        d.data, d.h, d.w = addr, shape[0], shape[1]
+        d.pitch = _pitch(shape, strides, 3 * shape[1], "frame")
+    elif fmt == FRAME_NV12:
+        if isinstance(obj, (tuple, list)):
+            y, uv = obj
+            addr, shape, strides, on_device = _rows(y, (2,))
+            uaddr, ushape, ustrides, uon = _rows(uv, (2, 3))
+            h, w = shape
+            if uon != on_device:
+                raise ValueError("frame_desc: the Y and UV planes must both be host or both be device arrays")
+            if ushape[0] != h // 2 or int(np.prod(ushape[1:])) != w or (len(ushape) == 3 and ushape[2] != 2):
+                raise ValueError(f"frame_desc: the UV plane of a {w}x{h} NV12 frame is [h/2][w] or [h/2][w/2][2], "
+                                 f"got {ushape}")
+            d.uv, d.uv_pitch = uaddr, _pitch(ushape, ustrides, w, "UV")
+        else:
+            addr, shape, strides, on_device = _rows(obj, (2,))
+            if shape[0] % 3:
+                raise ValueError(f"frame_desc: a one-array NV12 frame is [h*3/2][w], got {shape}")
+            h, w = shape[0] * 2 // 3, shape[1]
+        d.data, d.h, d.w = addr, h, w
+        d.pitch = _pitch(shape, strides, w, "Y")
+    else:
+        raise ValueError(f"frame_desc: unknown format {fmt}")
+    d.format, d.on_device = fmt, on_device
+    rc = _lib.load().y2_frame_desc_rows(C.byref(d), C.byref(_lib.FrameRows()))
+    if rc:
+        raise ValueError(f"frame_desc: {_FRAME_RULES.get(rc, rc)}: {d.w}x{d.h}, pitch {d.pitch}, uv_pitch "
+                         f"{d.uv_pitch}, format {fmt}")
+    d._keep = obj
+    return d
+
+
+def _descs_arg(descs):
+    n = len(descs)
+    return n, (FrameDesc * max(n, 1))(*descs)
+
+
+def network_pipeline_staging_frame_descs(net: Network, slot: int, descs):
+    """The slot's pinned staging buffer laid out for a descriptor list (only sizes, formats and on_device are read):
+    per frame a writable uint8 view at its place ([h][w][3], or [h*3/2][w] for NV12), None for a device frame.  Fill
+    the views and pass frame_desc(view, fmt) to skip the host copy; they stay valid until a larger list makes the
+    slot's buffer grow."""
+    n, arr = _descs_arg(descs)
+    offsets = (C.c_size_t * max(n, 1))()
+    base = C.cast(lib().network_pipeline_staging_frame_descs(net, slot, n, arr, offsets), C.c_void_p).value
+    views = []
+    for i, d in enumerate(descs):
+        if d.on_device:
+            views.append(None)
+            continue
+        shape = (d.h * 3 // 2, d.w) if d.format == FRAME_NV12 else (d.h, d.w, 3)
+        views.append(np.ctypeslib.as_array(C.cast(base + offsets[i], C.POINTER(C.c_ubyte)), shape=shape))
+    return views
+
+
+def network_detect_frame_descs(net: Network, descs, thresh: float, nms: float, max_det: int = 256, ready=None):
+    """Extension: detection on a list of 1 .. batch frame descriptors (frame_desc), converted to RGB and resized on
+    the device.  ready: a raw cudaEvent_t (torch.cuda.Event().cuda_event) the network waits for before it reads any
+    device frame.  Returns (per-image detection arrays, counts) for len(descs) images."""
+    n, arr = _descs_arg(descs)
+    dets = (Detection * (max(n, 1) * max_det))()
+    counts = (C.c_int * max(n, 1))()
+    lib().network_detect_batch_frame_descs(net, n, arr, ready, thresh, nms, dets, counts, max_det)
+    return _det_lists(dets, counts, n, max_det)
+
+
+def network_detect_submit_frame_descs(net: Network, descs, thresh: float, nms: float, max_det: int = 256,
+                                      ready=None) -> int:
+    """Queue a descriptor list on the submit/wait pipeline; network_detect_wait_n(net, len(descs), ...) collects it."""
+    n, arr = _descs_arg(descs)
+    return lib().network_detect_submit_frame_descs(net, n, arr, ready, thresh, nms, max_det)
+
+
+def network_detect_streams_descs(net: Network, stream_ids, descs, thresh: float, nms: float, max_det: int = 256,
+                                 ready=None):
+    """network_detect_streams on frame descriptors."""
+    n, arr = _descs_arg(descs)
+    dets = (Detection * (max(n, 1) * max_det))()
+    counts = (C.c_int * max(n, 1))()
+    lib().network_detect_batch_streams_descs(net, n, _stream_ids(stream_ids, n), arr, ready, thresh, nms, dets, counts,
+                                             max_det)
+    return _det_lists(dets, counts, n, max_det)
+
+
+def network_detect_submit_streams_descs(net: Network, stream_ids, descs, thresh: float, nms: float,
+                                        max_det: int = 256, ready=None) -> int:
+    n, arr = _descs_arg(descs)
+    return lib().network_detect_submit_streams_descs(net, n, _stream_ids(stream_ids, n), arr, ready, thresh, nms,
+                                                     max_det)
+
+
+def network_detect_streams_tracked_descs(net: Network, stream_ids, descs, thresh: float, nms: float,
+                                         use_mean: bool = True, max_det: int = 256, ready=None):
+    """network_detect_streams_tracked on frame descriptors; boxes are scaled to each descriptor's w x h."""
+    n, arr = _descs_arg(descs)
+    boxes = (BBox * (max(n, 1) * max_det))()
+    counts = (C.c_int * max(n, 1))()
+    lib().network_detect_batch_streams_tracked_descs(net, n, _stream_ids(stream_ids, n), arr, ready, thresh, nms,
+                                                     int(use_mean), boxes, counts, max_det)
+    return _det_lists(boxes, counts, n, max_det)
+
+
+def network_detect_submit_streams_tracked_descs(net: Network, stream_ids, descs, thresh: float, nms: float,
+                                                use_mean: bool = True, max_det: int = 256, ready=None) -> int:
+    n, arr = _descs_arg(descs)
+    return lib().network_detect_submit_streams_tracked_descs(net, n, _stream_ids(stream_ids, n), arr, ready, thresh,
+                                                             nms, int(use_mean), max_det)
+
+
+def network_classify_frame_descs(net: Network, descs, top: int = 5, ready=None):
+    """Extension: classification of a list of frame descriptors, each converted to RGB and letterboxed on the device:
+    (indices int32 [n][top], probs float32 [n][top])."""
+    n, arr = _descs_arg(descs)
+    hits = (ClassHit * (max(n, 1) * top))()
+    lib().network_classify_batch_frame_descs(net, n, arr, ready, top, hits)
+    return _hits_arrays(hits, n, top)
+
+
+def network_classify_submit_frame_descs(net: Network, descs, top: int = 5, ready=None) -> int:
+    """Queue a descriptor list for classification; network_classify_wait(net, top, n=len(descs)) collects it."""
+    n, arr = _descs_arg(descs)
+    return lib().network_classify_submit_frame_descs(net, n, arr, ready, top)
 
 
 def network_classify_batch(net: Network, images: np.ndarray | None = None, frames: np.ndarray | None = None,

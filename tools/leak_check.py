@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Developer tool (GPU box): device-memory leak check - parse / predict / detect / resize / free in a loop,
-parse / classify / change the batch / free for a classifier, frame lists whose packed size grows and shrinks, and
-video streams (open, submit with repeats, reset, reopen larger, change the batch, free) and tracked video streams
-(enable tracking, submit with repeats, reset, reopen and enable again, change the batch, free)."""
+parse / classify / change the batch / free for a classifier, frame lists whose packed size grows and shrinks, frame
+descriptor lists (host and device, RGB, BGR and NV12) whose staged size grows and shrinks, video streams (open,
+submit with repeats, reset, reopen larger, change the batch, free) and tracked video streams (enable tracking, submit
+with repeats, reset, reopen and enable again, change the batch, free)."""
 import sys
 import tempfile
 from pathlib import Path
@@ -88,6 +89,37 @@ def frame_list_cycle(name, side, batch):
     dn.free_network(net)
 
 
+def descs_cycle(name, side, batch):
+    text = synth.CFGS[name](batch=batch, w=side, h=side)
+    (tmp / "d.cfg").write_text(text)
+    w = tmp / f"{name}.weights"
+    if not w.exists():
+        synth.write_weights(w, text, seed=1234)
+    net = dn.parse_network_cfg(tmp / "d.cfg")
+    dn.load_weights(net, w)
+    rng = np.random.default_rng(5)
+    fmts = (dn.FRAME_RGB24, dn.FRAME_NV12, dn.FRAME_BGR24)
+    # staged sizes small, large, all on the device (the table alone), larger: host and device frames mixed
+    for n, (fw, fh), host in ((1, (500, 376), True), (batch, (1280, 720), True), (batch, (1920, 1080), False),
+                              (batch, (1920, 1080), True)):
+        frames, descs = [], []
+        for i in range(n):
+            fmt = fmts[i % 3]
+            shape = (fh * 3 // 2, fw) if fmt == dn.FRAME_NV12 else (fh, fw, 3)
+            a = rng.integers(0, 256, size=shape, dtype=np.uint8)
+            if not (host and i % 2 == 0):
+                a = torch.from_numpy(a).cuda()
+            frames.append(a)
+            descs.append(dn.frame_desc(a, fmt))
+        torch.cuda.synchronize()
+        dn.network_detect_submit_frame_descs(net, descs, 0.02, 0.4, 64)
+        dn.network_detect_submit_frame_descs(net, descs[::-1], 0.02, 0.4, 64)
+        dn.network_detect_wait_n(net, n, 64)
+        dn.network_detect_wait_n(net, n, 64)
+        del frames, descs
+    dn.free_network(net)
+
+
 def streams_cycle(name, side, batch):
     text = synth.CFGS[name](batch=batch, w=side, h=side)
     (tmp / "s.cfg").write_text(text)
@@ -140,6 +172,7 @@ def tracked_cycle(name, side, batch):
 
 for fn, name, side, batch in ((cycle, "tiny-yolo-voc", 416, 8), (cycle, "yolo-voc", 416, 64),
                               (classify_cycle, "darknet19_448", 448, 16), (frame_list_cycle, "tiny-yolo-voc", 416, 16),
+                              (descs_cycle, "tiny-yolo-voc", 416, 16),
                               (streams_cycle, "tiny-yolo-voc", 416, 16), (tracked_cycle, "tiny-yolo-voc", 416, 16)):
     fn(name, side, batch)  # warm: allocator pools, per-device scratch
     torch.cuda.synchronize()
