@@ -900,14 +900,17 @@ __device__ __forceinline__ float activate_any(float x, int a)
     case 2: return x > 0.f ? x : .01f * x;
     case 3: return x;
     case 4: return (x > 0.f ? x : 0.f) + .1f * x;
-    case 5: return (2.f / (1.f + expf(-2.f * x)) - 1.f);
+    case 5: return tanhf(x); /* = 2/(1+e^-2x) - 1, which keeps only a few bits for |x| << 1 */
     case 6: return x < -4.f ? .01f * (x + 4.f) : x > 4.f ? .01f * (x - 4.f) + 1.f : .125f * x + .5f;
     case 7: return x > 0.f ? x : .1f * x;
-    case 8: return x >= 0.f ? x : expf(x) - 1.f;
-    case 9: return 2.f / (1.f + expf(-x)) - 1.f;
+    case 8: return x >= 0.f ? x : expm1f(x);
+    case 9: return tanhf(.5f * x); /* = 2/(1+e^-x) - 1 */
     case 10: {
+        /* floor(x / 2.) of the reference, in double there: floor(floor(x) / 2), x / 2.f would underflow to -0
+         * for the smallest negative denormal */
         const int n = (int)floorf(x);
-        return (n % 2 == 0) ? floorf(x / 2.f) : (x - n) + floorf(x / 2.f);
+        const float half = (float)(n >> 1);
+        return (n % 2 == 0) ? half : (x - n) + half;
     }
     case 11: return x < -1.f ? -1.f : x > 1.f ? 1.f : x;
     case 12: return x < 0.f ? .001f * x : x > 1.f ? .001f * (x - 1.f) + 1.f : x;
