@@ -464,6 +464,38 @@ int network_detect_submit_frame_descs(network net, int n, const y2_frame_desc *d
                                       float nms, int max_det);
 void network_detect_batch_frame_descs(network net, int n, const y2_frame_desc *descs, void *ready, float thresh,
                                       float nms, y2_detection *dets, int *counts, int max_det);
+/* ---- tiled detection of large frames ("sliced inference"): each frame of W x H pixels goes through the network as
+ * overlapping tiles, and the tiles' detections are merged per frame by do_nms_sort over their union.
+ * Tiles, per frame: the whole frame first when full = 1, then a cols x rows grid, row-major, of tw x th windows with
+ *   tw = min(W, ceil((W + (cols-1)*overlap) / cols)) (NV12: rounded up to even),
+ *   x0_i = cols == 1 ? 0 : floor(i*(W - tw) / (cols-1)) (NV12: bit 0 cleared), the same for rows, H, th and y0_j:
+ * the first tile starts at 0, the last ends at W, and neighbours share at least overlap columns (NV12: overlap - 1).
+ * Each tile is converted, resized and run as a frame of network_detect_submit_frame_descs; its boxes (get_region_boxes
+ * relative to the tile) go to frame coordinates as x = ((float)x0 + x*(float)tw) / (float)W, w = (w*(float)tw) /
+ * (float)W (fp32, round-to-nearest, no FMA; an axis the tile spans whole passes unchanged), likewise y and h.  The
+ * tiles' boxes and probability rows, in tile order (union index t * l.w*l.h*l.n + i), then take do_nms_sort (nms <= 0
+ * skips it) and the final pick of Detector::detect, in union-index order.  dets [n][max_det] are relative to the frame
+ * with box_index the union index; counts hold the full number.  A 1 x 1 tiling without full is exactly
+ * network_detect_submit_frame_descs.
+ * A frame's tiles are network images of one batch, so the list may hold at most net.batch tiles.  A host frame is
+ * staged and uploaded once, however many tiles read it; device frames are read in place.  ready and the lifetimes are
+ * those of the descriptor entries.  Collected by network_detect_wait (n frames).
+ * Refused through error(), before anything is staged: what the descriptor entries refuse, a NULL tiling, cols or rows
+ * outside 1 .. Y2_TILE_MAX, overlap < 0, full not 0 or 1, more tiles than net.batch, and a softmax-tree region. */
+#ifndef Y2_TILING_DEFINED
+#define Y2_TILING_DEFINED
+#define Y2_TILE_MAX 16
+typedef struct y2_tiling {
+    int cols, rows; /* 1 .. Y2_TILE_MAX */
+    int overlap;    /* columns (rows) neighbours share at least; NV12: at least overlap - 1 */
+    int full;       /* 1: the whole frame is the frame's first tile */
+} y2_tiling;
+#endif
+int network_detect_submit_tiled_descs(network net, int n, const y2_frame_desc *descs, const y2_tiling *tiling,
+                                      void *ready, float thresh, float nms, int max_det);
+void network_detect_batch_tiled_descs(network net, int n, const y2_frame_desc *descs, const y2_tiling *tiling,
+                                      void *ready, float thresh, float nms, y2_detection *dets, int *counts,
+                                      int max_det);
 /* ---- many video streams in one batch, each frame detected on the 3-frame mean of its stream: per stream the
  * result is bit-identical to Detector::detect(img, thresh, use_mean = true) (yolo_v2_class.cpp:206-216) on that
  * stream's frames in order.  A stream is a ring of the last 3 region outputs, all zero at the start, and a
@@ -613,7 +645,8 @@ int network_launch_count(network net);
 int network_profile_layers(network net, float *ms_per_layer, int n);
 /* 1 -> run layers eagerly instead of replaying the captured CUDA graph */
 void network_set_eager(network net, int eager);
-/* sizeof(layer|network|network_state|y2_detection|box|y2_class_hit|y2_bbox|y2_frame_desc) for what = 0..7: lets a
+/* sizeof(layer|network|network_state|y2_detection|box|y2_class_hit|y2_bbox|y2_frame_desc|y2_tiling) for what = 0..8:
+ * lets a
  * binding that passes these structs by value check its mirror against the library it loaded. */
 size_t y2_abi_sizeof(int what);
 

@@ -282,6 +282,78 @@ size_t y2_frame_desc_layout(int n, const y2_frame_desc *descs, int w, int h, int
  * resize_image into its window, bit-identical to y2_frames_u8_to_f32 on the converted tight RGB frame; images
  * n..batch-1 are all .5f.  Every address in the table must be readable device memory over its frame's rows. */
 int y2_frames_src_to_f32(const y2_frame_src *table, int n, float *dst, int batch, int w, int h, y2_stream_t s);
+
+/* Tiled detection of large frames (the tiling is also declared in darknet_b200.h): every frame of W x H pixels is cut
+ * into the whole frame (full = 1) and a cols x rows grid of tiles, row-major, each tile read in place with the frame's
+ * pitch.  tw = min(W, ceil((W + (cols-1)*overlap) / cols)), rounded up to even for NV12; x0_i = cols == 1 ? 0 :
+ * floor(i*(W - tw) / (cols-1)), bit 0 cleared for NV12; the same with rows, H, th and y0_j. */
+#ifndef Y2_TILING_DEFINED
+#define Y2_TILING_DEFINED
+#define Y2_TILE_MAX 16
+typedef struct y2_tiling {
+    int cols, rows; /* 1 .. Y2_TILE_MAX */
+    int overlap;    /* columns (rows) neighbours share at least; NV12: at least overlap - 1 */
+    int full;       /* 1: the whole frame is the frame's first tile */
+} y2_tiling;
+#endif
+/* One tile: its frame in the list, its window in that frame, and the frame's size */
+typedef struct y2_tile {
+    int frame;
+    int x0, y0, w, h;
+    int frame_w, frame_h;
+    int reserved;
+} y2_tile;
+/* A frame's tiles are the consecutive network images first .. first + count - 1 */
+typedef struct y2_tile_span {
+    int first, count;
+} y2_tile_span;
+/* Where y2_tile_plan puts things in the staged region: the host frames (as y2_frame_desc_layout stages them: each once,
+ * tight), then y2_frame_src[n_tiles], y2_tile[n_tiles] and y2_tile_span[n], each 16-byte aligned. */
+typedef struct y2_tile_layout {
+    int n_tiles;
+    int max_tiles;        /* tiles of the frame with the most */
+    size_t recs_offset;
+    size_t tiles_offset;
+    size_t spans_offset;
+    size_t bytes;         /* the whole region */
+} y2_tile_layout;
+enum {
+    Y2_TILE_OK = 0,
+    Y2_TILE_BAD_DESC = 1,     /* n < 1, descs NULL, or a descriptor breaks a rule of y2_frame_desc_rows */
+    Y2_TILE_NULL = 2,         /* tiling NULL */
+    Y2_TILE_BAD_GRID = 3,     /* cols or rows outside 1 .. Y2_TILE_MAX */
+    Y2_TILE_BAD_OVERLAP = 4,  /* overlap < 0 */
+    Y2_TILE_BAD_FULL = 5,     /* full not 0 or 1 */
+    Y2_TILE_TOO_MANY = 6      /* more tiles than max_tiles */
+};
+/* The tile plan of n descriptors for a w x h network: fills *layout and, with staged non-NULL, writes the records,
+ * tiles and spans at their offsets in staged.  A tile's record is its window of the frame resized to w x h
+ * (resize_image), with win.offset / uv the frame's record (y2_frame_desc_layout, letterbox 0) advanced to (x0, y0): for
+ * a host frame an offset into the staged region (the caller adds the region's device address), for a device frame an
+ * address.  Returns Y2_TILE_OK or the first rule broken (checked in the order of the enum), before anything is
+ * written.  Host only. */
+int y2_tile_plan(int n, const y2_frame_desc *descs, const y2_tiling *tiling, int w, int h, int max_tiles,
+                 unsigned char *staged, y2_tile_layout *layout);
+/* The tiles' boxes to frame coordinates, in place: boxes [n_tiles][total][4] (relative to the tile) become
+ * x = ((float)x0 + x*(float)tw) / (float)W, w = (w*(float)tw) / (float)W, the same for y and h, in fp32
+ * round-to-nearest without contraction; an axis the tile spans whole (x0 == 0 && tw == W) passes unchanged.  tiles: a
+ * device table. */
+int y2_tile_map(float *boxes, const y2_tile *tiles, int n_tiles, int total, y2_stream_t s);
+/* do_nms_sort over each frame's union of tiles: for frame f, the boxes and probability rows of its tiles
+ * spans[f].first .. + count, in tile order (union index t*total + i), are one do_nms_sort of count*total boxes,
+ * bit-exact with the reference (order carried across classes, ties by union index).  Suppressed entries are left
+ * NEGATIVE, as by y2_nms_mark.  nz_count [n_tiles][classes]: the decode's candidate counters.  The number of
+ * candidates is not bounded by shared memory: a class with more than fit spills to ws, y2_tile_nms_ws_bytes(n,
+ * classes, max_tiles * total) bytes (max_tiles: the most tiles of one frame).  spans: a device table. */
+size_t y2_tile_nms_ws_bytes(int n, int classes, long long max_span);
+int y2_tile_nms(const float *boxes, float *probs, const int *nz_count, const y2_tile_span *spans, int n, int total,
+                int classes, int max_tiles, float thresh, void *ws, size_t ws_bytes, y2_stream_t s);
+struct y2_det;
+/* The final pick of each frame over its union: max_index with negative entries read as 0, kept when prob > thresh, in
+ * union-index order, into det [n][max_det] (box_index the union index) and count [n] (the full number).  Hands
+ * the spans' rows of nz_count [tiles][classes] back zeroed. */
+int y2_tile_collect(const float *boxes, const float *probs, const y2_tile_span *spans, int n, int total, int classes,
+                    float thresh, struct y2_det *det, int *count, int max_det, int *nz_count, y2_stream_t s);
 /* The device ordinal of the device or managed allocation that holds all of [p, p + bytes), or -1 when p is host or
  * unknown memory or the range leaves its allocation. */
 int y2_pointer_device(const void *p, size_t bytes);

@@ -83,6 +83,51 @@ def frame_desc_layout(descs, w: int, h: int, letterbox: bool):
     return list(recs)[:n], toff.value, total
 
 
+class Tiling(C.Structure):
+    """Mirror of `y2_tiling`: a cols x rows grid of tiles sharing `overlap` pixels, with the whole frame first when
+    `full` is 1."""
+    _fields_ = [("cols", C.c_int), ("rows", C.c_int), ("overlap", C.c_int), ("full", C.c_int)]
+
+
+class Tile(C.Structure):
+    """Mirror of `y2_tile`: a tile's frame, its window in that frame and the frame's size."""
+    _fields_ = [("frame", C.c_int), ("x0", C.c_int), ("y0", C.c_int), ("w", C.c_int), ("h", C.c_int),
+                ("frame_w", C.c_int), ("frame_h", C.c_int), ("reserved", C.c_int)]
+
+
+class TileSpan(C.Structure):
+    """Mirror of `y2_tile_span`: a frame's tiles are network images first .. first + count - 1."""
+    _fields_ = [("first", C.c_int), ("count", C.c_int)]
+
+
+class TileLayout(C.Structure):
+    """Mirror of `y2_tile_layout`: where the tile plan's tables sit in the staged region."""
+    _fields_ = [("n_tiles", C.c_int), ("max_tiles", C.c_int), ("recs_offset", C.c_size_t),
+                ("tiles_offset", C.c_size_t), ("spans_offset", C.c_size_t), ("bytes", C.c_size_t)]
+
+
+def tile_plan(descs, tiling, w: int, h: int, max_tiles: int):
+    """y2_tile_plan for a list of FrameDesc and a Tiling (or None) on a w x h network: (code, layout, records, tiles,
+    spans).  With a code other than Y2_TILE_OK (0) the last four are None."""
+    lib = load()
+    n = len(descs)
+    arr = (FrameDesc * max(n, 1))(*descs)
+    lay = TileLayout()
+    tp = C.byref(tiling) if tiling is not None else None
+    rc = lib.y2_tile_plan(n, arr, tp, w, h, max_tiles, None, C.byref(lay))
+    if rc:
+        return rc, None, None, None, None
+    buf = (C.c_ubyte * lay.bytes)()
+    check(lib.y2_tile_plan(n, arr, tp, w, h, max_tiles, buf, None), "y2_tile_plan")
+    base = C.addressof(buf)
+    recs = list((FrameSrc * lay.n_tiles).from_address(base + lay.recs_offset))
+    tiles = list((Tile * lay.n_tiles).from_address(base + lay.tiles_offset))
+    spans = list((TileSpan * n).from_address(base + lay.spans_offset))
+    # the records outlive the buffer as copies
+    return rc, lay, [FrameSrc.from_buffer_copy(r) for r in recs], [Tile.from_buffer_copy(t) for t in tiles], \
+        [TileSpan.from_buffer_copy(s) for s in spans]
+
+
 class StreamSrc(C.Structure):
     """Mirror of `y2_stream_src`: where the 3 ring slots of an image's stream come from, and the ring row it commits."""
     _fields_ = [("src", C.c_int * 3), ("commit", C.c_int)]
@@ -199,6 +244,11 @@ def _declare(lib: C.CDLL) -> None:
         "y2_frame_desc_rows": (i, [C.POINTER(FrameDesc), C.POINTER(FrameRows)]),
         "y2_frames_src_to_f32": (i, [vp, i, vp, i, i, i, vp]),
         "y2_pointer_device": (i, [vp, C.c_size_t]),
+        "y2_tile_plan": (i, [i, C.POINTER(FrameDesc), C.POINTER(Tiling), i, i, i, vp, C.POINTER(TileLayout)]),
+        "y2_tile_map": (i, [vp, vp, i, i, vp]),
+        "y2_tile_nms_ws_bytes": (C.c_size_t, [i, i, C.c_longlong]),
+        "y2_tile_nms": (i, [vp, vp, vp, vp, i, i, i, i, f, vp, C.c_size_t, vp]),
+        "y2_tile_collect": (i, [vp, vp, vp, i, i, i, f, vp, vp, i, vp, vp]),
         "y2_stream_plan": (i, [i, C.POINTER(i), i, C.POINTER(i), C.POINTER(i), C.POINTER(StreamSrc)]),
         "y2_stream_mean": (i, [vp, vp, vp, i, i, vp, vp]),
         "y2_stream_commit": (i, [vp, vp, vp, i, i, vp]),

@@ -1202,6 +1202,80 @@ extern "C" size_t y2_frame_desc_layout(int n, const y2_frame_desc *descs, int w,
     return off + (size_t)n * sizeof(y2_frame_src);
 }
 
+// One axis of the tiling: the tile extent of a frame extent `ext`, and the origin of tile i of `k`.
+static int tile_extent(int ext, int k, int overlap, bool nv12)
+{
+    long long t = ((long long)ext + (long long)(k - 1) * overlap + k - 1) / k;
+    if (t > ext) t = ext;
+    if (nv12 && (t & 1)) ++t; // ext is even, so t stays <= ext
+    return (int)t;
+}
+static int tile_origin(int i, int k, int ext, int t, bool nv12)
+{
+    const int o = k == 1 ? 0 : (int)((long long)i * (ext - t) / (k - 1));
+    return nv12 ? o & ~1 : o;
+}
+
+static size_t align16(size_t v) { return (v + 15) & ~(size_t)15; }
+
+extern "C" int y2_tile_plan(int n, const y2_frame_desc *descs, const y2_tiling *tiling, int w, int h, int max_tiles,
+                            unsigned char *staged, y2_tile_layout *layout)
+{
+    if (n < 1 || !descs || w <= 0 || h <= 0) return Y2_TILE_BAD_DESC;
+    for (int i = 0; i < n; ++i) {
+        y2_frame_rows fr;
+        if (y2_frame_desc_rows(&descs[i], &fr) != Y2_FRAME_OK) return Y2_TILE_BAD_DESC;
+    }
+    if (!tiling) return Y2_TILE_NULL;
+    const y2_tiling t = *tiling;
+    if (t.cols < 1 || t.cols > Y2_TILE_MAX || t.rows < 1 || t.rows > Y2_TILE_MAX) return Y2_TILE_BAD_GRID;
+    if (t.overlap < 0) return Y2_TILE_BAD_OVERLAP;
+    if (t.full != 0 && t.full != 1) return Y2_TILE_BAD_FULL;
+    const int per_frame = t.full + t.cols * t.rows;
+    const long long n_tiles = (long long)n * per_frame;
+    if (n_tiles > max_tiles) return Y2_TILE_TOO_MANY;
+    y2_tile_layout lay = {};
+    lay.n_tiles = (int)n_tiles;
+    lay.max_tiles = per_frame;
+    lay.recs_offset = y2_frame_desc_layout(n, descs, w, h, 0, nullptr, nullptr) - (size_t)n * sizeof(y2_frame_src);
+    lay.tiles_offset = align16(lay.recs_offset + (size_t)n_tiles * sizeof(y2_frame_src));
+    lay.spans_offset = align16(lay.tiles_offset + (size_t)n_tiles * sizeof(y2_tile));
+    lay.bytes = lay.spans_offset + (size_t)n * sizeof(y2_tile_span);
+    if (layout) *layout = lay;
+    if (!staged) return Y2_TILE_OK;
+    // each frame's own record (host frames at their staged offsets), written where the tile records go, then each
+    // frame's tiles from the last frame back, so a frame's record is read before a tile record covers it
+    y2_frame_src *recs = reinterpret_cast<y2_frame_src *>(staged + lay.recs_offset);
+    y2_tile *tiles = reinterpret_cast<y2_tile *>(staged + lay.tiles_offset);
+    y2_tile_span *spans = reinterpret_cast<y2_tile_span *>(staged + lay.spans_offset);
+    y2_frame_desc_layout(n, descs, w, h, 0, recs, nullptr);
+    for (int f = n - 1; f >= 0; --f) {
+        const y2_frame_src fr = recs[f];
+        const y2_frame_desc &d = descs[f];
+        const bool nv12 = d.format == Y2_FRAME_NV12;
+        const int tw = tile_extent(d.w, t.cols, t.overlap, nv12), th = tile_extent(d.h, t.rows, t.overlap, nv12);
+        const int first = f * per_frame;
+        spans[f] = y2_tile_span{first, per_frame};
+        for (int k = per_frame - 1; k >= 0; --k) {
+            y2_tile g = {f, 0, 0, d.w, d.h, d.w, d.h, 0};
+            if (k >= t.full) {
+                const int j = k - t.full;
+                g.w = tw;
+                g.h = th;
+                g.x0 = tile_origin(j % t.cols, t.cols, d.w, tw, nv12);
+                g.y0 = tile_origin(j / t.cols, t.rows, d.h, th, nv12);
+            }
+            y2_frame_src r = fr;
+            r.win = frame_window(g.w, g.h, w, h, 0);
+            r.win.offset = fr.win.offset + (unsigned long long)g.y0 * fr.pitch + (unsigned long long)g.x0 * (nv12 ? 1 : 3);
+            if (nv12) r.uv = fr.uv + (unsigned long long)(g.y0 / 2) * fr.uv_pitch + g.x0;
+            recs[first + k] = r;
+            tiles[first + k] = g;
+        }
+    }
+    return Y2_TILE_OK;
+}
+
 extern "C" int y2_frames_src_to_f32(const y2_frame_src *table, int n, float *dst, int batch, int w, int h,
                                     y2_stream_t s)
 {

@@ -220,9 +220,295 @@ __global__ void __launch_bounds__(1024) nms_unsorted_kernel(float *probs, const 
     }
 }
 
+// ---- tiled detection: do_nms_sort over a frame's union of tiles --------------------------------------------------
+// A frame's tiles are consecutive images of the batch, so the union of their boxes and probability rows is one
+// contiguous span of count * total rows, union index u = tile * total + box.
+
+// boxes relative to a tile -> relative to its frame (x0 == 0 && tw == W: the axis passes unchanged)
+__global__ void tile_map_kernel(float4 *__restrict__ boxes, const y2_tile *__restrict__ tiles, long long nboxes,
+                                int total)
+{
+    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < nboxes;
+         t += (long long)gridDim.x * blockDim.x) {
+        const y2_tile g = tiles[t / total];
+        float4 b = boxes[t];
+        if (!(g.x0 == 0 && g.w == g.frame_w)) {
+            const float tw = (float)g.w, fw = (float)g.frame_w;
+            b.x = ((float)g.x0 + b.x * tw) / fw;
+            b.z = (b.z * tw) / fw;
+        }
+        if (!(g.y0 == 0 && g.h == g.frame_h)) {
+            const float th = (float)g.h, fh = (float)g.frame_h;
+            b.y = ((float)g.y0 + b.y * th) / fh;
+            b.w = (b.w * th) / fh;
+        }
+        boxes[t] = b;
+    }
+}
+
+static const int TILE_NMS_THREADS = 256;
+static const int TILE_NMS_SMEM_CAP = 2048; // candidates a block stages in shared memory (a power of two)
+static const int TILE_NMS_PER_SM = 4;      // blocks of TILE_NMS_SMEM_CAP * 25 bytes each fit an SM
+
+// a candidate's sort key: ascending keys are p descending, then union index ascending (p > 0, so its bits order like
+// its value)
+__device__ __forceinline__ unsigned long long cand_key(float p, int u)
+{
+    return ((unsigned long long)(0xffffffffu - __float_as_uint(p)) << 32) | (unsigned)u;
+}
+__device__ __forceinline__ unsigned key_hi(unsigned long long k) { return (unsigned)(k >> 32); }
+
+// Persistent grid over (frame, class) pairs with two or more candidates, as nms_mark_kernel, but without a bound on
+// the candidates: up to TILE_NMS_SMEM_CAP they are staged in shared memory, beyond that in the block's slice of ws
+// (ws_stride 8-byte words: the keys, the boxes in sorted order, one alive byte per key).  The order is
+// nms_mark_kernel's rank order, found by a bitonic sort on (p desc, union index asc) and then, inside each run of
+// equal p, an insertion sort with sorts_before; sorts_before is a total order that agrees with the key wherever the p
+// differ, so both give the same sequence.  Dynamic smem: box[cap] float4, key[cap] u64, alive[cap] u8.
+__global__ void __launch_bounds__(TILE_NMS_THREADS)
+    tile_nms_kernel(const float4 *__restrict__ boxes, float *probs, const int *__restrict__ cnt,
+                    const y2_tile_span *__restrict__ spans, int n, int total, int classes, float thresh,
+                    unsigned long long *__restrict__ ws, long long ws_stride)
+{
+    extern __shared__ __align__(16) unsigned char tile_smem[];
+    float4 *s_box = reinterpret_cast<float4 *>(tile_smem);
+    unsigned long long *s_key = reinterpret_cast<unsigned long long *>(s_box + TILE_NMS_SMEM_CAP);
+    unsigned char *s_alive = reinterpret_cast<unsigned char *>(s_key + TILE_NMS_SMEM_CAP);
+    __shared__ int s_m;
+    const long long pairs = (long long)n * classes;
+    for (long long pair = blockIdx.x; pair < pairs; pair += gridDim.x) {
+        const int f = (int)(pair / classes), k = (int)(pair - (long long)f * classes);
+        const y2_tile_span sp = spans[f];
+        int m = 0;
+        for (int t = 0; t < sp.count; ++t) m += cnt[(size_t)(sp.first + t) * classes + k];
+        if (m <= 1) continue; // uniform per block
+        const int span = sp.count * total;
+        float *pimg = probs + (size_t)sp.first * total * classes;
+        const float4 *bimg = boxes + (size_t)sp.first * total;
+        int P = 1;
+        while (P < m) P <<= 1;
+        const bool fits = P <= TILE_NMS_SMEM_CAP;
+        unsigned long long *key = fits ? s_key : ws + blockIdx.x * ws_stride;
+        float4 *box = fits ? s_box : reinterpret_cast<float4 *>(key + P);
+        unsigned char *alive = fits ? s_alive : reinterpret_cast<unsigned char *>(key + 3 * (long long)P);
+
+        // 1. the candidates, in any order (the sort decides it)
+        if (threadIdx.x == 0) s_m = 0;
+        __syncthreads();
+        for (int u = threadIdx.x; u < span; u += blockDim.x) {
+            const float p = pimg[(size_t)u * classes + k];
+            if (p != 0.f) {
+                const int pos = atomicAdd(&s_m, 1);
+                if (pos < P) key[pos] = cand_key(fabsf(p), u);
+            }
+        }
+        __syncthreads();
+        m = min(s_m, P);
+        for (int a = m + threadIdx.x; a < P; a += blockDim.x) key[a] = ~0ull;
+        __syncthreads();
+
+        // 2. bitonic sort of the keys
+        for (int size = 2; size <= P; size <<= 1)
+            for (int stride = size >> 1; stride > 0; stride >>= 1) {
+                for (int a = threadIdx.x; a < P; a += blockDim.x) {
+                    const int b = a ^ stride;
+                    if (b > a) {
+                        const unsigned long long ka = key[a], kb = key[b];
+                        if ((ka > kb) == ((a & size) == 0)) {
+                            key[a] = kb;
+                            key[b] = ka;
+                        }
+                    }
+                }
+                __syncthreads();
+            }
+
+        // 3. runs of equal p, now in union-index order, take the order do_nms_sort carried over from the earlier
+        //    classes: the thread at a run's start sorts it (a run only permutes keys with its own p)
+        if (k > 0)
+            for (int a = threadIdx.x; a < m; a += blockDim.x) {
+                const unsigned hi = key_hi(key[a]);
+                if ((a > 0 && key_hi(key[a - 1]) == hi) || a + 1 >= m || key_hi(key[a + 1]) != hi) continue;
+                const float p = __uint_as_float(0xffffffffu - hi);
+                int e = a + 1;
+                while (e < m && key_hi(key[e]) == hi) ++e;
+                for (int x = a + 1; x < e; ++x) {
+                    const unsigned long long kx = key[x];
+                    int y = x - 1;
+                    while (y >= a && sorts_before(pimg, classes, k, (int)(unsigned)kx, p, (int)(unsigned)key[y], p)) {
+                        key[y + 1] = key[y];
+                        --y;
+                    }
+                    key[y + 1] = kx;
+                }
+            }
+        __syncthreads();
+
+        // 4. greedy suppression in that order, the boxes staged in it; a barrier only after a live box acted
+        for (int a = threadIdx.x; a < m; a += blockDim.x) {
+            box[a] = bimg[(unsigned)key[a]];
+            alive[a] = 1;
+        }
+        __syncthreads();
+        for (int i = 0; i < m - 1; ++i) {
+            if (!alive[i]) continue; // uniform: everyone reads the same flag
+            const float4 a = box[i];
+            for (int j = i + 1 + threadIdx.x; j < m; j += blockDim.x)
+                if (alive[j] && box_iou_ref(a, box[j]) > thresh) alive[j] = 0;
+            __syncthreads();
+        }
+
+        // 5. mark the suppressed entries (the sign flip keeps |p| for the other classes' tie-breaks)
+        for (int a = threadIdx.x; a < m; a += blockDim.x)
+            if (!alive[a]) {
+                float *q = pimg + (size_t)(unsigned)key[a] * classes + k;
+                *q = -fabsf(*q);
+            }
+        __syncthreads(); // the staging is reused by this block's next pair
+    }
+}
+
+// The final pick over each frame's union (one block per frame): per row max_index (utils.c:533-545, first maximum,
+// negative = suppressed = 0), kept when > thresh, compacted in union-index order as collect_kernel does.  Hands the
+// frame's tiles' candidate counters back zeroed.
+static const int TILE_COLLECT_THREADS = 512;
+__global__ void __launch_bounds__(TILE_COLLECT_THREADS)
+    tile_collect_kernel(const float4 *__restrict__ boxes, const float *__restrict__ probs,
+                        const y2_tile_span *__restrict__ spans, int total, int classes, float thresh,
+                        y2_det *__restrict__ det, int *__restrict__ count, int max_det, int *__restrict__ nz_count)
+{
+    __shared__ int s_warp_total[32];
+    __shared__ int s_running;
+    const int f = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const y2_tile_span sp = spans[f];
+    const int span = sp.count * total;
+    const float *pimg = probs + (size_t)sp.first * total * classes;
+    const float4 *bimg = boxes + (size_t)sp.first * total;
+    y2_det *d = det + (size_t)f * max_det;
+    if (threadIdx.x == 0) s_running = 0;
+    __syncthreads();
+    for (int base = 0; base < span; base += blockDim.x) {
+        const int i = base + threadIdx.x;
+        int obj = -1;
+        float best = 0.f;
+        if (i < span) {
+            const float *p = pimg + (size_t)i * classes;
+            best = fmaxf(p[0], 0.f);
+            int arg = 0;
+            for (int j = 1; j < classes; ++j) {
+                const float v = fmaxf(p[j], 0.f);
+                if (v > best) {
+                    best = v;
+                    arg = j;
+                }
+            }
+            if (best > thresh) obj = arg;
+        }
+        const unsigned ballot = __ballot_sync(0xffffffffu, obj >= 0);
+        if (lane == 0) s_warp_total[warp] = __popc(ballot);
+        __syncthreads();
+        int before = s_running;
+        for (int wv = 0; wv < warp; ++wv) before += s_warp_total[wv];
+        const int pos = before + __popc(ballot & ((1u << lane) - 1u));
+        if (obj >= 0 && pos < max_det) {
+            const float4 q = bimg[i];
+            d[pos] = y2_det{q.x, q.y, q.z, q.w, best, obj, i};
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            int t = s_running;
+            for (int wv = 0; wv < nw; ++wv) t += s_warp_total[wv];
+            s_running = t;
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) count[f] = s_running;
+    for (int j = threadIdx.x; j < sp.count * classes; j += blockDim.x) nz_count[(size_t)sp.first * classes + j] = 0;
+}
+
 } // namespace y2
 
 using namespace y2;
+
+extern "C" int y2_tile_map(float *boxes, const y2_tile *tiles, int n_tiles, int total, y2_stream_t s)
+{
+    if (!boxes || !tiles || n_tiles < 1 || total < 1) return Y2_EINVAL;
+    const long long nb = (long long)n_tiles * total;
+    long long blocks = (nb + 255) / 256;
+    if (blocks > (long long)sm_count() * 8) blocks = (long long)sm_count() * 8;
+    tile_map_kernel<<<(int)blocks, 256, 0, to_stream(s)>>>(reinterpret_cast<float4 *>(boxes), tiles, nb, total);
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
+}
+
+static int tile_nms_grid(int n, int classes)
+{
+    const long long pairs = (long long)n * classes, cap = (long long)sm_count() * TILE_NMS_PER_SM;
+    return (int)(pairs < cap ? pairs : cap);
+}
+
+static long long pow2_at_least(long long v)
+{
+    long long p = 1;
+    while (p < v) p <<= 1;
+    return p;
+}
+
+extern "C" size_t y2_tile_nms_ws_bytes(int n, int classes, long long max_span)
+{
+    if (n < 1 || classes < 1 || max_span <= TILE_NMS_SMEM_CAP) return 0;
+    const long long P = pow2_at_least(max_span);
+    return (size_t)tile_nms_grid(n, classes) * (size_t)(3 * P + P / 8) * 8;
+}
+
+extern "C" int y2_tile_nms(const float *boxes, float *probs, const int *cnt, const y2_tile_span *spans, int n,
+                           int total, int classes, int max_tiles, float thresh, void *ws, size_t ws_bytes,
+                           y2_stream_t s)
+{
+    const long long max_span = (long long)max_tiles * total;
+    if (!boxes || !probs || !cnt || !spans || n < 1 || total < 1 || classes < 1 || max_tiles < 1 ||
+        max_span > 0x40000000LL) {
+        set_error("y2_tile_nms: invalid arguments (n=%d total=%d classes=%d max_tiles=%d)", n, total, classes,
+                  max_tiles);
+        return Y2_EINVAL;
+    }
+    const size_t need = y2_tile_nms_ws_bytes(n, classes, max_span);
+    if (need > ws_bytes || (need && !ws)) {
+        set_error("y2_tile_nms: %zu bytes of scratch needed, %zu given", need, ws_bytes);
+        return Y2_EINVAL;
+    }
+    const long long P = pow2_at_least(max_span);
+    const size_t smem = (size_t)TILE_NMS_SMEM_CAP * (sizeof(float4) + sizeof(unsigned long long) + 1);
+    static bool attr_done[64] = {false};
+    int dev = 0;
+    Y2_CUDA_CHECK(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64 || !attr_done[dev]) {
+        Y2_CUDA_CHECK(cudaFuncSetAttribute(tile_nms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (dev >= 0 && dev < 64) attr_done[dev] = true;
+    }
+    tile_nms_kernel<<<tile_nms_grid(n, classes), TILE_NMS_THREADS, smem, to_stream(s)>>>(
+        reinterpret_cast<const float4 *>(boxes), probs, cnt, spans, n, total, classes, thresh,
+        (unsigned long long *)ws, need ? 3 * P + P / 8 : 0);
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
+}
+
+extern "C" int y2_tile_collect(const float *boxes, const float *probs, const y2_tile_span *spans, int n, int total,
+                               int classes, float thresh, y2_det *det, int *count, int max_det, int *nz_count,
+                               y2_stream_t s)
+{
+    if (!boxes || !probs || !spans || !det || !count || !nz_count || n < 1 || n > 65535 || total < 1 ||
+        classes < 1 || max_det < 0) {
+        set_error("y2_tile_collect: invalid arguments (n=%d total=%d classes=%d max_det=%d)", n, total, classes,
+                  max_det);
+        return Y2_EINVAL;
+    }
+    tile_collect_kernel<<<n, TILE_COLLECT_THREADS, 0, to_stream(s)>>>(reinterpret_cast<const float4 *>(boxes), probs,
+                                                                     spans, total, classes, thresh, det, count,
+                                                                     max_det, nz_count);
+    Y2_LAUNCH_CHECK();
+    return Y2_OK;
+}
 
 extern "C" int y2_nms_unsorted(const float *boxes, float *probs, int total, int classes, float thresh, y2_stream_t s)
 {

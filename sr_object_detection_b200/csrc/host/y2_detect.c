@@ -4,7 +4,7 @@
  * caller-owned host arrays (boxes[total], probs[total][classes]) across, as the reference's
  * callers expect (detector.c:486-495, yolo_v2_class.cpp:71-73,215-216).  The batched entries describe their input
  * (y2_input) and hand it to the submit/wait pipeline of y2_pipeline.c; what is left here is their tails: decode, NMS
- * and pick (also on the 3-frame means of video streams), or WordTree and top-k.
+ * and pick (also on the 3-frame means of video streams, or merged over a frame's tiles), or WordTree and top-k.
  *
  * Reference interfaces replaced: get_region_boxes (region_layer.c:328-379), do_nms_sort
  * (box.c:249-277), box_iou & friends (box.c:67-97); for classification, the tail of predict_classifier
@@ -197,6 +197,33 @@ static void detect_tail(y2_net_rt *rt, layer *l, void *head_rt, float *pred, int
         Y2_CHECK(y2_nms_mark(r->boxes_dev, r->probs_dev, r->nms_cnt_dev, B, total, l->classes, nms, rt->stream));
     Y2_CHECK(y2_collect_ws(r->boxes_dev, r->probs_dev, B, total, l->classes, thresh, res->det_dev, res->cnt_dev,
                            res->det_cap, r->collect_ws, r->nms_cnt_dev, rt->stream));
+}
+
+/* The tail of a tiled batch on the network's stream: get_region_boxes on each of the tiles, their boxes to frame
+ * coordinates, do_nms_sort over each frame's union of tiles and the pick over it, into res's n detection lists (4
+ * launches).  The tile and span tables are in the slot's staged region on the device. */
+static void tiled_tail(y2_net_rt *rt, layer *l, float *pred, const unsigned char *staged_dev, const y2_tile_layout *lay,
+                       int n, float thresh, float nms, const y2_results *res)
+{
+    y2_layer_rt *r = (y2_layer_rt *)l->b200;
+    const int total = l->w * l->h * l->n, T = lay->n_tiles;
+    const y2_tile_span *spans = (const y2_tile_span *)(staged_dev + lay->spans_offset);
+    Y2_CHECK(y2_region_boxes_counted(pred, r->biases_dev, r->boxes_dev, r->probs_dev, T, l->w, l->h, l->n, l->classes,
+                                     1.f, 1.f, thresh, 0, l->classfix, 0, 0, 0, 0, r->nms_cnt_dev, rt->stream));
+    Y2_CHECK(y2_tile_map(r->boxes_dev, (const y2_tile *)(staged_dev + lay->tiles_offset), T, total, rt->stream));
+    if (nms > 0) {
+        const size_t ws = y2_tile_nms_ws_bytes(n, l->classes, (long long)lay->max_tiles * total);
+        if (ws > r->tile_ws_bytes) {
+            Y2_CHECK(y2_stream_sync(rt->stream)); /* the other slot's merge may still use the old scratch */
+            y2_free(r->tile_ws);
+            Y2_CHECK(y2_malloc(&r->tile_ws, ws));
+            r->tile_ws_bytes = ws;
+        }
+        Y2_CHECK(y2_tile_nms(r->boxes_dev, r->probs_dev, r->nms_cnt_dev, spans, n, total, l->classes, lay->max_tiles,
+                             nms, r->tile_ws, r->tile_ws_bytes, rt->stream));
+    }
+    Y2_CHECK(y2_tile_collect(r->boxes_dev, r->probs_dev, spans, n, total, l->classes, thresh, res->det_dev,
+                             res->cnt_dev, res->det_cap, r->nms_cnt_dev, rt->stream));
 }
 
 void network_detect_device(network net, float thresh, float nms, y2_detection *dets, int *counts, int max_det)
@@ -448,6 +475,8 @@ static int detect_submit(network net, y2_input in, const stream_list *streams, f
                                      (const int *)(st->table_dev[s] + track_offsets_at(n)), n_streams, total,
                                      st->classes, st->story, st->hist_dev, st->hist_cnt_dev, st->next_id_dev,
                                      ps->res.box_dev, ps->res.box_stride, rt->stream));
+    } else if (in.kind == Y2_IN_TILED) {
+        tiled_tail(rt, l, (float *)r->out, ps->frames_dev, &in.tiles, n, thresh, nms, &ps->res);
     } else {
         detect_tail(rt, l, head_rt, (float *)r->out, B, thresh, nms, &ps->res);
     }
@@ -625,6 +654,28 @@ void network_detect_batch_streams_descs(network net, int n, const int *stream_id
     detect_batch(net, "network_detect_batch_streams_descs: batches of the submit/wait pipeline are in flight",
                  descs_input(n, descs, ready), &(stream_list){n, stream_ids, 0, 1}, thresh, nms, dets, NULL, counts,
                  max_det);
+}
+
+/* ---- tiled detection: each frame as overlapping tiles, merged by do_nms_sort over their union -------------------- */
+static y2_input tiled_input(network net, int n, const y2_frame_desc *descs, const y2_tiling *tiling, void *ready)
+{
+    if (y2_rt(net) && region_of(net)->softmax_tree)
+        error("network tiled descs: needs a flat-softmax region head (softmax-tree heads are not supported)");
+    return (y2_input){.kind = Y2_IN_TILED, .descs = {n, descs, ready}, .tiling = tiling};
+}
+
+int network_detect_submit_tiled_descs(network net, int n, const y2_frame_desc *descs, const y2_tiling *tiling,
+                                      void *ready, float thresh, float nms, int max_det)
+{
+    return detect_submit(net, tiled_input(net, n, descs, tiling, ready), NULL, thresh, nms, max_det);
+}
+
+void network_detect_batch_tiled_descs(network net, int n, const y2_frame_desc *descs, const y2_tiling *tiling,
+                                      void *ready, float thresh, float nms, y2_detection *dets, int *counts,
+                                      int max_det)
+{
+    detect_batch(net, "network_detect_batch_tiled_descs: batches of the submit/wait pipeline are in flight",
+                 tiled_input(net, n, descs, tiling, ready), NULL, thresh, nms, dets, NULL, counts, max_det);
 }
 
 /* the frame widths then heights of a descriptor list, for the tracking plan (NULL for a list the pipeline refuses) */

@@ -67,6 +67,8 @@ typedef struct y2_layer_rt {
     int *nms_cnt_dev;   /* [B][classes] NMS candidate counters, zero between batches (owned per network: two
                            networks in flight on one GPU must not share them) */
     void *collect_ws;   /* per-box maxima scratch of the final pick (wide class rows) */
+    void *tile_ws;      /* spill scratch of the tiled merge's NMS (y2_tile_nms_ws_bytes), grown on demand */
+    size_t tile_ws_bytes;
     /* softmax tree: CSR of the groups below every node (node `classes` = virtual root) and the per-box records
      * of the sparse detection path; the dense region forward then runs on demand only (region_stale) */
     int *child_ptr_dev, *child_grp_dev;
@@ -116,6 +118,7 @@ typedef enum {
     Y2_IN_FRAMES,     /* uint8 interleaved RGB frames [B][fh][fw][3] of any size */
     Y2_IN_FRAME_LIST, /* 1 .. B frames of their own sizes */
     Y2_IN_FRAME_DESCS, /* 1 .. B frame descriptors: RGB, BGR or NV12 with a pitch, in host or device memory */
+    Y2_IN_TILED,      /* frame descriptors cut into tiles (descs + tiling), 1 .. B tiles in all */
     Y2_IN_RESIDENT,   /* nothing: the slot's device input already holds the batch */
 } y2_input_kind;
 
@@ -133,7 +136,9 @@ typedef struct {
         const y2_frame_desc *d;
         void *ready;           /* cudaEvent_t the compute stream waits for before it reads device frames, or NULL */
     } descs;
-    int n;                     /* images the batch hands back: the list's length, else the batch */
+    const y2_tiling *tiling;   /* Y2_IN_TILED */
+    y2_tile_layout tiles;      /* Y2_IN_TILED: the staged plan, y2_pipe_claim fills it */
+    int n;                     /* images the batch hands back: the list's length (frames), else the batch */
 } y2_input;
 
 typedef struct y2_net_rt {

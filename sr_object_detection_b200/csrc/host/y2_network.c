@@ -511,6 +511,7 @@ static void free_layer_rt(layer *l)
     y2_free(r->biases_dev);
     y2_free(r->nms_cnt_dev);
     y2_free(r->collect_ws);
+    y2_free(r->tile_ws);
     y2_free(r->child_ptr_dev);
     y2_free(r->child_grp_dev);
     y2_free(r->tree_rec_dev);
@@ -1537,6 +1538,7 @@ size_t y2_abi_sizeof(int what)
     case 5: return sizeof(y2_class_hit);
     case 6: return sizeof(y2_bbox);
     case 7: return sizeof(y2_frame_desc);
+    case 8: return sizeof(y2_tiling);
     default: return 0;
     }
 }

@@ -1,7 +1,7 @@
 /*
  * The two-deep submit/wait pipeline: the H2D copy of batch i+1 overlaps the forward pass of batch i, and the results
  * of batch i return under the forward pass of batch i+1.  This file owns the slots (creating them, growing their
- * buffers, releasing them on a re-plan, freeing them), the staging getters, the frame-list and frame-descriptor
+ * buffers, releasing them on a re-plan, freeing them), the staging getters, the frame-list, frame-descriptor and tiled
  * checks and staging, the input half of a submission, and claiming and retiring a slot.  The detection and classify
  * tails and their entry points are in y2_detect.c.
  */
@@ -248,19 +248,39 @@ static void check_frame_descs(network net, const struct y2_frame_descs *fd)
     }
 }
 
+/* The refusals of the tiled entries, before anything is staged: the descriptor list's, then the tiling's; fills the
+ * input's tile plan (layout only). */
+static void check_tiled(network net, y2_input *in)
+{
+    static const char *const broken[] = {
+        [Y2_TILE_BAD_DESC] = "network tiled descs: a descriptor the tile plan refuses",
+        [Y2_TILE_NULL] = "network tiled descs: NULL tiling",
+        [Y2_TILE_BAD_GRID] = "network tiled descs: cols and rows must be in 1 .. Y2_TILE_MAX",
+        [Y2_TILE_BAD_OVERLAP] = "network tiled descs: overlap must be 0 or more",
+        [Y2_TILE_BAD_FULL] = "network tiled descs: full must be 0 or 1",
+        [Y2_TILE_TOO_MANY] = "network tiled descs: more tiles than the network's batch (a frame's tiles are images of "
+                             "one batch)"};
+    check_frame_descs(net, &in->descs);
+    const int rc = y2_tile_plan(in->descs.n, in->descs.d, in->tiling, net.w, net.h, net.batch, NULL, &in->tiles);
+    if (rc != Y2_TILE_OK) error(broken[rc]);
+}
+
 /* The one place an input is decided: frames at the network's resolution become uint8 input when the network has the
  * first-layer kernel for it; each kind's refusals and lazy set-up; in.n. */
 static y2_input pipe_input(network net, y2_input in)
 {
     if (in.kind == Y2_IN_FRAME_LIST) check_frame_list(net, &in.list);
     if (in.kind == Y2_IN_FRAME_DESCS) check_frame_descs(net, &in.descs);
+    if (in.kind == Y2_IN_TILED) check_tiled(net, &in);
     if (!y2_rt(net)) error("network submit: network has no device plan");
     if (in.kind == Y2_IN_FRAMES && in.fw == net.w && in.fh == net.h && takes_u8(net)) in.kind = Y2_IN_U8;
     pipe_init(y2_rt(net));
     if (in.kind == Y2_IN_U8) pipe_init_u8(net);
     if (in.kind == Y2_IN_FRAMES && (net.c != 3 || in.fw <= 0 || in.fh <= 0))
         error("network submit of frames: needs 3-channel input and a frame size");
-    in.n = in.kind == Y2_IN_FRAME_LIST ? in.list.n : in.kind == Y2_IN_FRAME_DESCS ? in.descs.n : net.batch;
+    in.n = in.kind == Y2_IN_FRAME_LIST                               ? in.list.n
+           : in.kind == Y2_IN_FRAME_DESCS || in.kind == Y2_IN_TILED ? in.descs.n
+                                                                     : net.batch;
     return in;
 }
 
@@ -411,6 +431,39 @@ static size_t stage_frame_descs(network net, int s, const struct y2_frame_descs 
     return table_off;
 }
 
+/* A tiled descriptor list into slot s: the tile plan's region in the slot's pinned buffer, each host frame copied in
+ * once (tight) and its tiles' records pointed into the device buffer, then one H2D copy of the whole region on the
+ * copy stream.  Device frames' tiles read them in place. */
+static void stage_tiled(network net, int s, const y2_input *in)
+{
+    y2_net_rt *rt = y2_rt(net);
+    struct y2_pipe_slot *ps = &rt->pipe[s];
+    const struct y2_frame_descs *fd = &in->descs;
+    const y2_tile_layout *lay = &in->tiles;
+    unsigned char *old = NULL;
+    pipe_reserve_frames(rt, s, lay->bytes, &old);
+    y2_tile_plan(fd->n, fd->d, in->tiling, net.w, net.h, net.batch, ps->frames_pinned, NULL);
+    y2_frame_src *rec = (y2_frame_src *)(ps->frames_pinned + lay->recs_offset);
+    const y2_tile_span *spans = (const y2_tile_span *)(ps->frames_pinned + lay->spans_offset);
+    const unsigned long long base = (unsigned long long)(uintptr_t)ps->frames_dev;
+    for (int i = 0; i < fd->n; ++i) {
+        const y2_frame_desc *d = &fd->d[i];
+        if (d->on_device) continue;
+        const int nv12 = d->format == Y2_FRAME_NV12;
+        const y2_frame_src *r0 = &rec[spans[i].first]; /* the first tile starts at (0, 0): the frame's own place */
+        y2_frame_rows fr;
+        y2_frame_desc_rows(d, &fr);
+        copy_rows(ps->frames_pinned + r0->win.offset, (const unsigned char *)d->data, d->h, fr.row, fr.pitch);
+        if (nv12) copy_rows(ps->frames_pinned + r0->uv, fr.uv, d->h / 2, fr.row, fr.uv_pitch);
+        for (int t = spans[i].first; t < spans[i].first + spans[i].count; ++t) {
+            rec[t].win.offset += base;
+            if (nv12) rec[t].uv += base;
+        }
+    }
+    Y2_CHECK(y2_host_free(old));
+    Y2_CHECK(y2_memcpy_h2d(ps->frames_dev, ps->frames_pinned, lay->bytes, rt->copy_stream));
+}
+
 /* pageable caller memory is staged through the slot's pinned buffer (a host copy; fill the slot's staging buffer
  * directly to avoid it), then copied to the device on the copy stream */
 static void stage(void *dev, void *pinned, const void *src, size_t bytes, y2_stream_t copy_stream)
@@ -443,6 +496,9 @@ void y2_pipe_submit_input(network net, int s, const y2_input *in, int letterbox)
         table_off = stage_frame_list(net, s, &in->list, letterbox);
     } else if (in->kind == Y2_IN_FRAME_DESCS) {
         table_off = stage_frame_descs(net, s, &in->descs, letterbox);
+    } else if (in->kind == Y2_IN_TILED) {
+        stage_tiled(net, s, in);
+        table_off = in->tiles.recs_offset;
     } else if (in->kind == Y2_IN_FRAMES) {
         const size_t bytes = (size_t)B * in->fh * in->fw * 3;
         pipe_reserve_frames(rt, s, bytes, NULL);
@@ -456,13 +512,14 @@ void y2_pipe_submit_input(network net, int s, const y2_input *in, int letterbox)
         Y2_CHECK(y2_event_record(ps->ev_h2d, rt->copy_stream));
         Y2_CHECK(y2_stream_wait_event(rt->stream, ps->ev_h2d));
     }
-    if (in->kind == Y2_IN_FRAME_DESCS && in->descs.ready) /* the producer of the device frames */
+    if ((in->kind == Y2_IN_FRAME_DESCS || in->kind == Y2_IN_TILED) && in->descs.ready) /* the device frames' producer */
         Y2_CHECK(y2_stream_wait_event(rt->stream, in->descs.ready));
     if (in->kind == Y2_IN_FRAME_LIST) /* byte/255. + resize_image or letterbox_image per frame, .5f behind the list */
         Y2_CHECK(y2_frames_u8_to_f32(ps->frames_dev, (const y2_frame_window *)(ps->frames_dev + table_off), in->n,
                                      ps->in_dev, B, net.w, net.h, rt->stream));
-    else if (in->kind == Y2_IN_FRAME_DESCS) /* to RGB, then as the frame list */
-        Y2_CHECK(y2_frames_src_to_f32((const y2_frame_src *)(ps->frames_dev + table_off), in->n, ps->in_dev, B, net.w,
+    else if (in->kind == Y2_IN_FRAME_DESCS || in->kind == Y2_IN_TILED) /* to RGB, then as the frame list; per tile */
+        Y2_CHECK(y2_frames_src_to_f32((const y2_frame_src *)(ps->frames_dev + table_off),
+                                      in->kind == Y2_IN_TILED ? in->tiles.n_tiles : in->n, ps->in_dev, B, net.w,
                                       net.h, rt->stream));
     else if (in->kind == Y2_IN_FRAMES && letterbox) /* byte/255. + letterbox_image, into the slot's fp32 input */
         Y2_CHECK(y2_letterbox_u8_to_f32(ps->frames_dev, ps->in_dev, B, in->fw, in->fh, net.w, net.h, rt->stream));

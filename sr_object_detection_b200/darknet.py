@@ -110,6 +110,8 @@ class BBox(C.Structure):
 
 FrameDesc = _lib.FrameDesc
 FRAME_RGB24, FRAME_BGR24, FRAME_NV12 = 0, 1, 2  # y2_frame_desc.format
+Tiling = _lib.Tiling
+TILE_MAX = 16  # Y2_TILE_MAX: most columns or rows of a tiling
 
 
 class Image(C.Structure):
@@ -205,6 +207,10 @@ def lib() -> C.CDLL:
                                                              i, i]),
         "network_detect_batch_streams_tracked_descs": (None, [Network, i, _ip, C.POINTER(FrameDesc), C.c_void_p, f,
                                                               f, i, C.POINTER(BBox), _ip, i]),
+        "network_detect_submit_tiled_descs": (i, [Network, i, C.POINTER(FrameDesc), C.POINTER(Tiling), C.c_void_p, f,
+                                                   f, i]),
+        "network_detect_batch_tiled_descs": (None, [Network, i, C.POINTER(FrameDesc), C.POINTER(Tiling), C.c_void_p,
+                                                    f, f, C.POINTER(Detection), _ip, i]),
         "network_classify_submit_frame_descs": (i, [Network, i, C.POINTER(FrameDesc), C.c_void_p, i]),
         "network_classify_batch_frame_descs": (None, [Network, i, C.POINTER(FrameDesc), C.c_void_p, i,
                                                       C.POINTER(ClassHit)]),
@@ -272,6 +278,7 @@ def lib() -> C.CDLL:
     assert l.y2_abi_sizeof(5) == C.sizeof(ClassHit)
     assert l.y2_abi_sizeof(6) == C.sizeof(BBox)
     assert l.y2_abi_sizeof(7) == C.sizeof(FrameDesc), (l.y2_abi_sizeof(7), C.sizeof(FrameDesc))
+    assert l.y2_abi_sizeof(8) == C.sizeof(Tiling), (l.y2_abi_sizeof(8), C.sizeof(Tiling))
     _declared = True
     return l
 
@@ -670,6 +677,35 @@ def network_detect_submit_frame_descs(net: Network, descs, thresh: float, nms: f
     """Queue a descriptor list on the submit/wait pipeline; network_detect_wait_n(net, len(descs), ...) collects it."""
     n, arr = _descs_arg(descs)
     return lib().network_detect_submit_frame_descs(net, n, arr, ready, thresh, nms, max_det)
+
+
+def _tiling_arg(tiling):
+    if tiling is None:
+        return None
+    if not isinstance(tiling, Tiling):
+        tiling = Tiling(*tiling)
+    return C.byref(tiling)
+
+
+def network_detect_tiled_descs(net: Network, descs, tiling, thresh: float, nms: float, max_det: int = 256,
+                               ready=None):
+    """Extension: tiled detection of a list of frame descriptors (frame_desc).  Each frame goes through the network as
+    the tiles of `tiling` (a Tiling, or a (cols, rows, overlap, full) tuple), and its detections are merged by
+    do_nms_sort over the union of its tiles' boxes.  Returns (per-frame detection arrays relative to the frame,
+    counts); box_index is the index in the frame's union (tile * l.w*l.h*l.n + box)."""
+    n, arr = _descs_arg(descs)
+    dets = (Detection * (max(n, 1) * max_det))()
+    counts = (C.c_int * max(n, 1))()
+    lib().network_detect_batch_tiled_descs(net, n, arr, _tiling_arg(tiling), ready, thresh, nms, dets, counts, max_det)
+    return _det_lists(dets, counts, n, max_det)
+
+
+def network_detect_submit_tiled_descs(net: Network, descs, tiling, thresh: float, nms: float, max_det: int = 256,
+                                      ready=None) -> int:
+    """Queue a tiled descriptor list on the submit/wait pipeline; network_detect_wait_n(net, len(descs), ...) collects
+    it."""
+    n, arr = _descs_arg(descs)
+    return lib().network_detect_submit_tiled_descs(net, n, arr, _tiling_arg(tiling), ready, thresh, nms, max_det)
 
 
 def network_detect_streams_descs(net: Network, stream_ids, descs, thresh: float, nms: float, max_det: int = 256,

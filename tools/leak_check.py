@@ -120,6 +120,35 @@ def descs_cycle(name, side, batch):
     dn.free_network(net)
 
 
+def tiled_cycle(name, side, batch):
+    text = synth.CFGS[name](batch=batch, w=side, h=side)
+    (tmp / "tl.cfg").write_text(text)
+    w = tmp / f"{name}.weights"
+    if not w.exists():
+        synth.write_weights(w, text, seed=1234)
+    net = dn.parse_network_cfg(tmp / "tl.cfg")
+    dn.load_weights(net, w)
+    rng = np.random.default_rng(6)
+    frames, descs = [], []
+    for i, fmt in enumerate((dn.FRAME_NV12, dn.FRAME_RGB24, dn.FRAME_BGR24)):
+        a = rng.integers(0, 256, size=(1620, 1920) if fmt == dn.FRAME_NV12 else (1080, 1920, 3), dtype=np.uint8)
+        if i == 1:
+            a = torch.from_numpy(a).cuda()
+        frames.append(a)
+        descs.append(dn.frame_desc(a, fmt))
+    torch.cuda.synchronize()
+    # the spill scratch of the merge grows with the tiles of a frame and the candidates (a low thresh)
+    dn.network_detect_submit_tiled_descs(net, descs, (2, 2, 64, 1), 0.02, 0.45, 64)
+    dn.network_detect_submit_tiled_descs(net, descs[:2], (3, 2, 64, 1), 0.0001, 0.45, 64)
+    dn.network_detect_wait_n(net, 3, 64)
+    dn.network_detect_wait_n(net, 2, 64)
+    dn.network_detect_tiled_descs(net, descs[1:2], (4, 3, 32, 1), 0.0001, 0.45, 64)
+    dn.set_batch_network(net, batch * 2)  # a re-plan drops the scratch with the region's buffers
+    dn.network_detect_tiled_descs(net, descs, (3, 3, 16, 0), 0.02, 0.45, 64)
+    dn.free_network(net)
+    del frames, descs
+
+
 def streams_cycle(name, side, batch):
     text = synth.CFGS[name](batch=batch, w=side, h=side)
     (tmp / "s.cfg").write_text(text)
@@ -172,7 +201,7 @@ def tracked_cycle(name, side, batch):
 
 for fn, name, side, batch in ((cycle, "tiny-yolo-voc", 416, 8), (cycle, "yolo-voc", 416, 64),
                               (classify_cycle, "darknet19_448", 448, 16), (frame_list_cycle, "tiny-yolo-voc", 416, 16),
-                              (descs_cycle, "tiny-yolo-voc", 416, 16),
+                              (descs_cycle, "tiny-yolo-voc", 416, 16), (tiled_cycle, "tiny-yolo-voc", 416, 16),
                               (streams_cycle, "tiny-yolo-voc", 416, 16), (tracked_cycle, "tiny-yolo-voc", 416, 16)):
     fn(name, side, batch)  # warm: allocator pools, per-device scratch
     torch.cuda.synchronize()
